@@ -2,7 +2,7 @@
 """bench.py -- the hot path of sparsify.me on B200: 2:4 magnitude prune+compress of every weight
 matrix of a ResNet shape table, then the 2:4 sparse GEMM (spmma) of every layer.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One STEP = one pass over one batch of synthetic input: ONE batched prune+compress launch over all
 layers' weights (spfy_prune24_batched) + the spmma of every layer through one plan
@@ -363,6 +363,8 @@ def run_coo(args):
     cnt = collections.Counter((s.n, s.k, s.m) for s in shapes)  # (M, K, n = H*W) -> layers of that shape
     gen = torch.Generator(device=dev)
     gen.manual_seed(0x5EED)  # same weights on every rank (replicated, pruned redundantly)
+    gen_b = torch.Generator(device=dev)
+    gen_b.manual_seed(0xB0 + rank)  # every rank its own images
     work = []
     for (M, K, n), c in cnt.items():
         w = torch.rand(M, K, device=dev, generator=gen) * 2 - 1
@@ -370,7 +372,7 @@ def run_coo(args):
         thr = float(torch.kthvalue(w.abs().flatten(), kth).values)
         per_set = 4 * (K + M) * n * max(nb, 1)
         nsets = max(1, min(4, -(-300_000_000 // max(per_set, 1))))  # rotate so that nothing is served from L2
-        bs = [torch.rand(max(nb, 1), n, K, device=dev) * 2 - 1 for _ in range(nsets)]
+        bs = [torch.rand(max(nb, 1), n, K, device=dev, generator=gen_b) * 2 - 1 for _ in range(nsets)]
         cs = [torch.empty(max(nb, 1), n, M, device=dev) for _ in range(nsets)]
         nnz = int((w.abs() > thr).sum())
         work.append(dict(M=M, K=K, n=n, count=c, w=w, thr=thr, b=bs, c=cs, nnz=nnz, cap=nnz + 16))
@@ -398,10 +400,10 @@ def run_coo(args):
                 by += 12 * nnz + 4.0 * (x["K"] + x["M"]) * x["n"] * nb
         return fl, by
 
-    for i in range(max(1, min(args.warmup, 3))):
+    for i in range(args.warmup):
         spmm_step(i, prune_step())
     torch.cuda.synchronize()
-    steps = max(1, min(args.steps, 20))  # a step is tens of milliseconds
+    steps = args.steps
 
     # The step is ~600 short launches with no host read-back anywhere, i.e. bound by how fast the host can
     # launch (and with eight ranks on one box, by the host cores they share): capture it once per operand
@@ -476,10 +478,24 @@ def run_coo(args):
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         t[:3] = tmax[:3]
     ms, prune_ms, spmm_ms, fl_all, by_all = (float(x) for x in t.tolist())
+    if args.dump_outputs and rank == 0:
+        # the last step: every layer's C (this rank's images; a layer's operand set depends on the step), and the COO /
+        # CSR weights of every shape (the layers of one shape share them)
+        arrays, coos, i = {}, (coos_g if graphs else coos), 0
+        for xi, x in enumerate(work):
+            ri, ci, va, nnz, rp = coos[i]
+            n = int(nnz.item())
+            arrays.update({f"coo_rows_{xi:03d}": ri[:n], f"coo_cols_{xi:03d}": ci[:n], f"coo_vals_{xi:03d}": va[:n],
+                           f"csr_row_ptr_{xi:03d}": rp})
+            for rep in range(x["count"]):
+                if nb:
+                    arrays[f"c_{i:03d}"] = x["c"][((steps - 1) * x["count"] + rep) % len(x["c"])]
+                i += 1
+        dump_outputs(args.dump_outputs, arrays)
     if rank == 0:
         print(json.dumps({
             "metric": "batched COO SpMM TFLOP/s (2*nnz*N) over a ResNet table, threshold prune included", "value": fl_all / ms / 1e9,
-            "unit": UNIT, "n_gpus": world, "steps": steps, "warmup": max(1, min(args.warmup, 3)), "ms_per_step": ms,
+            "unit": UNIT, "n_gpus": world, "steps": steps, "warmup": args.warmup, "ms_per_step": ms,
             "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"datasets/{csv}: all {len(shapes)} layers, weights kept above the {args.sparsity:.2f} magnitude "
                                    f"quantile -> COO, batched COO SpMM over {args.batch} images sharded across {world} rank(s)",
@@ -565,6 +581,8 @@ def run_strong(args):
             d = arena[rank, off: off + g.M * g.N].view(g.M, g.N)
             off += g.M * g.N
             comp = spfy.alloc_compressed(tdt, g.M, g.K, dev)
+            comp.vals.zero_()  # padding bytes prune24 leaves alone are the same in every run (--dump-outputs)
+            comp.meta.zero_()
             layers.append((g, w, b, d, comp, c, off - g.M * g.N))
             probs.append(dict(comp=comp, b=b, out=d))
         plans.append(spfy.SpmmaPlan(probs))
@@ -637,7 +655,7 @@ def run_strong(args):
     clocks = sampler.stop() if rank == 0 else None
     launches = (spfy.launch_count() - launches0) // (args.steps + max(1, args.warmup // 2))
     compute_ms = timed(True, False, args.steps)
-    gather_ms = timed(False, True, max(2, args.steps // 2)) if world > 1 else 0.0
+    gather_ms = timed(False, True, args.steps) if world > 1 else 0.0
     fused_ms = timed(True, True, args.steps, step=step_fused) if fused else None
 
     # ---- the gathered slabs are what the other ranks computed: per-rank checksums travel by all_gather and are compared
@@ -682,6 +700,14 @@ def run_strong(args):
         dist.all_reduce(flag, op=dist.ReduceOp.MIN)
     if float(flag.item()) != 1.0:
         raise SystemExit(f"bench.py --strong: verification failed on some rank (gather ok {ok_gather}, max rel err {worst:.3e})")
+    if args.dump_outputs and rank == 0:
+        # the step above is the timed step once more (compute + gather): every layer's output as gathered onto this rank,
+        # [world][M][N / world], and the compressed weights
+        arrays = {}
+        for i, (g, w, b, d, comp, c, off) in enumerate(layers):
+            arrays[f"d_{i:03d}"] = arenas[c][:, off: off + g.M * g.N]
+            arrays.update(compressed_arrays(i, comp))
+        dump_outputs(args.dump_outputs, arrays)
 
     if rank == 0:
         flops = sum(spfy.shapes.spmma_flops(g) for g in gemms_global)
@@ -751,7 +777,14 @@ def main():
                          "outputs all-gathered onto every rank (compute-only / gather-only / overlapped are all reported)")
     ap.add_argument("--chunks", type=int, default=6, help="--strong: groups of layers per gather")
     ap.add_argument("--no-fused", action="store_true", help="--strong: skip the fused gather (epilogue stores to peer memory)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (every layer's output and its compressed or COO weights) "
+                         "to DIR/<name>.npy; not with --impl reference")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a bounded CPU sample, not the whole step")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "coo":
@@ -789,8 +822,9 @@ def main():
         b = (torch.rand(g.K, g.N, device=dev, generator=gen) * 2 - 1).to(tdt)
         d = torch.empty(g.M, g.N, device=dev, dtype=tdt)
         vb, mb = spfy.compressed_bytes(tdt, g.M, g.K)
-        comp = spfy.Compressed24(torch.empty(vb, dtype=torch.uint8, device=dev),
-                                 torch.empty(mb, dtype=torch.uint8, device=dev), g.M, g.K, tdt, spfy.LAYOUT_SM100)
+        # zero-filled, so that bytes of the padded tiles that prune24 leaves alone are the same in every run (--dump-outputs)
+        comp = spfy.Compressed24(torch.zeros(vb, dtype=torch.uint8, device=dev),
+                                 torch.zeros(mb, dtype=torch.uint8, device=dev), g.M, g.K, tdt, spfy.LAYOUT_SM100)
         layers.append((g, w, b, d, comp))
 
     def prune_all():
@@ -842,6 +876,12 @@ def main():
     total_ms, prune_ms, spmma_ms = (float(x) for x in t.tolist())
     ms_per_step = total_ms / args.steps
     value = flops_step * world / (ms_per_step * 1e-3) / 1e12
+    if args.dump_outputs and rank == 0:
+        arrays = {}
+        for i, (g, w, b, d, comp) in enumerate(layers):
+            arrays[f"d_{i:03d}"] = d
+            arrays.update(compressed_arrays(i, comp))
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- the timed outputs are checked, not just produced: D of the last timed step against a torch fp32 matmul of
     #      the pruned weights (decoded by the same prune kernel family), first / middle / last / largest-K layers, every
@@ -1126,6 +1166,31 @@ def main():
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_BYTES = 48 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """`arrays` ({name: tensor}, in a fixed order) to out_dir/<name>.npy, DUMP_BYTES in all whatever the table:
+    float32, or float64 for int32 indices so that they stay exact.  An array larger than its share is written as a
+    1-D sample at sorted positions drawn with its position in `arrays` as seed, so two builds run with the same
+    arguments write the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // 8 // len(arrays)
+    for i, (name, a) in enumerate(arrays.items()):
+        if a.numel() > cap:
+            idx = np.sort(np.random.default_rng(i).choice(a.numel(), cap, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        a = a.double() if a.dtype == torch.int32 else a.float()
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
+def compressed_arrays(i, comp):
+    """the compressed operand prune24_batched hands its caller: values (in the weights' dtype) and metadata bytes"""
+    return {f"vals_{i:03d}": comp.vals.view(comp.dtype), f"meta_{i:03d}": comp.meta}
 
 
 def per_layer_report(spfy, layers, hbm_peak, tc_peak, quiet=False):
