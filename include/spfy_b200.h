@@ -64,8 +64,9 @@ enum { SPFY_LAYOUT_CANONICAL = 0, SPFY_LAYOUT_SM100 = 1 };
 
 enum { SPFY_OP_N = 0, SPFY_OP_T = 1 }; /* == cusparseOperation_t values */
 /* OR-ed into the `opB` argument of spfy_spmma / spfy_spmma_problem: D is written TRANSPOSED, [n][m] row-major with pitch
- * ldd >= m -- for a convolution layer that is NHWC, what spfy_spmma_conv of the next layer reads.  beta must be 0 and
- * m a multiple of 8 (the contiguous dimension of an output always is: n for the row-major one). */
+ * ldd >= m -- for a convolution layer that is NHWC, what spfy_spmma_conv of the next layer reads.  beta must be 0 (except
+ * in the _ex entry points, see spfy_epilogue) and m a multiple of 8 (the contiguous dimension of an output always is: n
+ * for the row-major one). */
 enum { SPFY_OUT_T = 0x10 };
 
 enum {
@@ -186,6 +187,38 @@ SPFY_API int spfy_spmma_conv(int dtype, const spfy_conv_desc* conv, size_t m, fl
 SPFY_API int spfy_spmma_conv_nhwc(int dtype, const spfy_conv_desc* conv, size_t m, float alpha,
                                   const void* comp_vals, const void* meta, const void* X, void* Y, size_t ldy,
                                   spfy_stream_t stream);
+/* Epilogue of the _ex entry points (cusparseLt's ALPHA_VECTOR_SCALING, BIAS_POINTER, ACTIVATION_RELU / _GELU): what
+ * happens between two layers -- batch norm folded into a per-channel scale and bias, the activation, the shortcut add
+ * of a residual block (beta * C) -- done on the accumulators, before the output is written once.  Per output element
+ * (i, j), all in fp32, rounded to 16 bit once at the end:
+ *     v = (alpha * scale[i]) * acc + beta * C + bias[i],   D = act(v)
+ * alpha * scale[i] is formed once per row (exactly alpha when scale is NULL); the product with acc is rounded, then
+ * beta * C is added with one fused multiply-add, then bias[i].  SPFY_ACT_GELU_TANH is the tanh form
+ * 0.5 v (1 + tanh(sqrt(2/pi) (v + 0.044715 v^3))) -- torch's gelu(approximate="tanh"), cuBLASLt's and cusparseLt's
+ * GELU -- with the hardware tanh approximation (relative error ~2^-11).  i is the output row of A: the output channel
+ * of a convolution, the output feature of a Linear layer (y = x W^T + b is opB = T with B = x and SPFY_OUT_T).
+ * scale / bias are device arrays of m floats, 4-byte aligned; NULL means 1 / 0.  A NULL epilogue pointer, or one with
+ * both arrays NULL and SPFY_ACT_NONE, is the identity: the call computes exactly what the plain entry point does.
+ * In the _ex entries beta != 0 is also allowed with SPFY_OUT_T: C then has D's layout, [n][m] with ldc >= m,
+ * ldc % 8 == 0 and a 16-byte aligned base, and D may alias C (the shortcut add of a bottleneck block, in NHWC). */
+enum { SPFY_ACT_NONE = 0, SPFY_ACT_RELU = 1, SPFY_ACT_GELU_TANH = 2 };
+typedef struct spfy_epilogue {
+  const float* scale; /* [m] device, per output row / channel; NULL = 1 */
+  const float* bias;  /* [m] device; NULL = 0 */
+  int act;            /* SPFY_ACT_* */
+} spfy_epilogue;
+/* spfy_spmma with an epilogue (NULL = identity) */
+SPFY_API int spfy_spmma_ex(int dtype, int opB, size_t m, size_t n, size_t k, float alpha,
+                           const void* comp_vals, const void* meta, const void* B, size_t ldb,
+                           float beta, const void* C, size_t ldc, void* D, size_t ldd,
+                           void* workspace, size_t workspace_bytes, const spfy_epilogue* epi,
+                           spfy_stream_t stream);
+/* spfy_spmma_conv / spfy_spmma_conv_nhwc with an epilogue: layout 0 writes D[m][N] (ldd >= N), SPFY_OUT_T writes NHWC
+ * D[N][m] (ldd >= m); C, read when beta != 0, has D's layout. */
+SPFY_API int spfy_spmma_conv_ex(int dtype, const spfy_conv_desc* conv, size_t m, float alpha,
+                                const void* comp_vals, const void* meta, const void* X, float beta,
+                                const void* C, size_t ldc, void* D, size_t ldd, int layout,
+                                const spfy_epilogue* epi, spfy_stream_t stream);
 /* weights [m][c * kh * kw] in (c, kh, kw) column order (what torch's unfold / a flattened conv weight uses)
  * -> [m][kh * kw * c] in (kh, kw, c) order; 16-bit elements */
 SPFY_API int spfy_permute_conv_weights(const void* in, void* out, size_t m, size_t c, size_t kh, size_t kw,
@@ -230,6 +263,12 @@ SPFY_API int spfy_spmma_plan_create_replicated(int dtype, const spfy_spmma_probl
  * only.  Results are bitwise those of the single calls. */
 SPFY_API int spfy_spmma_plan_create_conv(int dtype, const spfy_spmma_problem* problems,
                                          const spfy_conv_desc* const* convs, size_t count, spfy_spmma_plan_t* plan);
+/* A plan with epilogues: as spfy_spmma_plan_create_conv (convs may be NULL), plus epilogues[i] for problem i (the array
+ * and its entries may be NULL; read at creation only).  Same launches as without epilogues; every output is bitwise
+ * that of the single _ex call. */
+SPFY_API int spfy_spmma_plan_create_ex(int dtype, const spfy_spmma_problem* problems,
+                                       const spfy_conv_desc* const* convs, const spfy_epilogue* const* epilogues,
+                                       size_t count, spfy_spmma_plan_t* plan);
 SPFY_API int spfy_spmma_plan_run(spfy_spmma_plan_t plan, spfy_stream_t stream);
 SPFY_API int spfy_spmma_plan_launches(spfy_spmma_plan_t plan); /* kernel launches per run */
 /* introspection / profiling: run one of the plan's launches, or describe it */

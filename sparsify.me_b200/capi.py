@@ -22,6 +22,7 @@ OUT_T = 0x10  # flag OR-ed into opB: D is written transposed, [n][m]
 SPMM_ALG_DEFAULT, SPMM_ALG_CUDA_CORE, SPMM_ALG_TENSOR, SPMM_ALG_TENSOR_FAST = 0, 1, 2, 3
 GEMM_PRECISE, GEMM_FAST = 0, 1
 GEMM_CTA_PAIRS = 0x10  # flag, OR-ed into `precision`: the cta_group::2 kernel where it applies
+ACT_NONE, ACT_RELU, ACT_GELU_TANH = 0, 1, 2
 OK, E_INVALID, E_UNSUPPORTED, E_CUDA, E_WORKSPACE, E_NCCL = 0, -1, -2, -3, -4, -5
 
 
@@ -56,10 +57,14 @@ SIGNATURES = {
                            _P, _SZ, _P, _SZ, _P]),
     "spfy_spmma_conv": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _SZ, _P, _SZ, _P]),
     "spfy_spmma_conv_nhwc": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, _P, _SZ, _P]),
+    "spfy_spmma_ex": (c_int, [c_int, c_int, _SZ, _SZ, _SZ, c_float, _P, _P, _P, _SZ, c_float, _P, _SZ,
+                              _P, _SZ, _P, _SZ, _P, _P]),
+    "spfy_spmma_conv_ex": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _SZ, _P, _SZ, c_int, _P, _P]),
     "spfy_permute_conv_weights": (c_int, [_P, _P, _SZ, _SZ, _SZ, _SZ, _P]),
     "spfy_spmma_plan_create": (c_int, [c_int, _P, _SZ, POINTER(c_void_p)]),
     "spfy_spmma_plan_create_replicated": (c_int, [c_int, _P, _SZ, _SZ, _P, POINTER(c_void_p)]),
     "spfy_spmma_plan_create_conv": (c_int, [c_int, _P, _P, _SZ, POINTER(c_void_p)]),
+    "spfy_spmma_plan_create_ex": (c_int, [c_int, _P, _P, _P, _SZ, POINTER(c_void_p)]),
     "spfy_spmma_plan_run": (c_int, [_P, _P]),
     "spfy_spmma_plan_launches": (c_int, [_P]),
     "spfy_spmma_plan_run_launch": (c_int, [_P, c_int, _P]),
@@ -114,6 +119,11 @@ class ConvDesc(ctypes.Structure):
     """struct spfy_conv_desc"""
     _fields_ = [("batch", c_size_t), ("h", c_size_t), ("w", c_size_t), ("c", c_size_t), ("kh", c_size_t), ("kw", c_size_t),
                 ("stride", c_size_t), ("pad", c_size_t)]
+
+
+class Epilogue(ctypes.Structure):
+    """struct spfy_epilogue"""
+    _fields_ = [("scale", c_void_p), ("bias", c_void_p), ("act", c_int)]
 
 
 class Prune24Item(ctypes.Structure):

@@ -4,7 +4,8 @@
 //     D[m x n] = alpha * A(2:4)[m x k] * op(B)[k x n] + beta * C[m x n]
 // all row-major like the reference's descriptors (spmma.hxx:56-64), fp16 or bf16 in, fp32
 // accumulation in TMEM, fp16/bf16 out.  Two entry points share one kernel:
-//     spfy_spmma            one problem (what the header template calls)
+//     spfy_spmma            one problem (what the header template calls); spfy_spmma_ex adds the epilogue
+//                           (per-row scale / bias, ReLU / GELU, beta * C with the transposed output)
 //     spfy_spmma_plan_*     a list of independent problems (the per-layer GEMMs of a
 //                           datasets/*.csv table) executed by one persistent launch per launch class
 //                           present (ring geometry; six classes), chained tail-to-head
@@ -29,7 +30,7 @@
 //                          tcgen05.mma.sp.cta_group::1.kind::f16 (M128 x N128 x K32);
 //                          tcgen05.commit frees ring stages / publishes accumulators
 //   warps 2-9   epilogue : a warp owns 32 rows x 64 columns of an accumulator: tcgen05.ld ->
-//                          alpha/beta -> fp16/bf16 -> its own swizzled 4 KiB staging buffer -> its own
+//                          alpha/beta (or the epilogue) -> fp16/bf16 -> its own swizzled 4 KiB staging buffer -> its own
 //                          TMA store.  No CTA-wide barrier in steady state.  Streaming classes
 //                          run 4 of the 8 warps (2 column halves each) to leave room for the ring.
 // TMEM: three 128-column accumulator slots used as a ring over (unit, m-tile) jobs, so the epilogue
@@ -102,6 +103,13 @@ struct alignas(64) ProblemDev {
   uint32_t conv_c, conv_kw;    // channels (multiple of 64), filter width
   uint32_t conv_wo, conv_ho;   // output width / height
   uint32_t conv_stride, conv_pad;
+  // epilogue of the _ex entry points: v = (alpha * scale[row]) * acc + beta * C + bias[row], D = act(v).  epi != 0 selects
+  // the epilogue code that applies it (also taken for beta != 0 with the transposed output, whose C is [n][m] like D);
+  // epi == 0 runs the alpha / beta code of the plain entry points, unchanged.
+  const float* scale;  // [m] or null
+  const float* bias;   // [m] or null
+  uint32_t act;        // SPFY_ACT_*
+  uint32_t epi;
 };
 
 struct LaunchParams {
@@ -140,6 +148,13 @@ __device__ __forceinline__ uint32_t rows_valid_of(uint32_t m, uint32_t mt) {
   return left >= (uint32_t)BM ? (uint32_t)BM : ((left + 15u) & ~15u);
 }
 
+
+// GELU, tanh form (torch's gelu(approximate="tanh")): one tanh.approx per value on the MUFU pipe
+__device__ __forceinline__ float gelu_tanh(float x) {
+  float t;
+  asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.7978845608028654f * fmaf(0.044715f * x, x * x, x)));
+  return 0.5f * x * (1.f + t);
+}
 
 // All three roles walk the same sequence of units: u = blockIdx.x, blockIdx.x + gridDim.x, ...
 // The walker keeps the unit's position inside its problem -- (n-tile, m-group) -> first m-tile and m-tiles of the unit --
@@ -218,7 +233,9 @@ struct UnitWalker {
 };
 
 // ------------------------------------------------------------------- kernel
-template <bool BF16, bool OPB_T>
+// EPI: some problem of the launch has an epilogue (ProblemDev::epi).  A launch without one compiles to the code the kernel
+// had before epilogues existed (152 registers instead of 168, measured 0.3-1 % faster on the ResNet-50 plans).
+template <bool BF16, bool OPB_T, bool EPI>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ LaunchParams L) {
   extern __shared__ uint8_t smem_raw[];
@@ -546,6 +563,10 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
     uint64_t ldc = 0;
     uint32_t pm = 0, pn = 0;
     float alpha = 1.f, beta = 0.f;
+    float alpha_t = 1.f;  // the factor the transposed staging loop applies: 1 once the epilogue has applied alpha
+    const float* scale = nullptr;
+    const float* bias = nullptr;
+    uint32_t act = 0, epi = 0;
     for (; W.valid(); W.next()) {
       const ProblemDev* P = W.current();
       if (W.changed) {
@@ -558,6 +579,10 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
         ldc = P->ldc;
         pm = P->m; pn = P->n;
         alpha = P->alpha; beta = P->beta;
+        if (EPI) {
+          scale = P->scale; bias = P->bias; act = P->act; epi = P->epi;
+        }
+        alpha_t = epi ? 1.f : alpha;
       }
       const uint32_t nt = W.nt, mt0 = W.mt0, g_count = W.g_count;
       for (uint32_t g = 0; g < g_count; ++g, ++job) {
@@ -591,17 +616,76 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
             __syncwarp();
             if (e == 0 && hh == 0) SPFY_TRACE(2, job, 3);
             const uint32_t grow = m0 + row_in_tile;
+            if (epi) {
+              // the epilogue, in place on the accumulators: v = (alpha * scale[row]) * acc + beta * C + bias[row], then
+              // the activation; the staging below only converts.  A missing bias adds -0, which leaves every value as it is.
+              const bool row_ok = grow < pm;
+              const float as = scale && row_ok ? alpha * scale[grow] : alpha;
+              const float bs = bias && row_ok ? bias[grow] : -0.f;
+              if (beta != 0.f && out_t) {
+                // C is [n][m] like D: the warp copies its (64 n x 32 m) box of C into its staging buffer -- the geometry
+                // of the store box, 64 contiguous bytes per n -- with 16-byte asynchronous copies that bypass the
+                // registers, and every lane then reads its own column of it, where the staging loop below writes the
+                // result.  (Halfword loads of C into registers spill at the 168 registers this CTA shape allows.)
+                const uint32_t mc = m0 + quarter * 32 + (lane & 3u) * 8;  // m % 8 == 0: these 8 m are all in or all out
+                const uint32_t r0 = lane >> 2, n_in = mc < pm ? pn - n0 : 0u;   // rows r0, r0 + 8, ... of the box
+                const uint16_t* src = Cptr + (size_t)(n0 + r0) * ldc + mc;
+                const uint32_t dst = sc + r0 * 64u + (lane & 3u) * 16u;
+#pragma unroll
+                for (uint32_t i = 0; i < 8; ++i, src += 8 * ldc)
+                  cp_async_16(dst + i * 512u, r0 + 8 * i < n_in ? src : Cptr, r0 + 8 * i < n_in);
+                cp_async_wait_all();
+                __syncwarp();
+#pragma unroll
+                for (int j = 0; j < 64; ++j) {
+                  const float c = unpack2<BF16>(ld_shared_u16(sc + (uint32_t)j * 64u + lane * 2u)).x;
+                  acc[j] = __float_as_uint(__fadd_rn(__fmaf_rn(beta, c, __fmul_rn(as, __uint_as_float(acc[j]))), bs));
+                }
+              } else if (beta != 0.f && row_ok) {
+                {
+#pragma unroll
+                  for (int q = 0; q < 8; ++q) {
+                    float v[8];
+#pragma unroll
+                    for (int x = 0; x < 8; ++x) v[x] = __fmul_rn(as, __uint_as_float(acc[q * 8 + x]));
+                    if (n0 + q * 8 < pn) {
+                      const uint4 cw = *reinterpret_cast<const uint4*>(Cptr + (size_t)grow * ldc + n0 + q * 8);
+                      const uint32_t cws[4] = {cw.x, cw.y, cw.z, cw.w};
+#pragma unroll
+                      for (int x = 0; x < 4; ++x) {
+                        const float2 f = unpack2<BF16>(cws[x]);
+                        v[2 * x] = __fmaf_rn(beta, f.x, v[2 * x]);
+                        v[2 * x + 1] = __fmaf_rn(beta, f.y, v[2 * x + 1]);
+                      }
+                    }
+#pragma unroll
+                    for (int x = 0; x < 8; ++x) acc[q * 8 + x] = __float_as_uint(__fadd_rn(v[x], bs));
+                  }
+                }
+              } else {
+#pragma unroll
+                for (int j = 0; j < 64; ++j) acc[j] = __float_as_uint(__fadd_rn(__fmul_rn(as, __uint_as_float(acc[j])), bs));
+              }
+              if (act == SPFY_ACT_RELU) {
+#pragma unroll
+                for (int j = 0; j < 64; ++j) acc[j] = __float_as_uint(fmaxf(__uint_as_float(acc[j]), 0.f));
+              } else if (act == SPFY_ACT_GELU_TANH) {
+#pragma unroll
+                for (int j = 0; j < 64; ++j) acc[j] = __float_as_uint(gelu_tanh(__uint_as_float(acc[j])));
+              }
+            }
             if (out_t) {
               // transposed output [n][m]: the staging buffer holds 64 rows (n) of 32 halfwords (my quarter's m), so a
-              // lane -- one m -- drops column j of its 64 into row j; beta == 0 by contract
+              // lane -- one m -- drops column j of its 64 into row j; C (beta != 0) only through the epilogue above
 #pragma unroll
               for (int j = 0; j < 32; ++j) {
-                const uint32_t w = pack2<BF16>(alpha * __uint_as_float(acc[2 * j]), alpha * __uint_as_float(acc[2 * j + 1]));
+                const uint32_t w = pack2<BF16>(alpha_t * __uint_as_float(acc[2 * j]), alpha_t * __uint_as_float(acc[2 * j + 1]));
                 st_shared_u16(sc + (uint32_t)(2 * j) * 64u + lane * 2u, w);
                 st_shared_u16(sc + (uint32_t)(2 * j + 1) * 64u + lane * 2u, w >> 16);
               }
-            } else if (alpha == 1.f && beta == 0.f) {
-              // the common case (the reference's defaults, spmma.hxx:32-33): convert and stage, nothing else.
+            } else if (epi || (alpha == 1.f && beta == 0.f)) {
+              // the common case (the reference's defaults, spmma.hxx:32-33), or values the epilogue has finished:
+              // convert and stage, nothing else.
               // Kept apart from the general path: predicated-off C loads / FMAs still cost issue slots, and
               // with two epilogue warps per scheduler the conversion loop is what bounds the small-K classes.
 #pragma unroll
@@ -715,6 +799,8 @@ struct HostProblem {
   float alpha, beta;
   const spfy_conv_desc* conv = nullptr;  // implicit GEMM: B is the NHWC activation tensor, never unfolded
   bool out_t = false;                    // D is written transposed: [n][m] row-major, pitch ldd >= m (SPFY_OUT_T)
+  spfy_epilogue epi{nullptr, nullptr, SPFY_ACT_NONE};
+  bool ex = false;                       // called through an _ex entry: beta != 0 allowed with out_t (C is then [n][m])
 };
 
 // the `opB` argument of the C ABI carries the output layout in bit 4 (SPFY_OUT_T)
@@ -747,6 +833,10 @@ int validate(int dtype, const HostProblem& h, const char* who) {
   if (dtype != SPFY_F16 && dtype != SPFY_BF16)
     return fail(SPFY_E_UNSUPPORTED, "%s: dtype %d (need F16/BF16)", who, dtype);
   if (h.opB != SPFY_OP_N && h.opB != SPFY_OP_T) return fail(SPFY_E_INVALID, "%s: bad opB %d", who, h.opB);
+  if (h.epi.act < SPFY_ACT_NONE || h.epi.act > SPFY_ACT_GELU_TANH)
+    return fail(SPFY_E_INVALID, "%s: bad epilogue activation %d", who, h.epi.act);
+  if ((uintptr_t)h.epi.scale % 4 || (uintptr_t)h.epi.bias % 4)
+    return fail(SPFY_E_INVALID, "%s: epilogue scale / bias must be 4-byte aligned", who);
   if (h.m == 0 || h.n == 0) return SPFY_OK;
   if (!h.comp_vals || !h.meta || !h.B || !h.D) return fail(SPFY_E_INVALID, "%s: null operand", who);
   if (h.beta != 0.f && !h.C) return fail(SPFY_E_INVALID, "%s: beta != 0 needs C", who);
@@ -754,12 +844,12 @@ int validate(int dtype, const HostProblem& h, const char* who) {
   if (h.m >= (1u << 31) || h.n >= (1u << 31) || h.k >= (1u << 31))
     return fail(SPFY_E_UNSUPPORTED, "%s: dimension too large", who);
   const size_t b_inner = h.opB == SPFY_OP_N ? h.n : h.k;
-  if (h.out_t && h.beta != 0.f)
+  if (h.out_t && h.beta != 0.f && !h.ex)
     return fail(SPFY_E_UNSUPPORTED, "%s: a transposed output (SPFY_OUT_T) needs beta == 0", who);
   // (a TMA store moves whole 16-byte pieces of a row: the contiguous dimension of the output is a multiple of 8 elements)
   if (h.out_t && h.m % 8)
     return fail(SPFY_E_UNSUPPORTED, "%s: a transposed output (SPFY_OUT_T) needs m %% 8 == 0 (m=%zu)", who, h.m);
-  if ((!h.conv && h.ldb < b_inner) || h.ldd < (h.out_t ? h.m : h.n) || (h.beta != 0.f && h.ldc < h.n))
+  if ((!h.conv && h.ldb < b_inner) || h.ldd < (h.out_t ? h.m : h.n) || (h.beta != 0.f && h.ldc < (h.out_t ? h.m : h.n)))
     return fail(SPFY_E_INVALID, "%s: leading dimension too small", who);
   // TMA contract == the reference's own fp16 contract (spmma.hxx:45-49): multiples of 8
   if ((!h.conv && h.ldb % 8) || h.ldd % 8 || (h.beta != 0.f && h.ldc % 8) || h.n % 8 || (h.opB == SPFY_OP_T && h.k % 8))
@@ -876,6 +966,11 @@ int fill_problem(ProblemDev* d, int dtype, const HostProblem& h, int cls) {
   d->split_nt = d->n_tiles;
   d->alpha = h.alpha;
   d->beta = h.beta;
+  d->scale = h.epi.scale;
+  d->bias = h.epi.bias;
+  d->act = (uint32_t)h.epi.act;
+  // an identity epilogue (no scale, no bias, no activation) runs the code of the plain entry points
+  d->epi = h.epi.scale || h.epi.bias || h.epi.act != SPFY_ACT_NONE || (h.out_t && h.beta != 0.f);
   // B is streamed once when one unit covers all of M; otherwise the other m-groups of the same
   // columns will want it from L2 shortly after
   d->hint_b = d->m_groups == 1 ? HINT_EVICT_FIRST : HINT_EVICT_NORMAL;
@@ -944,14 +1039,14 @@ uint32_t make_idesc(int dtype, int opB) {
          ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 }
 
-template <bool BF16, bool OPB_T>
+template <bool BF16, bool OPB_T, bool EPI>
 int launch_t(const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid, cudaStream_t s,
              bool overlap_previous) {
   static std::atomic<int> attr_set[64];
   int dev = 0;
   SPFY_CUDA_OK(cudaGetDevice(&dev));
   if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(spmma_kernel<BF16, OPB_T>,
+    SPFY_CUDA_OK(cudaFuncSetAttribute(spmma_kernel<BF16, OPB_T, EPI>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_set[dev & 63].store(1);
   }
@@ -967,19 +1062,27 @@ int launch_t(const ProblemDev& single, const LaunchParams& L, uint32_t smem, int
   attr.val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = &attr;
   cfg.numAttrs = overlap_previous ? 1 : 0;
-  SPFY_CUDA_OK(cudaLaunchKernelEx(&cfg, spmma_kernel<BF16, OPB_T>, single, L));
+  SPFY_CUDA_OK(cudaLaunchKernelEx(&cfg, spmma_kernel<BF16, OPB_T, EPI>, single, L));
   SPFY_LAUNCH_OK("spmma_kernel");
   return SPFY_OK;
 }
 
-// overlap_previous: the kernel launched just before on this stream is another launch of the same plan
-int launch(int dtype, int opB, const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid,
-           cudaStream_t s, bool overlap_previous = false) {
+template <bool EPI>
+int launch_e(int dtype, int opB, const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid,
+             cudaStream_t s, bool overlap_previous) {
   if (dtype == SPFY_BF16)
-    return opB == SPFY_OP_N ? launch_t<true, false>(single, L, smem, grid, s, overlap_previous)
-                            : launch_t<true, true>(single, L, smem, grid, s, overlap_previous);
-  return opB == SPFY_OP_N ? launch_t<false, false>(single, L, smem, grid, s, overlap_previous)
-                          : launch_t<false, true>(single, L, smem, grid, s, overlap_previous);
+    return opB == SPFY_OP_N ? launch_t<true, false, EPI>(single, L, smem, grid, s, overlap_previous)
+                            : launch_t<true, true, EPI>(single, L, smem, grid, s, overlap_previous);
+  return opB == SPFY_OP_N ? launch_t<false, false, EPI>(single, L, smem, grid, s, overlap_previous)
+                          : launch_t<false, true, EPI>(single, L, smem, grid, s, overlap_previous);
+}
+
+// overlap_previous: the kernel launched just before on this stream is another launch of the same plan;
+// epi: some problem of the launch has an epilogue
+int launch(int dtype, int opB, bool epi, const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid,
+           cudaStream_t s, bool overlap_previous = false) {
+  return epi ? launch_e<true>(dtype, opB, single, L, smem, grid, s, overlap_previous)
+             : launch_e<false>(dtype, opB, single, L, smem, grid, s, overlap_previous);
 }
 
 #ifdef SPFY_DEV_SWITCHES
@@ -991,7 +1094,7 @@ int launch_traced(const char* path, int dtype, int opB, const ProblemDev& d, Lau
   SPFY_CUDA_OK(cudaStreamSynchronize(s));
   memset(trace, 0, n * sizeof(long long));
   L.trace = trace;
-  int rc = launch(dtype, opB, d, L, smem, grid, s);
+  int rc = launch(dtype, opB, d.epi != 0, d, L, smem, grid, s);
   if (rc) return rc;
   SPFY_CUDA_OK(cudaStreamSynchronize(s));
   if (FILE* f = fopen(path, "w")) {
@@ -1023,8 +1126,8 @@ uint32_t res_meta_bytes(const ProblemDev& d) { return res_tiles(d) * res_rows(d)
 // a convolution layer as a GEMM problem: n and k follow from the descriptor, B is the NHWC activation tensor (opB = T:
 // a B stage is [128 positions][128 k], gathered by the im2col tensor map)
 int conv_problem(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals, const void* meta,
-                 const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd, bool out_t, const char* who,
-                 HostProblem* out) {
+                 const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd, bool out_t,
+                 const spfy_epilogue* epi, bool ex, const char* who, HostProblem* out) {
   if (!conv) return fail(SPFY_E_INVALID, "%s: null descriptor", who);
   const spfy_conv_desc& c = *conv;
   if (!c.batch || !c.h || !c.w || !c.c || !c.kh || !c.kw || !c.stride)
@@ -1039,6 +1142,8 @@ int conv_problem(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, c
   HostProblem h{SPFY_OP_T, m, n, k, comp_vals, meta, X, C, D, /*ldb*/ k, ldc, ldd, alpha, beta};
   h.conv = conv;
   h.out_t = out_t;
+  if (epi) h.epi = *epi;
+  h.ex = ex;
   *out = h;
   return validate(dtype, h, who);
 }
@@ -1053,6 +1158,7 @@ struct Plan {
     LaunchParams L;
     uint32_t smem;
     int grid;
+    bool epi;  // some problem of the launch has an epilogue
   };
   std::vector<Launch> launches;
 };
@@ -1061,10 +1167,14 @@ struct Plan {
 }  // namespace spfy
 
 void spfy::warm_spmma_kernels() {
-  touch_kernel(spmma_kernel<false, false>);
-  touch_kernel(spmma_kernel<false, true>);
-  touch_kernel(spmma_kernel<true, false>);
-  touch_kernel(spmma_kernel<true, true>);
+  touch_kernel(spmma_kernel<false, false, false>);
+  touch_kernel(spmma_kernel<false, true, false>);
+  touch_kernel(spmma_kernel<true, false, false>);
+  touch_kernel(spmma_kernel<true, true, false>);
+  touch_kernel(spmma_kernel<false, false, true>);
+  touch_kernel(spmma_kernel<false, true, true>);
+  touch_kernel(spmma_kernel<true, false, true>);
+  touch_kernel(spmma_kernel<true, true, true>);
   EncodeTiledFn enc;
   (void)get_encoder(&enc);
 }
@@ -1079,12 +1189,13 @@ int spfy_spmma_workspace_bytes(int dtype, size_t m, size_t n, size_t k, size_t* 
   return SPFY_OK;
 }
 
-int spfy_spmma(int dtype, int opB, size_t m, size_t n, size_t k, float alpha, const void* comp_vals,
-               const void* meta, const void* B, size_t ldb, float beta, const void* C, size_t ldc,
-               void* D, size_t ldd, void* workspace, size_t workspace_bytes, spfy_stream_t stream) {
-  (void)workspace; (void)workspace_bytes;
+static int spmma_impl(int dtype, int opB, size_t m, size_t n, size_t k, float alpha, const void* comp_vals,
+                      const void* meta, const void* B, size_t ldb, float beta, const void* C, size_t ldc, void* D,
+                      size_t ldd, const spfy_epilogue* epi, bool ex, spfy_stream_t stream) {
   HostProblem h{op_of(opB), m, n, k, comp_vals, meta, B, C, D, ldb, ldc, ldd, alpha, beta};
   h.out_t = out_t_of(opB);
+  if (epi) h.epi = *epi;
+  h.ex = ex;
   opB = h.opB;
   int rc = validate(dtype, h, "spmma");
   if (rc) return rc;
@@ -1116,29 +1227,52 @@ int spfy_spmma(int dtype, int opB, size_t m, size_t n, size_t k, float alpha, co
 #ifdef SPFY_DEV_SWITCHES
   if (const char* path = dev_switch("SPFY_SPMMA_TRACE")) return launch_traced(path, dtype, opB, d, L, smem, grid, (cudaStream_t)stream);
 #endif
-  return launch(dtype, opB, d, L, smem, grid, (cudaStream_t)stream);
+  return launch(dtype, opB, d.epi != 0, d, L, smem, grid, (cudaStream_t)stream);
+}
+
+int spfy_spmma(int dtype, int opB, size_t m, size_t n, size_t k, float alpha, const void* comp_vals,
+               const void* meta, const void* B, size_t ldb, float beta, const void* C, size_t ldc,
+               void* D, size_t ldd, void* workspace, size_t workspace_bytes, spfy_stream_t stream) {
+  (void)workspace; (void)workspace_bytes;
+  return spmma_impl(dtype, opB, m, n, k, alpha, comp_vals, meta, B, ldb, beta, C, ldc, D, ldd, nullptr, false, stream);
+}
+
+int spfy_spmma_ex(int dtype, int opB, size_t m, size_t n, size_t k, float alpha, const void* comp_vals,
+                  const void* meta, const void* B, size_t ldb, float beta, const void* C, size_t ldc,
+                  void* D, size_t ldd, void* workspace, size_t workspace_bytes, const spfy_epilogue* epi,
+                  spfy_stream_t stream) {
+  (void)workspace; (void)workspace_bytes;
+  return spmma_impl(dtype, opB, m, n, k, alpha, comp_vals, meta, B, ldb, beta, C, ldc, D, ldd, epi, true, stream);
 }
 
 static int spmma_conv_impl(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                            const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
-                           bool out_t, spfy_stream_t stream);
+                           bool out_t, const spfy_epilogue* epi, bool ex, spfy_stream_t stream);
 
 int spfy_spmma_conv(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                     const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
                     spfy_stream_t stream) {
-  return spmma_conv_impl(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, false, stream);
+  return spmma_conv_impl(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, false, nullptr, false, stream);
 }
 
 int spfy_spmma_conv_nhwc(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                          const void* meta, const void* X, void* Y, size_t ldy, spfy_stream_t stream) {
-  return spmma_conv_impl(dtype, conv, m, alpha, comp_vals, meta, X, 0.f, nullptr, 0, Y, ldy, true, stream);
+  return spmma_conv_impl(dtype, conv, m, alpha, comp_vals, meta, X, 0.f, nullptr, 0, Y, ldy, true, nullptr, false, stream);
+}
+
+int spfy_spmma_conv_ex(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
+                       const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
+                       int layout, const spfy_epilogue* epi, spfy_stream_t stream) {
+  if (layout != 0 && layout != SPFY_OUT_T) return fail(SPFY_E_INVALID, "spmma_conv_ex: bad output layout %d", layout);
+  return spmma_conv_impl(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, layout == SPFY_OUT_T, epi, true,
+                         stream);
 }
 
 static int spmma_conv_impl(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                            const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
-                           bool out_t, spfy_stream_t stream) {
+                           bool out_t, const spfy_epilogue* epi, bool ex, spfy_stream_t stream) {
   HostProblem h;
-  int rc = conv_problem(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, out_t, "spmma_conv", &h);
+  int rc = conv_problem(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, out_t, epi, ex, "spmma_conv", &h);
   if (rc) return rc;
   const size_t n = h.n;
   if (m == 0 || n == 0) return SPFY_OK;
@@ -1165,7 +1299,7 @@ static int spmma_conv_impl(int dtype, const spfy_conv_desc* conv, size_t m, floa
 #ifdef SPFY_DEV_SWITCHES
   if (const char* path = dev_switch("SPFY_SPMMA_TRACE")) return launch_traced(path, dtype, SPFY_OP_T, d, L, smem, grid, (cudaStream_t)stream);
 #endif
-  return launch(dtype, SPFY_OP_T, d, L, smem, grid, (cudaStream_t)stream);
+  return launch(dtype, SPFY_OP_T, d.epi != 0, d, L, smem, grid, (cudaStream_t)stream);
 }
 
 static void plan_free(Plan* plan) {
@@ -1173,17 +1307,23 @@ static void plan_free(Plan* plan) {
   if (plan->d_rep) cudaFree(plan->d_rep);
   delete plan;
 }
-static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs, size_t count,
-                            size_t n_rep, void* const* rep_d, spfy_spmma_plan_t* out);
+static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs,
+                            const spfy_epilogue* const* epis, bool ex, size_t count, size_t n_rep, void* const* rep_d,
+                            spfy_spmma_plan_t* out);
 
 int spfy_spmma_plan_create(int dtype, const spfy_spmma_problem* problems, size_t count,
                            spfy_spmma_plan_t* out) {
-  return plan_create_impl(dtype, problems, nullptr, count, 0, nullptr, out);
+  return plan_create_impl(dtype, problems, nullptr, nullptr, false, count, 0, nullptr, out);
 }
 
 int spfy_spmma_plan_create_conv(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs,
                                 size_t count, spfy_spmma_plan_t* out) {
-  return plan_create_impl(dtype, problems, convs, count, 0, nullptr, out);
+  return plan_create_impl(dtype, problems, convs, nullptr, false, count, 0, nullptr, out);
+}
+
+int spfy_spmma_plan_create_ex(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs,
+                              const spfy_epilogue* const* epilogues, size_t count, spfy_spmma_plan_t* out) {
+  return plan_create_impl(dtype, problems, convs, epilogues, true, count, 0, nullptr, out);
 }
 
 int spfy_spmma_plan_create_replicated(int dtype, const spfy_spmma_problem* problems, size_t count, size_t replicas,
@@ -1194,22 +1334,26 @@ int spfy_spmma_plan_create_replicated(int dtype, const spfy_spmma_problem* probl
     if (problems && problems[i / replicas].m && problems[i / replicas].n && (!replica_d[i] || (uintptr_t)replica_d[i] % 16))
       return fail(SPFY_E_INVALID, "spmma_plan_create_replicated: replica %zu of problem %zu is null or not 16-byte aligned",
                   i % replicas, i / replicas);
-  return plan_create_impl(dtype, problems, nullptr, count, replicas, replica_d, out);
+  return plan_create_impl(dtype, problems, nullptr, nullptr, false, count, replicas, replica_d, out);
 }
 
 // problem i of a plan as the host sees it (a convolution layer when convs[i] is given: B = X, n / k / ldb / opB from the
 // descriptor, the SPFY_OUT_T bit of opB still selects the NHWC output)
-static int plan_problem(int dtype, const spfy_spmma_problem& q, const spfy_conv_desc* conv, HostProblem* h) {
+static int plan_problem(int dtype, const spfy_spmma_problem& q, const spfy_conv_desc* conv, const spfy_epilogue* epi, bool ex,
+                        HostProblem* h) {
   if (conv)
     return conv_problem(dtype, conv, q.m, q.alpha, q.comp_vals, q.meta, q.B, q.beta, q.C, q.ldc, q.D, q.ldd, out_t_of(q.opB),
-                        "spmma_plan_create", h);
+                        epi, ex, "spmma_plan_create", h);
   *h = HostProblem{op_of(q.opB), q.m, q.n, q.k, q.comp_vals, q.meta, q.B, q.C, q.D, q.ldb, q.ldc, q.ldd, q.alpha, q.beta};
   h->out_t = out_t_of(q.opB);
+  if (epi) h->epi = *epi;
+  h->ex = ex;
   return validate(dtype, *h, "spmma_plan_create");
 }
 
-static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs, size_t count,
-                            size_t n_rep, void* const* rep_d, spfy_spmma_plan_t* out) {
+static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs,
+                            const spfy_epilogue* const* epis, bool ex, size_t count, size_t n_rep, void* const* rep_d,
+                            spfy_spmma_plan_t* out) {
   if (!out) return fail(SPFY_E_INVALID, "spmma_plan_create: null plan pointer");
   *out = nullptr;
   if (count && !problems) return fail(SPFY_E_INVALID, "spmma_plan_create: null problem list");
@@ -1237,6 +1381,7 @@ static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const
       Plan::Launch ln;
       memset(&ln.L, 0, sizeof(ln.L));
       ln.opB = opB;
+      ln.epi = false;
       ln.first = (uint32_t)table.size();
       ln.count = 0;
       uint32_t units = 0, res_vals = 0, res_meta = 0;
@@ -1248,7 +1393,7 @@ static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const
         const spfy_conv_desc* cv = convs ? convs[i] : nullptr;
         if ((cv ? SPFY_OP_T : op_of(q.opB)) != opB) continue;
         HostProblem h;
-        rc = plan_problem(dtype, q, cv, &h);
+        rc = plan_problem(dtype, q, cv, epis ? epis[i] : nullptr, ex, &h);
         if (rc) {
           plan_free(plan);
           return rc;
@@ -1266,7 +1411,7 @@ static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const
       });
       for (size_t i : members) {
         HostProblem h;
-        (void)plan_problem(dtype, problems[i], convs ? convs[i] : nullptr, &h);  // validated above
+        (void)plan_problem(dtype, problems[i], convs ? convs[i] : nullptr, epis ? epis[i] : nullptr, ex, &h);  // validated above
         ProblemDev d;
         rc = fill_problem(&d, dtype, h, cls);
         if (rc) {
@@ -1295,6 +1440,7 @@ static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const
         }
         if (d.resident && res_values_bytes(d) > res_vals) res_vals = res_values_bytes(d);
         if (d.resident && res_meta_bytes(d) > res_meta) res_meta = res_meta_bytes(d);
+        ln.epi = ln.epi || d.epi;
         table.push_back(d);
         ++ln.count;
       }
@@ -1335,7 +1481,7 @@ int spfy_spmma_plan_run(spfy_spmma_plan_t p, spfy_stream_t stream) {
   static const bool serial = dev_switch("SPFY_SPMMA_NO_OVERLAP") != nullptr;
   bool first = true;
   for (const auto& ln : plan->launches) {
-    int rc = launch(plan->dtype, ln.opB, dummy, ln.L, ln.smem, ln.grid, (cudaStream_t)stream, !first && !serial);
+    int rc = launch(plan->dtype, ln.opB, ln.epi, dummy, ln.L, ln.smem, ln.grid, (cudaStream_t)stream, !first && !serial);
     if (rc) return rc;
     first = false;
   }
@@ -1352,7 +1498,7 @@ int spfy_spmma_plan_run_launch(spfy_spmma_plan_t p, int index, spfy_stream_t str
   ProblemDev dummy;
   memset(&dummy, 0, sizeof(dummy));
   const auto& ln = plan->launches[index];
-  return launch(plan->dtype, ln.opB, dummy, ln.L, ln.smem, ln.grid, (cudaStream_t)stream);
+  return launch(plan->dtype, ln.opB, ln.epi, dummy, ln.L, ln.smem, ln.grid, (cudaStream_t)stream);
 }
 
 int spfy_spmma_plan_launch_info(spfy_spmma_plan_t p, int index, int* problems, int* units, int* stages,

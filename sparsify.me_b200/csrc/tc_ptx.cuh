@@ -302,6 +302,17 @@ __device__ __forceinline__ uint32_t ld_shared_u32(uint32_t addr) {
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
   return v;
 }
+// 16-byte global -> shared copy that bypasses the registers (zeros when !valid; src is not read then); complete for the
+// issuing thread after cp_async_wait_all
+__device__ __forceinline__ void cp_async_16(uint32_t dst, const void* src, bool valid) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(valid ? 16u : 0u) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+__device__ __forceinline__ uint32_t ld_shared_u16(uint32_t addr) {
+  uint16_t v;
+  asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr));
+  return v;
+}
 __device__ __forceinline__ uint4 ld_shared_v4(uint32_t addr) {
   uint4 v;
   asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));

@@ -169,11 +169,44 @@ def unpack_compressed(blob, device):
                         rows.value, cols.value, tdt, layout.value)
 
 
+_ACTS = {"none": capi.ACT_NONE, "relu": capi.ACT_RELU, "gelu_tanh": capi.ACT_GELU_TANH}
+
+
+@dataclass
+class Epilogue:
+    """What the spmma epilogue applies before the output is written (spfy_epilogue, cusparseLt's ALPHA_VECTOR_SCALING /
+    BIAS_POINTER / ACTIVATION_*): per output element (i, j), in fp32 and rounded to 16 bit once,
+        v = (alpha * scale[i]) * acc + beta * C + bias[i],   D = act(v)
+    i is the output row: the output channel of a convolution, the output feature of a Linear layer.  `scale` / `bias`:
+    fp32 CUDA tensors of m elements (None: 1 / 0); act: "none", "relu" or "gelu_tanh" (torch's gelu(approximate="tanh")).
+    fold_batchnorm turns an inference batch norm into (scale, bias)."""
+    scale: torch.Tensor = None
+    bias: torch.Tensor = None
+    act: str = "none"
+
+    def _c(self, m):
+        if self.act not in _ACTS:
+            raise ValueError(f"Epilogue: act must be one of {sorted(_ACTS)}, got {self.act!r}")
+        for name, t in (("scale", self.scale), ("bias", self.bias)):
+            if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < m):
+                raise ValueError(f"Epilogue: {name} must be a contiguous fp32 tensor of at least {m} elements")
+        return capi.Epilogue(_ptr(self.scale), _ptr(self.bias), _ACTS[self.act])
+
+
+def fold_batchnorm(gamma, beta, mean, var, eps=1e-5):
+    """An inference batch norm, y = gamma * (x - mean) / sqrt(var + eps) + beta, as the (scale, bias) of an Epilogue
+    (fp32 tensors on the device of `gamma`)."""
+    scale = gamma.float() / torch.sqrt(var.float() + eps)
+    return scale.contiguous(), (beta.float() - mean.float() * scale).contiguous()
+
+
 class SpmmaPlan:
     """spfy_spmma_plan_*: a list of independent D_i = alpha_i * A_i(2:4) * op(B_i) + beta_i * C_i executed
     by one persistent launch per ring-geometry class present (tensor maps + tile schedule built once, like
     cusparseLtMatmulPlanInit at spmma.hxx:79).  `problems`: dicts with comp, b, out and optional c, alpha,
-    beta, op_b, out_t (out is then [n, m], the transposed result; beta must be 0).  The plan keeps the tensors alive.
+    beta, op_b, out_t (out is then [n, m], the transposed result; beta must be 0 unless the plan has epilogues) and
+    epilogue (an Epilogue: any problem with one makes the plan go through spfy_spmma_plan_create_ex, same launches).
+    The plan keeps the tensors alive.
     Optional `replicas` per problem: device addresses (ints) of further copies of `out` (same shape and row pitch) that
     the epilogue stores every tile to as well -- e.g. the slab of this rank in the gather arena of every peer GPU
     (spfy_spmma_plan_create_replicated: the fused output gather); every problem must name the same number of them.
@@ -188,6 +221,9 @@ class SpmmaPlan:
         convs = (capi.ConvDesc * max(n, 1))()
         conv_ptrs = (ctypes.c_void_p * max(n, 1))()
         any_conv = False
+        epis = (capi.Epilogue * max(n, 1))()
+        epi_ptrs = (ctypes.c_void_p * max(n, 1))()
+        any_epi = False
         dtype = None
         for i, q in enumerate(problems):
             comp, b, out = q["comp"], q["b"], q["out"]
@@ -213,15 +249,25 @@ class SpmmaPlan:
                 nn = b.shape[1] if op_b == capi.OP_N else b.shape[0]
             if q.get("out_t"):  # `out` is [n, m]: the transposed result
                 op_b |= capi.OUT_T
+            if q.get("epilogue") is not None:
+                epis[i] = q["epilogue"]._c(comp.rows)
+                epi_ptrs[i] = ctypes.addressof(epis[i])
+                any_epi = True
             arr[i] = capi.SpmmaProblem(op_b, comp.rows, nn, comp.cols, comp.vals.data_ptr(), comp.meta.data_ptr(),
                                        b.data_ptr(), ldb, c.data_ptr() if c is not None else None,
-                                       c.stride(0) if c is not None else 0, out.data_ptr(), ldd,
+                                       c.stride(-2) if c is not None else 0, out.data_ptr(), ldd,
                                        float(q.get("alpha", 1.0)), float(q.get("beta", 0.0)))
         self._h = ctypes.c_void_p()
         nrep = len(problems[0].get("replicas", ())) if n else 0
         if any(len(q.get("replicas", ())) != nrep for q in problems):
             raise ValueError("SpmmaPlan: every problem needs the same number of replicas")
-        if any_conv:
+        if any_epi:
+            if nrep:
+                raise ValueError("SpmmaPlan: replicas and epilogues cannot be combined")
+            capi.spfy_spmma_plan_create_ex(_DT[dtype], ctypes.cast(arr, ctypes.c_void_p),
+                                           ctypes.cast(conv_ptrs, ctypes.c_void_p) if any_conv else None,
+                                           ctypes.cast(epi_ptrs, ctypes.c_void_p), n, ctypes.byref(self._h))
+        elif any_conv:
             if nrep:
                 raise ValueError("SpmmaPlan: replicas and convolution problems cannot be combined")
             capi.spfy_spmma_plan_create_conv(_DT[dtype], ctypes.cast(arr, ctypes.c_void_p), ctypes.cast(conv_ptrs, ctypes.c_void_p),
@@ -259,10 +305,13 @@ class SpmmaPlan:
 
 
 # ----------------------------------------------------------------------------- A4
-def spmma_compressed(comp, b, c=None, out=None, alpha=1.0, beta=0.0, op_b=capi.OP_N, out_t=False):
+def spmma_compressed(comp, b, c=None, out=None, alpha=1.0, beta=0.0, op_b=capi.OP_N, out_t=False, epilogue=None):
     """D = alpha * A(2:4) * op(B) + beta * C on tcgen05.mma.sp (cusparseLtMatmul, spmma.hxx:106-114).
     All dense operands row-major.  Returns D (== out, or a new tensor); out_t: D is [n, m], the transposed result
-    (SPFY_OUT_T: NHWC for a convolution layer; beta must be 0)."""
+    (SPFY_OUT_T: NHWC for a convolution layer; beta must be 0 without an epilogue).
+    epilogue: an Epilogue (per-row scale / bias, activation) applied before D is written (spfy_spmma_ex); with one,
+    out_t also takes beta * C with C as [n, m] like D.  A Linear layer y = act(x W^T + b) is
+    spmma_compressed(comp(W), x, op_b=OP_T, out_t=True, epilogue=Epilogue(bias=b, act=...))."""
     assert comp.layout == capi.LAYOUT_SM100
     m, k = comp.rows, comp.cols
     n = b.shape[1] if op_b == capi.OP_N else b.shape[0]
@@ -271,9 +320,15 @@ def spmma_compressed(comp, b, c=None, out=None, alpha=1.0, beta=0.0, op_b=capi.O
         out = torch.empty((n, m) if out_t else (m, n), dtype=comp.dtype, device=b.device)
     if out_t:
         op_b |= capi.OUT_T
-    capi.spfy_spmma(_DT[comp.dtype], op_b, m, n, k, float(alpha), _ptr(comp.vals), _ptr(comp.meta),
-                    _ptr(b), b.stride(0), float(beta), _ptr(c), c.stride(0) if c is not None else 0,
-                    _ptr(out), out.stride(0), None, 0, _stream())
+    if epilogue is None:
+        capi.spfy_spmma(_DT[comp.dtype], op_b, m, n, k, float(alpha), _ptr(comp.vals), _ptr(comp.meta),
+                        _ptr(b), b.stride(0), float(beta), _ptr(c), c.stride(0) if c is not None else 0,
+                        _ptr(out), out.stride(0), None, 0, _stream())
+    else:
+        epi = epilogue._c(m)
+        capi.spfy_spmma_ex(_DT[comp.dtype], op_b, m, n, k, float(alpha), _ptr(comp.vals), _ptr(comp.meta),
+                           _ptr(b), b.stride(0), float(beta), _ptr(c), c.stride(0) if c is not None else 0,
+                           _ptr(out), out.stride(0), None, 0, ctypes.byref(epi), _stream())
     return out
 
 
@@ -285,10 +340,11 @@ def permute_conv_weights(w, c, kh, kw):
     return out
 
 
-def spmma_conv(comp, x, kh, kw, stride=1, pad=0, c=None, out=None, alpha=1.0, beta=0.0):
+def spmma_conv(comp, x, kh, kw, stride=1, pad=0, c=None, out=None, alpha=1.0, beta=0.0, epilogue=None):
     """Implicit GEMM (spfy_spmma_conv): D[m, batch*ho*wo] = alpha * A(2:4) * im2col(x) + beta * C with x the NHWC
     activation tensor [batch, h, w, ch] -- the unfolded K x N operand of datasets/get_shapes.py:29-41 is never built.
-    `comp`: compressed weights whose K is ordered (kh, kw, ch) (permute_conv_weights before prune24)."""
+    `comp`: compressed weights whose K is ordered (kh, kw, ch) (permute_conv_weights before prune24).
+    epilogue: an Epilogue applied before D is written (spfy_spmma_conv_ex)."""
     assert x.dim() == 4 and x.is_contiguous()
     nb, h, w, ch = x.shape
     ho, wo = (h + 2 * pad - kh) // stride + 1, (w + 2 * pad - kw) // stride + 1
@@ -297,15 +353,23 @@ def spmma_conv(comp, x, kh, kw, stride=1, pad=0, c=None, out=None, alpha=1.0, be
     if out is None:
         out = torch.empty(comp.rows, n, dtype=comp.dtype, device=x.device)
     desc = capi.ConvDesc(nb, h, w, ch, kh, kw, stride, pad)
-    capi.spfy_spmma_conv(_DT[comp.dtype], ctypes.byref(desc), comp.rows, float(alpha), _ptr(comp.vals), _ptr(comp.meta),
-                         _ptr(x), float(beta), _ptr(c), c.stride(0) if c is not None else 0, _ptr(out), out.stride(0),
-                         _stream())
+    if epilogue is None:
+        capi.spfy_spmma_conv(_DT[comp.dtype], ctypes.byref(desc), comp.rows, float(alpha), _ptr(comp.vals),
+                             _ptr(comp.meta), _ptr(x), float(beta), _ptr(c), c.stride(0) if c is not None else 0, _ptr(out),
+                             out.stride(0), _stream())
+    else:
+        epi = epilogue._c(comp.rows)
+        capi.spfy_spmma_conv_ex(_DT[comp.dtype], ctypes.byref(desc), comp.rows, float(alpha), _ptr(comp.vals),
+                                _ptr(comp.meta), _ptr(x), float(beta), _ptr(c), c.stride(0) if c is not None else 0,
+                                _ptr(out), out.stride(0), 0, ctypes.byref(epi), _stream())
     return out
 
 
-def spmma_conv_nhwc(comp, x, kh, kw, stride=1, pad=0, out=None, alpha=1.0):
+def spmma_conv_nhwc(comp, x, kh, kw, stride=1, pad=0, out=None, alpha=1.0, c=None, beta=0.0, epilogue=None):
     """spfy_spmma_conv_nhwc: the same implicit GEMM with the result in NHWC, [batch, ho, wo, m] -- the `x` of the next
-    layer, so a chain of convolutions never transposes or unfolds anything."""
+    layer, so a chain of convolutions never transposes or unfolds anything.
+    epilogue (an Epilogue), c / beta (beta * C with C in NHWC like the result, e.g. the shortcut of a residual block; `c`
+    may be `out`) go through spfy_spmma_conv_ex: conv + batch norm + shortcut + ReLU in one pass over the output."""
     assert x.dim() == 4 and x.is_contiguous()
     nb, h, w, ch = x.shape
     ho, wo = (h + 2 * pad - kh) // stride + 1, (w + 2 * pad - kw) // stride + 1
@@ -314,8 +378,17 @@ def spmma_conv_nhwc(comp, x, kh, kw, stride=1, pad=0, out=None, alpha=1.0):
         out = torch.empty(nb, ho, wo, comp.rows, dtype=comp.dtype, device=x.device)
     assert out.is_contiguous() and out.numel() == nb * ho * wo * comp.rows
     desc = capi.ConvDesc(nb, h, w, ch, kh, kw, stride, pad)
-    capi.spfy_spmma_conv_nhwc(_DT[comp.dtype], ctypes.byref(desc), comp.rows, float(alpha), _ptr(comp.vals),
-                              _ptr(comp.meta), _ptr(x), _ptr(out), comp.rows, _stream())
+    if epilogue is None and c is None and beta == 0.0:
+        capi.spfy_spmma_conv_nhwc(_DT[comp.dtype], ctypes.byref(desc), comp.rows, float(alpha), _ptr(comp.vals),
+                                  _ptr(comp.meta), _ptr(x), _ptr(out), comp.rows, _stream())
+        return out
+    if c is not None:
+        assert c.shape[-1] == comp.rows and c.numel() == out.numel()
+        c = c if c.dim() == 2 else c.view(-1, comp.rows)
+    epi = (epilogue or Epilogue())._c(comp.rows)
+    capi.spfy_spmma_conv_ex(_DT[comp.dtype], ctypes.byref(desc), comp.rows, float(alpha), _ptr(comp.vals), _ptr(comp.meta),
+                            _ptr(x), float(beta), _ptr(c), c.stride(0) if c is not None else 0, _ptr(out), comp.rows,
+                            capi.OUT_T, ctypes.byref(epi), _stream())
     return out
 
 
