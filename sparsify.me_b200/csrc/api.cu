@@ -4,13 +4,6 @@
 namespace spfy {
 namespace {
 
-template <typename S, typename D>
-__device__ __forceinline__ D cvt(S v);
-template <> __device__ __forceinline__ __half cvt<float, __half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 cvt<float, __nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-template <> __device__ __forceinline__ float cvt<__half, float>(__half v) { return __half2float(v); }
-template <> __device__ __forceinline__ float cvt<__nv_bfloat16, float>(__nv_bfloat16 v) { return __bfloat162float(v); }
-
 // streaming element-wise conversion: 8 elements per thread per trip when both sides are 16-byte
 // aligned, scalar otherwise / for the tail
 template <typename S, typename D>
@@ -31,7 +24,7 @@ convert_kernel(const S* __restrict__ src, D* __restrict__ dst, size_t n, int vec
         *reinterpret_cast<uint4*>(in) = *reinterpret_cast<const uint4*>(src + c * 8);
       }
 #pragma unroll
-      for (int i = 0; i < 8; ++i) out[i] = cvt<S, D>(in[i]);
+      for (int i = 0; i < 8; ++i) out[i] = from_f32<D>(to_f32(in[i]));
       if (sizeof(D) == 4) {
         *reinterpret_cast<uint4*>(dst + c * 8) = *reinterpret_cast<uint4*>(out);
         *reinterpret_cast<uint4*>(dst + c * 8 + 4) = *reinterpret_cast<uint4*>(out + 4);
@@ -41,20 +34,16 @@ convert_kernel(const S* __restrict__ src, D* __restrict__ dst, size_t n, int vec
     }
     done = chunks * 8;
   }
-  for (size_t i = done + tid; i < n; i += nthreads) dst[i] = cvt<S, D>(src[i]);
+  for (size_t i = done + tid; i < n; i += nthreads) dst[i] = from_f32<D>(to_f32(src[i]));
 }
 
 template <typename S, typename D>
 int launch_convert(const void* src, void* dst, size_t n, cudaStream_t s) {
-  DeviceInfo di;
-  int rc = device_info(&di);
+  int grid = 1;
+  int rc = capped_grid(ceil_div(ceil_div(n, 8), 256), 8, &grid);
   if (rc) return rc;
-  size_t blocks = ceil_div(ceil_div(n, 8), 256);
-  const size_t cap = (size_t)di.sm_count * 8;
-  if (blocks > cap) blocks = cap;
-  if (!blocks) blocks = 1;
   const int vec = ((uintptr_t)src % 16 == 0) && ((uintptr_t)dst % 16 == 0);
-  convert_kernel<S, D><<<(unsigned)blocks, 256, 0, s>>>((const S*)src, (D*)dst, n, vec);
+  convert_kernel<S, D><<<grid, 256, 0, s>>>((const S*)src, (D*)dst, n, vec);
   SPFY_LAUNCH_OK("convert_kernel");
   return SPFY_OK;
 }
@@ -83,13 +72,11 @@ int spfy_permute_conv_weights(const void* in, void* out, size_t m, size_t c, siz
   if (!in || !out) return fail(SPFY_E_INVALID, "permute_conv_weights: null pointer");
   if (in == out) return fail(SPFY_E_INVALID, "permute_conv_weights: in place is not supported");
   if (c >= (1ull << 31) || kh * kw >= (1ull << 31)) return fail(SPFY_E_UNSUPPORTED, "permute_conv_weights: too large");
-  DeviceInfo di;
-  int rc = device_info(&di);
+  int grid = 1;
+  int rc = capped_grid(ceil_div(m * c * kh * kw, 256), 8, &grid);
   if (rc) return rc;
-  size_t blocks = ceil_div(m * c * kh * kw, 256);
-  if (blocks > (size_t)di.sm_count * 8) blocks = (size_t)di.sm_count * 8;
-  permute_conv_weights_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((const uint16_t*)in, (uint16_t*)out, m,
-                                                                                  (uint32_t)c, (uint32_t)(kh * kw));
+  permute_conv_weights_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const uint16_t*)in, (uint16_t*)out, m, (uint32_t)c,
+                                                                      (uint32_t)(kh * kw));
   SPFY_LAUNCH_OK("permute_conv_weights_kernel");
   return SPFY_OK;
 }

@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cstdarg>
 #include <cstdint>
@@ -89,6 +90,47 @@ inline int device_info(DeviceInfo* out) {
   *out = cache[dev];
   return SPFY_OK;
 }
+
+// the tcgen05 / TMA kernels run on sm_100a only; `di` is filled for the caller
+inline int require_sm100(const char* who, DeviceInfo* di) {
+  int rc = device_info(di);
+  if (rc) return rc;
+  if (di->cc_major != 10)
+    return fail(SPFY_E_UNSUPPORTED, "%s: needs an sm_100a device, found sm_%d%d", who, di->cc_major, di->cc_minor);
+  return SPFY_OK;
+}
+
+// grid of a grid-stride kernel: `blocks`, but at most `blocks_per_sm` per SM and at least one
+inline int capped_grid(size_t blocks, int blocks_per_sm, int* grid) {
+  DeviceInfo di;
+  int rc = device_info(&di);
+  if (rc) return rc;
+  *grid = (int)std::max<size_t>(1, std::min(blocks, (size_t)di.sm_count * blocks_per_sm));
+  return SPFY_OK;
+}
+
+// Raise the dynamic shared-memory limit of `Kernel` to `bytes`: once per device, and again when a call asks for more.
+// (Keyed on the kernel itself: different instances of one kernel template share a function type.)
+template <auto Kernel>
+inline int allow_dynamic_smem(size_t bytes) {
+  static std::atomic<size_t> set[64];
+  int dev = 0;
+  SPFY_CUDA_OK(cudaGetDevice(&dev));
+  if (set[dev & 63].load() < bytes) {
+    SPFY_CUDA_OK(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    set[dev & 63].store(bytes);
+  }
+  return SPFY_OK;
+}
+
+// ---- element conversion on the device: 16-bit and fp32 to fp32, and back with round-to-nearest-even
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T> __device__ __forceinline__ T from_f32(float v);
+template <> __device__ __forceinline__ float from_f32<float>(float v) { return v; }
+template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
 // CUDA loads device code lazily, kernel by kernel, at first use (tens of milliseconds for the big ones).
 // Each translation unit lists its kernels here so that spfy_init() can pay that once, outside anybody's timers.

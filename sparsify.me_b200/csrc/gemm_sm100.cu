@@ -143,14 +143,6 @@ struct OutT { using type = float; };
 template <> struct OutT<KIND_F16> { using type = __half; };
 template <> struct OutT<KIND_BF16> { using type = __nv_bfloat16; };
 
-template <int KIND> __device__ __forceinline__ float out_to_f32(typename OutT<KIND>::type v);
-template <> __device__ __forceinline__ float out_to_f32<KIND_F16>(__half v) { return __half2float(v); }
-template <> __device__ __forceinline__ float out_to_f32<KIND_BF16>(__nv_bfloat16 v) { return __bfloat162float(v); }
-template <> __device__ __forceinline__ float out_to_f32<KIND_F32>(float v) { return v; }
-template <int KIND> __device__ __forceinline__ typename OutT<KIND>::type f32_to_out(float v);
-template <> __device__ __forceinline__ __half f32_to_out<KIND_F16>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 f32_to_out<KIND_BF16>(float v) { return __float2bfloat16_rn(v); }
-template <> __device__ __forceinline__ float f32_to_out<KIND_F32>(float v) { return v; }
 
 // Epilogue role (4 warps: TMEM lane quarter = warp & 3), shared by the two kernels: drains accumulator slot
 // job % slots (slot_cols columns apart) of every unit the CTA walks.
@@ -219,8 +211,8 @@ __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base,
         for (uint32_t j = 0; j < 16; ++j)
           if (j < ncols) {
             float v = alpha * __uint_as_float(acc[j]);
-            if (beta != 0.f) v += beta * out_to_f32<KIND>(dst[(size_t)j * ldc]);
-            dst[(size_t)j * ldc] = f32_to_out<KIND>(v);
+            if (beta != 0.f) v += beta * to_f32(dst[(size_t)j * ldc]);
+            dst[(size_t)j * ldc] = from_f32<out_t>(v);
           }
       } else {
         // element (row, col) at col + row*ldc: the thread owns 16 consecutive elements
@@ -236,12 +228,12 @@ __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base,
               const uint4 old = *reinterpret_cast<const uint4*>(dst + q * VEC);
               const out_t* o = reinterpret_cast<const out_t*>(&old);
 #pragma unroll
-              for (uint32_t x = 0; x < VEC; ++x) v[x] += beta * out_to_f32<KIND>(o[x]);
+              for (uint32_t x = 0; x < VEC; ++x) v[x] += beta * to_f32(o[x]);
             }
             uint4 w;
             out_t* wo = reinterpret_cast<out_t*>(&w);
 #pragma unroll
-            for (uint32_t x = 0; x < VEC; ++x) wo[x] = f32_to_out<KIND>(v[x]);
+            for (uint32_t x = 0; x < VEC; ++x) wo[x] = from_f32<out_t>(v[x]);
             *reinterpret_cast<uint4*>(dst + q * VEC) = w;
           }
         } else {
@@ -249,8 +241,8 @@ __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base,
           for (uint32_t j = 0; j < 16; ++j)
             if (j < ncols) {
               float v = alpha * __uint_as_float(acc[j]);
-              if (beta != 0.f) v += beta * out_to_f32<KIND>(dst[j]);
-              dst[j] = f32_to_out<KIND>(v);
+              if (beta != 0.f) v += beta * to_f32(dst[j]);
+              dst[j] = from_f32<out_t>(v);
             }
         }
       }
@@ -990,10 +982,6 @@ repack_kernel(const T* __restrict__ src, size_t ld, size_t stride, T* __restrict
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                             const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                             CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 size_t elem_bytes(int dtype) { return dtype == SPFY_F32 ? 4 : 2; }
 
 // One operand as the kernel sees it: extent `mn` x `k`, element (i, kk) at (mn_major ? i + kk*ld : kk + i*ld)
@@ -1023,10 +1011,6 @@ size_t repack_bytes(int dtype, const OperandView& v, size_t nb) {
 
 int make_operand_map(CUtensorMap* map, int dtype, const OperandView& v, size_t nb, uint32_t box_rows,
                      CUtensorMapSwizzle swizzle, uint32_t mn_box_k = 0) {
-  EncodeTiledFn enc0;
-  int rc = get_encoder(&enc0);
-  if (rc) return rc;
-  EncodeFn enc = (EncodeFn)enc0;
   const size_t es = elem_bytes(dtype);
   const uint32_t per_row = (uint32_t)(GM_ROW_BYTES / es);  // elements in 128 bytes
   const size_t inner = v.mn_major ? v.mn : v.k, outer = v.mn_major ? v.k : v.mn;
@@ -1036,16 +1020,7 @@ int make_operand_map(CUtensorMap* map, int dtype, const OperandView& v, size_t n
   cuuint64_t strides[2] = {v.ld * es, bstride};
   // K-major: box = 128 bytes of K x box_rows rows; MN-major: 128 bytes of MN x `per_row` k-rows (one group)
   cuuint32_t box[3] = {per_row, v.mn_major ? (mn_box_k ? mn_box_k : per_row) : box_rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  const CUtensorMapDataType dt = dtype == SPFY_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
-                                 : dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-                                                      : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  CUresult r = enc(map, dt, 3, const_cast<void*>(v.base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS)
-    return fail(SPFY_E_CUDA, "tc_gemm: cuTensorMapEncodeTiled failed (%d): inner %zu outer %zu ld %zu batches %zu", (int)r,
-                inner, outer, v.ld, nb);
-  return SPFY_OK;
+  return encode_tiled(map, dtype, 3, v.base, dims, strides, box, swizzle, "tc_gemm");
 }
 
 // column split of the Nu dimension: one tile when it fits a UMMA, equal tiles otherwise
@@ -1194,13 +1169,8 @@ int fill_problem(GemmProblemDev* d, int dtype, const TcGemmProblem& p, bool ts, 
 
 template <int KIND>
 int launch_kind(const GemmProblemDev& single, const GemmLaunch& L, uint32_t smem, int grid, cudaStream_t s) {
-  static std::atomic<int> attr_set[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(tcgemm_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, GM_SMEM_LIMIT));
-    attr_set[dev & 63].store(1);
-  }
+  int rc = allow_dynamic_smem<tcgemm_kernel<KIND>>(GM_SMEM_LIMIT);
+  if (rc) return rc;
   tcgemm_kernel<KIND><<<grid, GM_THREADS, smem, s>>>(single, L);
   SPFY_LAUNCH_OK("tcgemm_kernel");
   return SPFY_OK;
@@ -1208,26 +1178,16 @@ int launch_kind(const GemmProblemDev& single, const GemmLaunch& L, uint32_t smem
 
 template <int KIND>
 int launch_pairs(const GemmProblemDev& single, const GemmLaunch& L, uint32_t smem, int grid, cudaStream_t s) {
-  static std::atomic<int> attr_set[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(tcgemm2_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, GM_SMEM_LIMIT));
-    attr_set[dev & 63].store(1);
-  }
+  int rc = allow_dynamic_smem<tcgemm2_kernel<KIND>>(GM_SMEM_LIMIT);
+  if (rc) return rc;
   tcgemm2_kernel<KIND><<<grid, GM_THREADS, smem, s>>>(single, L);  // clusters of two (__cluster_dims__)
   SPFY_LAUNCH_OK("tcgemm2_kernel");
   return SPFY_OK;
 }
 
 int launch_ts(const GemmProblemDev& single, const GemmLaunch& L, uint32_t smem, int grid, cudaStream_t s) {
-  static std::atomic<int> attr_set[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(tcgemm_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GM_SMEM_LIMIT));
-    attr_set[dev & 63].store(1);
-  }
+  int rc = allow_dynamic_smem<tcgemm_ts_kernel>(GM_SMEM_LIMIT);
+  if (rc) return rc;
   tcgemm_ts_kernel<<<grid, TS_THREADS, smem, s>>>(single, L);
   SPFY_LAUNCH_OK("tcgemm_ts_kernel");
   return SPFY_OK;
@@ -1247,9 +1207,8 @@ void warm_gemm_kernels() {
 
 int tc_gemm_supported(int dtype, const TcGemmProblem& p, bool allow_repack) {
   DeviceInfo di;
-  int rc = device_info(&di);
+  int rc = require_sm100("tc_gemm", &di);
   if (rc) return rc;
-  if (di.cc_major != 10) return fail(SPFY_E_UNSUPPORTED, "tc_gemm: needs an sm_100a device, found sm_%d%d", di.cc_major, di.cc_minor);
   return check_problem(dtype, p, allow_repack);
 }
 
@@ -1292,10 +1251,9 @@ int repack_operand(int dtype, OperandView* v, size_t nb, uint8_t* ws, size_t ws_
   uint8_t* dst = ws + *used;
   *used += bytes;
   const size_t total = batches * outer * inner;
-  DeviceInfo di;
-  int rc = device_info(&di);
+  int grid = 1;
+  int rc = capped_grid(ceil_div(total, 256), 16, &grid);
   if (rc) return rc;
-  const unsigned grid = (unsigned)std::min<size_t>(ceil_div(total, 256), (size_t)di.sm_count * 16);
   if (es == 4)
     repack_kernel<uint32_t><<<grid, 256, 0, s>>>((const uint32_t*)v->base, v->ld, v->stride, (uint32_t*)dst, ldp, outer * ldp,
                                                 inner, outer, batches);
@@ -1314,9 +1272,8 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
   if (count == 0) return SPFY_OK;
   if (!problems) return fail(SPFY_E_INVALID, "tc_gemm: null problem list");
   DeviceInfo di;
-  int rc = device_info(&di);
+  int rc = require_sm100("tc_gemm", &di);
   if (rc) return rc;
-  if (di.cc_major != 10) return fail(SPFY_E_UNSUPPORTED, "tc_gemm: needs an sm_100a device, found sm_%d%d", di.cc_major, di.cc_minor);
   std::vector<GemmProblemDev> table;
   table.reserve(count);
   uint32_t units = 0, bn_max = 16;

@@ -939,18 +939,6 @@ prune24_check_kernel(const uint16_t* __restrict__ in, size_t ld_in, uint32_t row
   if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicExch(invalid, 1);
 }
 
-int grid_for(size_t work_items, int threads, int* grid) {
-  DeviceInfo di;
-  int rc = device_info(&di);
-  if (rc) return rc;
-  size_t blocks = ceil_div(work_items, (size_t)threads);
-  size_t cap = (size_t)di.sm_count * 16;  // 16 x 256 threads = 2 full waves of resident warps
-  if (blocks > cap) blocks = cap;
-  if (blocks == 0) blocks = 1;
-  *grid = (int)blocks;
-  return SPFY_OK;
-}
-
 // validate one matrix and fill the kernel's parameter block
 int fill_prune24(Prune24Params* out, int layout, const uint16_t* src, size_t ld_src, void* out_dense,
                  size_t ld_out, void* comp_vals, void* meta, uint64_t* mask, size_t rows, size_t cols) {
@@ -1041,7 +1029,7 @@ int spfy_prune_blocks_ref(int dtype, void* weights, uint64_t* mask, size_t m, si
       ++done;
     }
   int grid = 1;
-  int rc = grid_for(ceil_div(total, 4), 256, &grid);
+  int rc = capped_grid(ceil_div(ceil_div(total, 4), 256), 16, &grid);
   if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   if ((uintptr_t)mask % 8 || (uintptr_t)weights % eb)
@@ -1120,7 +1108,7 @@ int spfy_prune24(int dtype, int mode, int layout, const void* in, size_t ld_in, 
       if (rcf) return rcf;
       const size_t dom_cols = P.tile_order ? (size_t)P.k_tiles * 128 : cols;
       int blocksf = 1;
-      rcf = grid_for(ceil_div((size_t)P.dom_rows, 4) * (dom_cols / 4), 256, &blocksf);
+      rcf = capped_grid(ceil_div(ceil_div((size_t)P.dom_rows, 4) * (dom_cols / 4), 256), 16, &blocksf);
       if (rcf) return rcf;
       const size_t fx = ceil_div(dom_cols / 4, 32), fy_all = ceil_div(ceil_div((size_t)P.dom_rows, 4), 8);
       size_t fy = ceil_div((size_t)blocksf, fx);
@@ -1134,7 +1122,7 @@ int spfy_prune24(int dtype, int mode, int layout, const void* in, size_t ld_in, 
       return SPFY_OK;
     }
     int blocks = 1;
-    int rc = grid_for(ceil_div(rows, 4) * ceil_div(cols, 4), 256, &blocks);  // cap: two waves of resident warps
+    int rc = capped_grid(ceil_div(ceil_div(rows, 4) * ceil_div(cols, 4), 256), 16, &blocks);  // cap: two waves of resident warps
     if (rc) return rc;
     // 32 tile columns x 8 tile rows per block; the rows are walked with a stride when the cap binds
     const size_t gx = ceil_div(ceil_div(cols, 4), 32), gy_all = ceil_div(ceil_div(rows, 4), 8);
@@ -1168,13 +1156,13 @@ int spfy_prune24(int dtype, int mode, int layout, const void* in, size_t ld_in, 
   if (rc) return rc;
   int grid = 1;
   if (P.fast) {
-    rc = grid_for((size_t)fast_passes(P) * 256, 256, &grid);
+    rc = capped_grid(fast_passes(P), 16, &grid);
     if (rc) return rc;
     prune24_fast_kernel<<<grid, 256, 0, s>>>(P);
     SPFY_LAUNCH_OK("prune24_fast_kernel");
     return SPFY_OK;
   }
-  rc = grid_for((size_t)P.dom_rows * P.units_per_row, 256, &grid);
+  rc = capped_grid(ceil_div((size_t)P.dom_rows * P.units_per_row, 256), 16, &grid);
   if (rc) return rc;
   prune24_strip_kernel<<<grid, 256, 0, s>>>(P);
   SPFY_LAUNCH_OK("prune24_strip_kernel");
@@ -1189,9 +1177,7 @@ int spfy_prune24_batched(int dtype, int mode, int layout, const spfy_prune24_ite
   if (layout != SPFY_LAYOUT_CANONICAL && layout != SPFY_LAYOUT_SM100)
     return fail(SPFY_E_INVALID, "prune24_batched: bad layout %d", layout);
   if (count && !items) return fail(SPFY_E_INVALID, "prune24_batched: null item table");
-  DeviceInfo di;
-  int rc = device_info(&di);
-  if (rc) return rc;
+  int rc = SPFY_OK;
   cudaStream_t s = (cudaStream_t)stream;
   const bool tile = mode == SPFY_PRUNE_TILE_MAG;
   static thread_local Prune24Batch Bt;  // 10 KB: keep it off the stack
@@ -1229,9 +1215,9 @@ int spfy_prune24_batched(int dtype, int mode, int layout, const spfy_prune24_ite
       ++Bt.count;
     }
     if (Bt.count == 0) continue;
-    const uint32_t tiles = Bt.tile_prefix[Bt.count];
-    const uint32_t cap = (uint32_t)di.sm_count * 16;
-    const uint32_t grid = tiles < cap ? tiles : cap;
+    int grid = 1;
+    rc = capped_grid(Bt.tile_prefix[Bt.count], 16, &grid);
+    if (rc) return rc;
     if (!tile) {
       prune24_batched_kernel<<<grid, 256, 0, s>>>(Bt);
       SPFY_LAUNCH_OK("prune24_batched_kernel");
@@ -1254,7 +1240,7 @@ int spfy_prune24_check(int dtype, const void* in, size_t ld_in, size_t rows, siz
   if (rows == 0 || cols == 0) return SPFY_OK;
   const int vec = cols % 16 == 0 && ld_in % 8 == 0 && (uintptr_t)in % 16 == 0;
   int grid = 1;
-  int rc = grid_for(vec ? rows * (cols / 16) : rows * ceil_div(cols, 4), 256, &grid);
+  int rc = capped_grid(ceil_div(vec ? rows * (cols / 16) : rows * ceil_div(cols, 4), 256), 16, &grid);
   if (rc) return rc;
   prune24_check_kernel<<<grid, 256, 0, s>>>((const uint16_t*)in, ld_in, (uint32_t)rows, (uint32_t)cols, vec, d_invalid);
   SPFY_LAUNCH_OK("prune24_check_kernel");

@@ -1,4 +1,4 @@
-// spmm.cu -- unstructured path: threshold prune -> COO/CSR, and row-split SpMM
+// spmm.cu -- unstructured path: threshold prune -> COO/CSR, and SpMM with a CSR, COO or blocked-ELL operand
 //
 //   spfy_threshold_to_coo / spfy_coo_to_csr   magnitude-threshold compaction
 //   spfy_spmm_csr_strided_batched             C_b = alpha*A*B_b + beta*C_b  (A shared)
@@ -7,14 +7,14 @@
 //   spfy_spmm_bell_batched                    blocked-ELL A_b per batch, B shared
 //                                             (reference: include/sparsify.me/spmm.hxx:30-138)
 //
-// SpMM design (all dense operands column-major like the reference's cuSPARSE
-// descriptors, spmm.hxx:63,67,170,173): a CTA owns a tile of TM rows x 32 columns.
-// The dense operand tile B[k-chunk x 32] is staged TRANSPOSED in shared memory so
-// that for one non-zero (i, c) the 32 lanes of a warp read 32 consecutive words
-// (one per output column).  A warp owns RPW rows; it loads 32 non-zeros with one
-// coalesced request and broadcasts them with shuffles.  Accumulators live in
-// registers; the C tile goes back through shared memory so the column-major
-// stores are coalesced along rows.
+// All dense operands are column-major like the reference's cuSPARSE descriptors (spmm.hxx:63,67,170,173).
+// The file holds, in this order (each section's comment has the details):
+//   - the threshold compaction (one chained-scan pass to sorted COO, and the CSR row pointers);
+//   - the row-split kernel: the stand-in for 16-bit blocked-ELL operands that have no tensor-core route
+//     (operands outside the TMA contract, repeated block ids);
+//   - the CUDA-core kernels for fp32 CSR / blocked-ELL: one per non-zero, and the dense walk for dense operands;
+//   - the tensor-core route: the sparse operand scattered / expanded into a dense matrix and contracted by the
+//     tcgen05 GEMM of gemm_sm100.cu.
 #include "common.cuh"
 #include "gemm_sm100.cuh"
 
@@ -28,20 +28,6 @@ namespace {
 // threshold -> COO/CSR in one pass (chained scan over 4096-element chunks, see threshold_compact_kernel);
 // entries come out sorted by (row, col).
 // ------------------------------------------------------------------------
-template <typename T>
-__device__ __forceinline__ float load_as_float(const T* p);
-template <>
-__device__ __forceinline__ float load_as_float<__half>(const __half* p) { return __half2float(*p); }
-template <>
-__device__ __forceinline__ float load_as_float<__nv_bfloat16>(const __nv_bfloat16* p) { return __bfloat162float(*p); }
-
-template <typename T>
-__device__ __forceinline__ void store_from_float(T* p, float v);
-template <>
-__device__ __forceinline__ void store_from_float<__half>(__half* p, float v) { *p = __float2half_rn(v); }
-template <>
-__device__ __forceinline__ void store_from_float<__nv_bfloat16>(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
-
 // One pass, chained scan.  The matrix is walked in row-major element order in chunks of 4096 elements
 // (256 threads x 4 groups of 4), one per CTA.  A CTA counts the kept elements of its chunk, publishes the count,
 // looks back over its predecessors' (aggregate | inclusive prefix) words, 32 per step, until it meets an inclusive prefix,
@@ -317,7 +303,11 @@ coo_to_csr_kernel(const int32_t* __restrict__ row_idx, size_t nnz, uint32_t rows
 }
 
 // ------------------------------------------------------------------------
-// Row-split SpMM.
+// Row-split SpMM: a CTA owns a tile of TM rows x 32 columns.  The dense operand tile B[k-chunk x 32] is staged
+// TRANSPOSED in shared memory so that for one non-zero (i, c) the 32 lanes of a warp read 32 consecutive words
+// (one per output column).  A warp owns RPW rows; it loads 32 non-zeros with one coalesced request and broadcasts
+// them with shuffles.  Accumulators live in registers; the C tile goes back through shared memory so the
+// column-major stores are coalesced along rows.
 // ------------------------------------------------------------------------
 constexpr int SP_WARPS = 16;           // warps per CTA
 constexpr int SP_RPW = 8;              // rows per warp
@@ -337,7 +327,7 @@ struct BellRows {  // blocked-ELL, one matrix per batch (reference: containers/e
   __device__ __forceinline__ void fetch(uint32_t batch, uint32_t row, uint32_t idx, int32_t& c, float& v) const {
     const int64_t bc = col_idx[batch][(size_t)(row / block) * bcols + idx / block];
     c = bc < 0 ? -1 : (int32_t)(bc * block + idx % block);
-    v = load_as_float(values[batch] + (size_t)row * ell_cols + idx);
+    v = to_f32(values[batch][(size_t)row * ell_cols + idx]);
   }
 };
 
@@ -380,7 +370,7 @@ spmm_rowsplit_kernel(const Rows A, const SpmmDense D) {
       const bool col_ok = j0 + j < D.n;
       const T* src = Bb + (size_t)(j0 + j) * D.ldb + k0;
       for (uint32_t kk = lane; kk < kn; kk += 32)
-        sB[kk * SP_PAD + j] = col_ok ? load_as_float(src + kk) : 0.f;
+        sB[kk * SP_PAD + j] = col_ok ? to_f32(src[kk]) : 0.f;
     }
     __syncthreads();
 #pragma unroll
@@ -418,8 +408,8 @@ spmm_rowsplit_kernel(const Rows A, const SpmmDense D) {
     if (j0 + j < D.n && i0 + i < D.m) {
       T* dst = Cb + (size_t)(j0 + j) * D.ldc + i0 + i;
       float out = D.alpha * sC[j * (SP_TM + 1) + i];
-      if (D.beta != 0.f) out += D.beta * load_as_float(dst);
-      store_from_float(dst, out);
+      if (D.beta != 0.f) out += D.beta * to_f32(*dst);
+      *dst = from_f32<T>(out);
     }
   }
 }
@@ -438,32 +428,14 @@ int launch_spmm(const Rows& A, SpmmDense D, cudaStream_t s) {
   size_t smem = kc * SP_PAD * 4;
   if (smem < c_tile) smem = c_tile;
   D.kc = (uint32_t)kc;
-  static std::atomic<size_t> attr_bytes[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (attr_bytes[dev & 63].load() < smem) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(spmm_rowsplit_kernel<T, Rows>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
-    attr_bytes[dev & 63].store(budget);
-  }
+  rc = allow_dynamic_smem<spmm_rowsplit_kernel<T, Rows>>(budget);
+  if (rc) return rc;
   const size_t row_tiles = ceil_div(D.m, SP_TM), col_tiles = ceil_div(D.n, SP_TN);
   const size_t ctas = row_tiles * col_tiles * D.num_batches;
   if (ctas == 0) return SPFY_OK;
   if (ctas >= (1ull << 31)) return fail(SPFY_E_UNSUPPORTED, "spmm: grid too large");
   spmm_rowsplit_kernel<T, Rows><<<(unsigned)ctas, SP_WARPS * 32, smem, s>>>(A, D);
   SPFY_LAUNCH_OK("spmm_rowsplit_kernel");
-  return SPFY_OK;
-}
-
-int elementwise_grid(size_t items, int* grid) {
-  DeviceInfo di;
-  int rc = device_info(&di);
-  if (rc) return rc;
-  size_t blocks = ceil_div(items, 256);
-  const size_t cap = (size_t)di.sm_count * 8;
-  if (blocks > cap) blocks = cap;
-  if (!blocks) blocks = 1;
-  *grid = (int)blocks;
   return SPFY_OK;
 }
 
@@ -1124,13 +1096,8 @@ spmm_dense_walk_kernel(const __grid_constant__ CsrSpmmParams P) {
 template <int RPW, bool BELL>
 int launch_spmm_dense_walk(const CsrSpmmParams& P, int sm_count, cudaStream_t s) {
   const size_t smem = ((size_t)2 * CSR_TN * DW_PITCH + (size_t)DW_WARPS * 16 * DW_PITCH) * 4 + 2 * CSR_TN * sizeof(size_t);
-  static std::atomic<int> attr_set[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(spmm_dense_walk_kernel<RPW, BELL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set[dev & 63].store(1);
-  }
+  int rc = allow_dynamic_smem<spmm_dense_walk_kernel<RPW, BELL>>(smem);
+  if (rc) return rc;
   const uint32_t tiles = P.row_tiles * P.col_tiles * (BELL ? P.num_batches : 1u);
   const uint32_t grid = tiles < (uint32_t)sm_count ? tiles : (uint32_t)sm_count;
   spmm_dense_walk_kernel<RPW, BELL><<<grid, DW_THREADS, smem, s>>>(P);
@@ -1152,13 +1119,8 @@ int launch_spmm_csr(const CsrSpmmParams& P, int sm_count, cudaStream_t s) {
   constexpr bool BELL = MODE != SPMM_CSR;
   size_t smem = ((size_t)CSR_TN * CSR_PITCH_PAIRS) * 4;  // >= the C tile [CSR_TN][TM + 1] for TM <= 128
   smem += (size_t)CSR_SCRATCH_FLOATS * 4 + 2 * CSR_TN * sizeof(size_t);  // scratch lines + column offsets
-  static std::atomic<int> attr_set[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(spmm_csr_kernel<RPW, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set[dev & 63].store(1);
-  }
+  int rc = allow_dynamic_smem<spmm_csr_kernel<RPW, MODE>>(smem);
+  if (rc) return rc;
   const uint32_t tiles = P.row_tiles * P.col_tiles * (BELL ? P.num_batches : 1u);
   const uint32_t grid = tiles < (uint32_t)sm_count ? tiles : (uint32_t)sm_count;
   spmm_csr_kernel<RPW, MODE><<<grid, CSR_THREADS, smem, s>>>(P);
@@ -1258,6 +1220,21 @@ bell_expand_kernel(const int64_t* const* __restrict__ col_ptrs, const void* cons
     __syncwarp();
   }
   if (__any_sync(0xffffffffu, saw_dup) && lane == 0) atomicExch(dup, 1);
+}
+
+// (one signature for every T, so that the caller can pick the instance by dtype)
+template <typename T>
+int launch_bell_expand(int grid, size_t inv_bytes, cudaStream_t s, const int64_t* const* col_ptrs, const void* const* val_ptrs,
+                       uint32_t b0, uint32_t nbatch, uint32_t rows, uint32_t cols, uint32_t ell_cols, uint32_t block,
+                       uint32_t bcols, uint32_t block_rows, uint32_t nbc, void* D, size_t ld, size_t stride, int* dup) {
+  if (inv_bytes > 48 * 1024) {
+    int rc = allow_dynamic_smem<bell_expand_kernel<T>>(200 * 1024);
+    if (rc) return rc;
+  }
+  bell_expand_kernel<T><<<grid, 256, inv_bytes, s>>>(col_ptrs, val_ptrs, b0, nbatch, rows, cols, ell_cols, block, bcols,
+                                                    block_rows, nbc, (T*)D, ld, stride, dup);
+  SPFY_LAUNCH_OK("bell_expand_kernel");
+  return SPFY_OK;
 }
 
 // density of non-zeros from which the tensor-core route is taken when the caller leaves the choice to the library:
@@ -1389,7 +1366,7 @@ int spfy_coo_to_csr(const int32_t* row_idx, size_t nnz, size_t rows, int32_t* ro
   if ((!row_idx && nnz) || !row_ptr) return fail(SPFY_E_INVALID, "coo_to_csr: null pointer");
   if (nnz >= (1ull << 31) || rows >= (1ull << 31)) return fail(SPFY_E_UNSUPPORTED, "coo_to_csr: too large");
   int grid = 1;
-  int rc = elementwise_grid(nnz + 1, &grid);
+  int rc = capped_grid(ceil_div(nnz + 1, 256), 8, &grid);
   if (rc) return rc;
   coo_to_csr_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(row_idx, nnz, (uint32_t)rows, row_ptr);
   SPFY_LAUNCH_OK("coo_to_csr_kernel");
@@ -1481,7 +1458,7 @@ static int spmm_csr_impl(int alg, size_t m, size_t k, size_t n, size_t num_batch
   SPFY_CUDA_OK(cudaMemsetAsync(d_sorted, 0xff, sizeof(int), s));
   if (run_sparse || (run_dense && !tensor)) {
     int grid = 1;
-    rc = elementwise_grid(m * 32, &grid);
+    rc = capped_grid(ceil_div(m * 32, 256), 8, &grid);
     if (rc) return rc;
     csr_check_sorted_kernel<<<grid, 256, 0, s>>>(row_ptr, col_idx, (uint32_t)m, d_sorted, gated ? d_dense : nullptr,
                                                  dense_nnz);
@@ -1519,14 +1496,14 @@ static int spmm_csr_impl(int alg, size_t m, size_t k, size_t n, size_t num_batch
   {
     int grid = 1;
     if (coo_rows) {
-      rc = elementwise_grid((size_t)nnz_host, &grid);
+      rc = capped_grid(ceil_div((size_t)nnz_host, 256), 8, &grid);
       if (rc) return rc;
       if (nnz_host > 0) {
         coo_scatter_kernel<<<grid, 256, 0, s>>>(coo_rows, col_idx, vals, (size_t)nnz_host, (uint32_t)m, (uint32_t)k, dense, ld);
         SPFY_LAUNCH_OK("coo_scatter_kernel");
       }
     } else {
-      rc = elementwise_grid(m * 32, &grid);
+      rc = capped_grid(ceil_div(m * 32, 256), 8, &grid);
       if (rc) return rc;
       csr_scatter_kernel<<<grid, 256, 0, s>>>(row_ptr, col_idx, vals, (uint32_t)m, (uint32_t)k, dense, ld);
       SPFY_LAUNCH_OK("csr_scatter_kernel");
@@ -1679,7 +1656,7 @@ int spfy_spmm_bell_batched(int alg, int dtype, size_t rows, size_t cols, size_t 
   if (bcols > 1 && dtype == SPFY_F32) {
     // (the CUDA-core kernel's cursor mode needs to know whether the ids ascend; cheap next to the values)
     int grid = 1;
-    rc = elementwise_grid(num_batches * block_rows * bcols, &grid);
+    rc = capped_grid(ceil_div(num_batches * block_rows * bcols, 256), 8, &grid);
     if (rc) return rc;
     if (!tensor) {
       bell_check_sorted_kernel<<<grid, 256, 0, s>>>(col_idx, (uint32_t)block_rows, (uint32_t)bcols,
@@ -1696,27 +1673,15 @@ int spfy_spmm_bell_batched(int alg, int dtype, size_t rows, size_t cols, size_t 
   const int precision = alg == SPFY_SPMM_ALG_TENSOR_FAST ? TC_GEMM_FAST : TC_GEMM_PRECISE;
   for (size_t b0 = 0; b0 < num_batches; b0 += chunk) {
     const size_t nbatch = std::min(chunk, num_batches - b0);
-    const size_t warps_needed = nbatch * block_rows;
-    const int grid = (int)std::min<size_t>(ceil_div(warps_needed, 8), (size_t)di.sm_count * 8);
-#define SPFY_BELL_EXPAND(T)                                                                                            \
-    do {                                                                                                                \
-      static std::atomic<int> attr_set[64];                                                                             \
-      int dev = 0;                                                                                                      \
-      SPFY_CUDA_OK(cudaGetDevice(&dev));                                                                                \
-      if (inv_bytes > 48 * 1024 && !attr_set[dev & 63].load()) {                                                        \
-        SPFY_CUDA_OK(cudaFuncSetAttribute(bell_expand_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)); \
-        attr_set[dev & 63].store(1);                                                                                    \
-      }                                                                                                                 \
-      bell_expand_kernel<T><<<grid, 256, inv_bytes, s>>>(col_idx, values, (uint32_t)b0, (uint32_t)nbatch, (uint32_t)rows, \
-                                                        (uint32_t)cols, (uint32_t)ell_cols, (uint32_t)block,           \
-                                                        (uint32_t)bcols, (uint32_t)block_rows, (uint32_t)nbc,          \
-                                                        reinterpret_cast<T*>(dense), ld, mat / es, d_dup);             \
-    } while (0)
-    if (dtype == SPFY_F32) SPFY_BELL_EXPAND(float);
-    else if (dtype == SPFY_F16) SPFY_BELL_EXPAND(__half);
-    else SPFY_BELL_EXPAND(__nv_bfloat16);
-#undef SPFY_BELL_EXPAND
-    SPFY_LAUNCH_OK("bell_expand_kernel");
+    int grid = 1;
+    rc = capped_grid(ceil_div(nbatch * block_rows, 8), 8, &grid);  // one warp per block row
+    if (rc) return rc;
+    const auto expand = dtype == SPFY_F32 ? launch_bell_expand<float>
+                        : dtype == SPFY_F16 ? launch_bell_expand<__half> : launch_bell_expand<__nv_bfloat16>;
+    rc = expand(grid, inv_bytes, s, col_idx, values, (uint32_t)b0, (uint32_t)nbatch, (uint32_t)rows, (uint32_t)cols,
+                (uint32_t)ell_cols, (uint32_t)block, (uint32_t)bcols, (uint32_t)block_rows, (uint32_t)nbc, dense, ld, mat / es,
+                d_dup);
+    if (rc) return rc;
     TcGemmProblem p;
     p.opA = SPFY_OP_T; p.opB = SPFY_OP_N;  // row-major dense A_b = column-major k x m; B is k x n column-major
     p.m = rows; p.n = n; p.k = cols; p.nb = nbatch;

@@ -46,6 +46,7 @@
 
 #include <algorithm>
 #include <cstdlib>
+#include <memory>
 #include <vector>
 
 namespace spfy {
@@ -751,21 +752,9 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
 int make_tmap_2d(CUtensorMap* map, int dtype, const void* base, uint64_t inner, uint64_t outer,
                  uint64_t ld, uint32_t box_inner, uint32_t box_outer,
                  CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
-  EncodeTiledFn enc;
-  int rc = get_encoder(&enc);
-  if (rc) return rc;
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld * 2};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16,
-                   2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS)
-    return fail(SPFY_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for %llu x %llu ld %llu", (int)r,
-                (unsigned long long)outer, (unsigned long long)inner, (unsigned long long)ld);
-  return SPFY_OK;
+  const cuuint64_t dims[2] = {inner, outer}, strides[1] = {ld * 2};
+  const cuuint32_t box[2] = {box_inner, box_outer};
+  return encode_tiled(map, dtype, 2, base, dims, strides, box, swizzle, "spmma");
 }
 
 // The same matrix (inner % 64 == 0) viewed as [inner/64 groups][outer][64]: a box of
@@ -773,21 +762,9 @@ int make_tmap_2d(CUtensorMap* map, int dtype, const void* base, uint64_t inner, 
 // blocks -- exactly the two halves of a B stage -- with ONE TMA instruction.
 int make_tmap_grouped(CUtensorMap* map, int dtype, const void* base, uint64_t inner, uint64_t outer,
                       uint64_t ld, uint32_t box_outer, uint32_t box_groups) {
-  EncodeTiledFn enc;
-  int rc = get_encoder(&enc);
-  if (rc) return rc;
-  cuuint64_t dims[3] = {64, outer, inner / 64};
-  cuuint64_t strides[2] = {ld * 2, 128};
-  cuuint32_t box[3] = {64, box_outer, box_groups};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(map, dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16,
-                   3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS)
-    return fail(SPFY_E_CUDA, "cuTensorMapEncodeTiled (grouped) failed (%d) for %llu x %llu ld %llu", (int)r,
-                (unsigned long long)outer, (unsigned long long)inner, (unsigned long long)ld);
-  return SPFY_OK;
+  const cuuint64_t dims[3] = {64, outer, inner / 64}, strides[2] = {ld * 2, 128};
+  const cuuint32_t box[3] = {64, box_outer, box_groups};
+  return encode_tiled(map, dtype, 3, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, "spmma (grouped view)");
 }
 
 struct HostProblem {
@@ -806,6 +783,12 @@ struct HostProblem {
 // the `opB` argument of the C ABI carries the output layout in bit 4 (SPFY_OUT_T)
 inline int op_of(int opB) { return opB & ~SPFY_OUT_T; }
 inline bool out_t_of(int opB) { return (opB & SPFY_OUT_T) != 0; }
+
+// D of a problem, or a replica of D at `base`: boxes of 64 n x 32 m, or of 32 m x 64 n (unswizzled) when transposed
+int make_tmap_d(CUtensorMap* map, int dtype, const HostProblem& h, void* base) {
+  return h.out_t ? make_tmap_2d(map, dtype, base, h.m, h.n, h.ldd, 32, 64, CU_TENSOR_MAP_SWIZZLE_NONE)
+                 : make_tmap_2d(map, dtype, base, h.n, h.m, h.ldd, 64, 32);
+}
 
 // NHWC activations {C, W, H, N} in im2col mode: one instruction gathers 128 consecutive output positions x 64 channels
 // of one filter tap.  The bounding box of base pixels is [-pad, dim + pad - (filter - 1)) per spatial dimension, walked
@@ -944,8 +927,7 @@ int fill_problem(ProblemDev* d, int dtype, const HostProblem& h, int cls) {
     if (!d->b3d) rc = make_tmap_2d(&d->tmap_b, dtype, h.B, b_inner, b_outer, h.ldb, 64, box_outer);
     if (rc) return rc;
   }
-  rc = h.out_t ? make_tmap_2d(&d->tmap_d, dtype, h.D, h.m, h.n, h.ldd, 32, 64, CU_TENSOR_MAP_SWIZZLE_NONE)
-               : make_tmap_2d(&d->tmap_d, dtype, h.D, h.n, h.m, h.ldd, 64, 32);
+  rc = make_tmap_d(&d->tmap_d, dtype, h, h.D);
   if (rc) return rc;
   d->out_t = h.out_t;
   d->a_vals = (const uint8_t*)h.comp_vals;
@@ -1042,14 +1024,8 @@ uint32_t make_idesc(int dtype, int opB) {
 template <bool BF16, bool OPB_T, bool EPI>
 int launch_t(const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid, cudaStream_t s,
              bool overlap_previous) {
-  static std::atomic<int> attr_set[64];
-  int dev = 0;
-  SPFY_CUDA_OK(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63].load()) {
-    SPFY_CUDA_OK(cudaFuncSetAttribute(spmma_kernel<BF16, OPB_T, EPI>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    attr_set[dev & 63].store(1);
-  }
+  int rc = allow_dynamic_smem<spmma_kernel<BF16, OPB_T, EPI>>(SMEM_LIMIT);
+  if (rc) return rc;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)grid);
@@ -1148,6 +1124,40 @@ int conv_problem(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, c
   return validate(dtype, h, who);
 }
 
+// SPFY_SPMMA_DEBUG=mode: a dev-build ablation of the kernel (L.dbg)
+uint32_t debug_mode() {
+  const char* e = dev_switch("SPFY_SPMMA_DEBUG");
+  return e ? (uint32_t)atoi(e) : 0u;
+}
+
+// one validated problem (spfy_spmma*, spfy_spmma_conv*) in a launch of its own
+int run_single(int dtype, const HostProblem& h, cudaStream_t s) {
+  if (h.m == 0 || h.n == 0) return SPFY_OK;
+  DeviceInfo di;
+  int rc = require_sm100(h.conv ? "spmma_conv" : "spmma", &di);
+  if (rc) return rc;
+  const int cls = classify(h, false, di.sm_count);
+  ProblemDev d;
+  rc = fill_problem(&d, dtype, h, cls);
+  if (rc) return rc;
+  d.unit_begin = 0;
+  split_tail(&d, cls, di.sm_count);
+  LaunchParams L;
+  memset(&L, 0, sizeof(L));
+  uint32_t smem = 0;
+  geometry(cls, res_values_bytes(d), res_meta_bytes(d), &L, &smem);
+  L.table = nullptr;
+  L.num_problems = 1;
+  L.total_units = d.units;
+  L.idesc = make_idesc(dtype, h.opB);
+  L.dbg = debug_mode();
+  const int grid = (int)(d.units < (uint32_t)di.sm_count ? d.units : (uint32_t)di.sm_count);
+#ifdef SPFY_DEV_SWITCHES
+  if (const char* path = dev_switch("SPFY_SPMMA_TRACE")) return launch_traced(path, dtype, h.opB, d, L, smem, grid, s);
+#endif
+  return launch(dtype, h.opB, d.epi != 0, d, L, smem, grid, s);
+}
+
 struct Plan {
   int dtype = 0;
   ProblemDev* d_table = nullptr;  // all launches back to back
@@ -1196,38 +1206,9 @@ static int spmma_impl(int dtype, int opB, size_t m, size_t n, size_t k, float al
   h.out_t = out_t_of(opB);
   if (epi) h.epi = *epi;
   h.ex = ex;
-  opB = h.opB;
   int rc = validate(dtype, h, "spmma");
   if (rc) return rc;
-  if (m == 0 || n == 0) return SPFY_OK;
-  DeviceInfo di;
-  rc = device_info(&di);
-  if (rc) return rc;
-  if (di.cc_major != 10)
-    return fail(SPFY_E_UNSUPPORTED, "spmma: needs an sm_100a device, found sm_%d%d", di.cc_major, di.cc_minor);
-  const int cls = classify(h, false, di.sm_count);
-  ProblemDev d;
-  rc = fill_problem(&d, dtype, h, cls);
-  if (rc) return rc;
-  d.unit_begin = 0;
-  split_tail(&d, cls, di.sm_count);
-  LaunchParams L;
-  memset(&L, 0, sizeof(L));
-  uint32_t smem = 0;
-  geometry(cls, res_values_bytes(d), res_meta_bytes(d), &L, &smem);
-  L.table = nullptr;
-  L.num_problems = 1;
-  L.total_units = d.units;
-  L.idesc = make_idesc(dtype, opB);
-  {
-    const char* e = dev_switch("SPFY_SPMMA_DEBUG");
-    L.dbg = e ? (uint32_t)atoi(e) : 0u;
-  }
-  const int grid = (int)(d.units < (uint32_t)di.sm_count ? d.units : (uint32_t)di.sm_count);
-#ifdef SPFY_DEV_SWITCHES
-  if (const char* path = dev_switch("SPFY_SPMMA_TRACE")) return launch_traced(path, dtype, opB, d, L, smem, grid, (cudaStream_t)stream);
-#endif
-  return launch(dtype, opB, d.epi != 0, d, L, smem, grid, (cudaStream_t)stream);
+  return run_single(dtype, h, (cudaStream_t)stream);
 }
 
 int spfy_spmma(int dtype, int opB, size_t m, size_t n, size_t k, float alpha, const void* comp_vals,
@@ -1247,7 +1228,12 @@ int spfy_spmma_ex(int dtype, int opB, size_t m, size_t n, size_t k, float alpha,
 
 static int spmma_conv_impl(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                            const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
-                           bool out_t, const spfy_epilogue* epi, bool ex, spfy_stream_t stream);
+                           bool out_t, const spfy_epilogue* epi, bool ex, spfy_stream_t stream) {
+  HostProblem h;
+  int rc = conv_problem(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, out_t, epi, ex, "spmma_conv", &h);
+  if (rc) return rc;
+  return run_single(dtype, h, (cudaStream_t)stream);
+}
 
 int spfy_spmma_conv(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                     const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
@@ -1268,48 +1254,116 @@ int spfy_spmma_conv_ex(int dtype, const spfy_conv_desc* conv, size_t m, float al
                          stream);
 }
 
-static int spmma_conv_impl(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
-                           const void* meta, const void* X, float beta, const void* C, size_t ldc, void* D, size_t ldd,
-                           bool out_t, const spfy_epilogue* epi, bool ex, spfy_stream_t stream) {
-  HostProblem h;
-  int rc = conv_problem(dtype, conv, m, alpha, comp_vals, meta, X, beta, C, ldc, D, ldd, out_t, epi, ex, "spmma_conv", &h);
-  if (rc) return rc;
-  const size_t n = h.n;
-  if (m == 0 || n == 0) return SPFY_OK;
-  DeviceInfo di;
-  rc = device_info(&di);
-  if (rc) return rc;
-  if (di.cc_major != 10)
-    return fail(SPFY_E_UNSUPPORTED, "spmma_conv: needs an sm_100a device, found sm_%d%d", di.cc_major, di.cc_minor);
-  const int cls = classify(h, false, di.sm_count);
-  ProblemDev d;
-  rc = fill_problem(&d, dtype, h, cls);
-  if (rc) return rc;
-  d.unit_begin = 0;
-  split_tail(&d, cls, di.sm_count);
-  LaunchParams L;
-  memset(&L, 0, sizeof(L));
-  uint32_t smem = 0;
-  geometry(cls, res_values_bytes(d), res_meta_bytes(d), &L, &smem);
-  L.table = nullptr;
-  L.num_problems = 1;
-  L.total_units = d.units;
-  L.idesc = make_idesc(dtype, SPFY_OP_T);
-  const int grid = (int)(d.units < (uint32_t)di.sm_count ? d.units : (uint32_t)di.sm_count);
-#ifdef SPFY_DEV_SWITCHES
-  if (const char* path = dev_switch("SPFY_SPMMA_TRACE")) return launch_traced(path, dtype, SPFY_OP_T, d, L, smem, grid, (cudaStream_t)stream);
-#endif
-  return launch(dtype, SPFY_OP_T, d.epi != 0, d, L, smem, grid, (cudaStream_t)stream);
-}
-
 static void plan_free(Plan* plan) {
   if (plan->d_table) cudaFree(plan->d_table);
   if (plan->d_rep) cudaFree(plan->d_rep);
   delete plan;
 }
+
+// problem i of a plan as the host sees it (a convolution layer when convs[i] is given: B = X, n / k / ldb / opB from the
+// descriptor, the SPFY_OUT_T bit of opB still selects the NHWC output)
+static int plan_problem(int dtype, const spfy_spmma_problem& q, const spfy_conv_desc* conv, const spfy_epilogue* epi, bool ex,
+                        HostProblem* h) {
+  if (conv)
+    return conv_problem(dtype, conv, q.m, q.alpha, q.comp_vals, q.meta, q.B, q.beta, q.C, q.ldc, q.D, q.ldd, out_t_of(q.opB),
+                        epi, ex, "spmma_plan_create", h);
+  *h = HostProblem{op_of(q.opB), q.m, q.n, q.k, q.comp_vals, q.meta, q.B, q.C, q.D, q.ldb, q.ldc, q.ldd, q.alpha, q.beta};
+  h->out_t = out_t_of(q.opB);
+  if (epi) h->epi = *epi;
+  h->ex = ex;
+  return validate(dtype, *h, "spmma_plan_create");
+}
+
 static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs,
                             const spfy_epilogue* const* epis, bool ex, size_t count, size_t n_rep, void* const* rep_d,
-                            spfy_spmma_plan_t* out);
+                            spfy_spmma_plan_t* out) {
+  if (!out) return fail(SPFY_E_INVALID, "spmma_plan_create: null plan pointer");
+  *out = nullptr;
+  if (count && !problems) return fail(SPFY_E_INVALID, "spmma_plan_create: null problem list");
+  DeviceInfo di;
+  int rc = require_sm100("spmma_plan_create", &di);
+  if (rc) return rc;
+  // every non-empty problem, validated and classified once
+  struct Member {
+    size_t index;
+    HostProblem h;
+    int cls;
+  };
+  std::vector<Member> members;
+  for (size_t i = 0; i < count; ++i) {
+    HostProblem h;
+    rc = plan_problem(dtype, problems[i], convs ? convs[i] : nullptr, epis ? epis[i] : nullptr, ex, &h);
+    if (rc) return rc;
+    if (h.m && h.n) members.push_back(Member{i, h, classify(h, true, di.sm_count)});
+  }
+  // members of a launch, longest units first: the CTAs walk the unit list with a fixed stride, so
+  // whatever comes last sets the tail -- it should be the problems whose units are short
+  std::stable_sort(members.begin(), members.end(),
+                   [](const Member& a, const Member& b) { return ceil_div(a.h.k, 128) > ceil_div(b.h.k, 128); });
+  std::unique_ptr<Plan, decltype(&plan_free)> plan(new Plan(), plan_free);
+  plan->dtype = dtype;
+  std::vector<ProblemDev> table;
+  std::vector<CUtensorMap> reps;  // replica maps in table order
+  if (n_rep && count) {
+    const cudaError_t e = cudaMalloc((void**)&plan->d_rep, count * n_rep * sizeof(CUtensorMap));
+    if (e != cudaSuccess) return fail(SPFY_E_CUDA, "spmma_plan_create: %s", cudaGetErrorString(e));
+  }
+  // launches overlap tail-to-head (programmatic stream serialization), so only the last launch's tail is
+  // exposed: go from the class with the longest units (streaming, G = 2) to the one with the shortest (k <= 64)
+  for (int cls = NUM_CLASSES - 1; cls >= 0; --cls) {
+    for (int opB = 0; opB < 2; ++opB) {
+      Plan::Launch ln;
+      memset(&ln.L, 0, sizeof(ln.L));
+      ln.opB = opB;
+      ln.epi = false;
+      ln.first = (uint32_t)table.size();
+      ln.count = 0;
+      uint32_t units = 0, res_vals = 0, res_meta = 0;
+      for (const Member& mb : members) {
+        if (mb.cls != cls || mb.h.opB != opB) continue;
+        ProblemDev d;
+        rc = fill_problem(&d, dtype, mb.h, cls);
+        if (rc) return rc;
+        d.unit_begin = units;
+        if ((uint64_t)units + d.units >= (1ull << 32)) return fail(SPFY_E_UNSUPPORTED, "spmma_plan_create: too many tiles");
+        units += d.units;
+        if (n_rep) {
+          d.tmap_rep = plan->d_rep + reps.size();
+          d.n_rep = (uint32_t)n_rep;
+          for (size_t r = 0; r < n_rep; ++r) {
+            reps.emplace_back();
+            rc = make_tmap_d(&reps.back(), dtype, mb.h, rep_d[mb.index * n_rep + r]);
+            if (rc) return rc;
+          }
+        }
+        if (d.resident && res_values_bytes(d) > res_vals) res_vals = res_values_bytes(d);
+        if (d.resident && res_meta_bytes(d) > res_meta) res_meta = res_meta_bytes(d);
+        ln.epi = ln.epi || d.epi;
+        table.push_back(d);
+        ++ln.count;
+      }
+      if (!ln.count) continue;
+      geometry(cls, res_vals, res_meta, &ln.L, &ln.smem);
+      ln.L.num_problems = ln.count;
+      ln.L.total_units = units;
+      ln.L.idesc = make_idesc(dtype, opB);
+      ln.L.dbg = debug_mode();
+      ln.grid = (int)(units < (uint32_t)di.sm_count ? units : (uint32_t)di.sm_count);
+      plan->launches.push_back(ln);
+    }
+  }
+  if (!table.empty()) {
+    cudaError_t e = cudaMalloc((void**)&plan->d_table, table.size() * sizeof(ProblemDev));
+    if (e == cudaSuccess)
+      e = cudaMemcpy(plan->d_table, table.data(), table.size() * sizeof(ProblemDev), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && !reps.empty())
+      e = cudaMemcpy(plan->d_rep, reps.data(), reps.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) return fail(SPFY_E_CUDA, "spmma_plan_create: %s", cudaGetErrorString(e));
+    for (auto& ln : plan->launches) ln.L.table = plan->d_table + ln.first;
+  }
+  *out = (spfy_spmma_plan_t)plan.release();
+  return SPFY_OK;
+}
 
 int spfy_spmma_plan_create(int dtype, const spfy_spmma_problem* problems, size_t count,
                            spfy_spmma_plan_t* out) {
@@ -1335,142 +1389,6 @@ int spfy_spmma_plan_create_replicated(int dtype, const spfy_spmma_problem* probl
       return fail(SPFY_E_INVALID, "spmma_plan_create_replicated: replica %zu of problem %zu is null or not 16-byte aligned",
                   i % replicas, i / replicas);
   return plan_create_impl(dtype, problems, nullptr, nullptr, false, count, replicas, replica_d, out);
-}
-
-// problem i of a plan as the host sees it (a convolution layer when convs[i] is given: B = X, n / k / ldb / opB from the
-// descriptor, the SPFY_OUT_T bit of opB still selects the NHWC output)
-static int plan_problem(int dtype, const spfy_spmma_problem& q, const spfy_conv_desc* conv, const spfy_epilogue* epi, bool ex,
-                        HostProblem* h) {
-  if (conv)
-    return conv_problem(dtype, conv, q.m, q.alpha, q.comp_vals, q.meta, q.B, q.beta, q.C, q.ldc, q.D, q.ldd, out_t_of(q.opB),
-                        epi, ex, "spmma_plan_create", h);
-  *h = HostProblem{op_of(q.opB), q.m, q.n, q.k, q.comp_vals, q.meta, q.B, q.C, q.D, q.ldb, q.ldc, q.ldd, q.alpha, q.beta};
-  h->out_t = out_t_of(q.opB);
-  if (epi) h->epi = *epi;
-  h->ex = ex;
-  return validate(dtype, *h, "spmma_plan_create");
-}
-
-static int plan_create_impl(int dtype, const spfy_spmma_problem* problems, const spfy_conv_desc* const* convs,
-                            const spfy_epilogue* const* epis, bool ex, size_t count, size_t n_rep, void* const* rep_d,
-                            spfy_spmma_plan_t* out) {
-  if (!out) return fail(SPFY_E_INVALID, "spmma_plan_create: null plan pointer");
-  *out = nullptr;
-  if (count && !problems) return fail(SPFY_E_INVALID, "spmma_plan_create: null problem list");
-  DeviceInfo di;
-  int rc = device_info(&di);
-  if (rc) return rc;
-  if (di.cc_major != 10)
-    return fail(SPFY_E_UNSUPPORTED, "spmma_plan_create: needs an sm_100a device, found sm_%d%d", di.cc_major,
-                di.cc_minor);
-  Plan* plan = new Plan();
-  plan->dtype = dtype;
-  std::vector<ProblemDev> table;
-  std::vector<CUtensorMap> reps;  // replica maps in table order
-  if (n_rep && count) {
-    const cudaError_t e = cudaMalloc((void**)&plan->d_rep, count * n_rep * sizeof(CUtensorMap));
-    if (e != cudaSuccess) {
-      plan_free(plan);
-      return fail(SPFY_E_CUDA, "spmma_plan_create: %s", cudaGetErrorString(e));
-    }
-  }
-  // launches overlap tail-to-head (programmatic stream serialization), so only the last launch's tail is
-  // exposed: go from the class with the longest units (streaming, G = 2) to the one with the shortest (k <= 64)
-  for (int cls = NUM_CLASSES - 1; cls >= 0; --cls) {
-    for (int opB = 0; opB < 2; ++opB) {
-      Plan::Launch ln;
-      memset(&ln.L, 0, sizeof(ln.L));
-      ln.opB = opB;
-      ln.epi = false;
-      ln.first = (uint32_t)table.size();
-      ln.count = 0;
-      uint32_t units = 0, res_vals = 0, res_meta = 0;
-      // members of this launch, longest units first: the CTAs walk the unit list with a fixed stride, so
-      // whatever comes last sets the tail -- it should be the problems whose units are short
-      std::vector<size_t> members;
-      for (size_t i = 0; i < count; ++i) {
-        const spfy_spmma_problem& q = problems[i];
-        const spfy_conv_desc* cv = convs ? convs[i] : nullptr;
-        if ((cv ? SPFY_OP_T : op_of(q.opB)) != opB) continue;
-        HostProblem h;
-        rc = plan_problem(dtype, q, cv, epis ? epis[i] : nullptr, ex, &h);
-        if (rc) {
-          plan_free(plan);
-          return rc;
-        }
-        if (h.m == 0 || h.n == 0) continue;
-        if (classify(h, true, di.sm_count) != cls) continue;
-        members.push_back(i);
-      }
-      auto k_of = [&](size_t i) {
-        const spfy_conv_desc* cv = convs ? convs[i] : nullptr;
-        return cv ? cv->kh * cv->kw * cv->c : problems[i].k;
-      };
-      std::stable_sort(members.begin(), members.end(), [&](size_t a, size_t b) {
-        return ceil_div(k_of(a), 128) > ceil_div(k_of(b), 128);
-      });
-      for (size_t i : members) {
-        HostProblem h;
-        (void)plan_problem(dtype, problems[i], convs ? convs[i] : nullptr, epis ? epis[i] : nullptr, ex, &h);  // validated above
-        ProblemDev d;
-        rc = fill_problem(&d, dtype, h, cls);
-        if (rc) {
-          plan_free(plan);
-          return rc;
-        }
-        d.unit_begin = units;
-        if ((uint64_t)units + d.units >= (1ull << 32)) {
-          plan_free(plan);
-          return fail(SPFY_E_UNSUPPORTED, "spmma_plan_create: too many tiles");
-        }
-        units += d.units;
-        if (n_rep) {
-          d.tmap_rep = plan->d_rep + reps.size();
-          d.n_rep = (uint32_t)n_rep;
-          for (size_t r = 0; r < n_rep && !rc; ++r) {
-            CUtensorMap tm;
-            rc = h.out_t ? make_tmap_2d(&tm, dtype, rep_d[i * n_rep + r], h.m, h.n, h.ldd, 32, 64, CU_TENSOR_MAP_SWIZZLE_NONE)
-                         : make_tmap_2d(&tm, dtype, rep_d[i * n_rep + r], h.n, h.m, h.ldd, 64, 32);
-            reps.push_back(tm);
-          }
-          if (rc) {
-            plan_free(plan);
-            return rc;
-          }
-        }
-        if (d.resident && res_values_bytes(d) > res_vals) res_vals = res_values_bytes(d);
-        if (d.resident && res_meta_bytes(d) > res_meta) res_meta = res_meta_bytes(d);
-        ln.epi = ln.epi || d.epi;
-        table.push_back(d);
-        ++ln.count;
-      }
-      if (!ln.count) continue;
-      geometry(cls, res_vals, res_meta, &ln.L, &ln.smem);
-      ln.L.num_problems = ln.count;
-      ln.L.total_units = units;
-      ln.L.idesc = make_idesc(dtype, opB);
-      {
-        const char* e = dev_switch("SPFY_SPMMA_DEBUG");
-        ln.L.dbg = e ? (uint32_t)atoi(e) : 0u;
-      }
-      ln.grid = (int)(units < (uint32_t)di.sm_count ? units : (uint32_t)di.sm_count);
-      plan->launches.push_back(ln);
-    }
-  }
-  if (!table.empty()) {
-    cudaError_t e = cudaMalloc((void**)&plan->d_table, table.size() * sizeof(ProblemDev));
-    if (e == cudaSuccess)
-      e = cudaMemcpy(plan->d_table, table.data(), table.size() * sizeof(ProblemDev), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && !reps.empty())
-      e = cudaMemcpy(plan->d_rep, reps.data(), reps.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-      plan_free(plan);
-      return fail(SPFY_E_CUDA, "spmma_plan_create: %s", cudaGetErrorString(e));
-    }
-    for (auto& ln : plan->launches) ln.L.table = plan->d_table + ln.first;
-  }
-  *out = (spfy_spmma_plan_t)plan;
-  return SPFY_OK;
 }
 
 int spfy_spmma_plan_run(spfy_spmma_plan_t p, spfy_stream_t stream) {

@@ -428,4 +428,24 @@ inline int get_encoder(EncodeTiledFn* out) {
   return SPFY_OK;
 }
 
+// A tiled tensor map of `rank` <= 3 dimensions, innermost first (`byte_strides` has rank - 1 entries): element strides 1,
+// no interleave, L2 promotion in 256-byte lines, out-of-bounds elements read as zero.
+inline int encode_tiled(CUtensorMap* map, int dtype, uint32_t rank, const void* base, const cuuint64_t* dims,
+                        const cuuint64_t* byte_strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle, const char* who) {
+  EncodeTiledFn enc;
+  int rc = get_encoder(&enc);
+  if (rc) return rc;
+  const cuuint32_t estr[3] = {1, 1, 1};
+  const CUtensorMapDataType dt = dtype == SPFY_F32    ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                 : dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                                      : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  const CUresult r = enc(map, dt, rank, const_cast<void*>(base), dims, byte_strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                         swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS)
+    return fail(SPFY_E_CUDA, "%s: cuTensorMapEncodeTiled failed (%d) for dims %llu x %llu x %llu, row pitch %llu bytes", who,
+                (int)r, (unsigned long long)dims[0], (unsigned long long)dims[1],
+                (unsigned long long)(rank > 2 ? dims[2] : 1), (unsigned long long)byte_strides[0]);
+  return SPFY_OK;
+}
+
 }  // namespace spfy
