@@ -42,8 +42,18 @@ enum { SPFY_F16 = 0, SPFY_BF16 = 1, SPFY_F32 = 2, SPFY_F64 = 3 };
 
 /* prune24 modes.  STRIP_MAG is the contract mode (top-2-of-4 by |x| along K,
  * tie -> lower index).  TILE_MAG is the 4x4-tile variant the reference asks
- * cusparseLt for at include/sparsify.me/spmma.hxx:86. */
-enum { SPFY_PRUNE_STRIP_MAG = 0, SPFY_PRUNE_TILE_MAG = 1 };
+ * cusparseLt for at include/sparsify.me/spmma.hxx:86: each 4x4 tile keeps one of
+ * the 90 patterns with two of four along rows AND columns; its metadata is what
+ * the STRIP compressor makes of the pruned matrix (bit-exact with cusparseLt), so
+ * where a kept value is +-0 the recorded index may move to another zero.
+ * TILE_TRANSPOSABLE makes the same choice and the same dense output, but records
+ * the tile's pattern itself in the metadata: it stays two of four along columns,
+ * which spfy_transpose24 needs.  Values and metadata equal TILE_MAG's except in
+ * groups where a kept value is +-0; padding rows / columns keep the neutral nibble.
+ * Arguments as TILE_MAG (out_dense required, may alias `in`); `mask` is refused
+ * and the call needs cols % 16 == 0 and 8-byte aligned rows (SPFY_E_UNSUPPORTED
+ * otherwise).  spfy_prune24_batched refuses it. */
+enum { SPFY_PRUNE_STRIP_MAG = 0, SPFY_PRUNE_TILE_MAG = 1, SPFY_PRUNE_TILE_TRANSPOSABLE = 2 };
 
 /* layouts of the compressed operand.
  *   CANONICAL : values  [rows][ceil4(cols)/2]   row-major, ascending index
@@ -145,6 +155,47 @@ SPFY_API int spfy_prune24_batched(int dtype, int mode, int layout, const spfy_pr
  * (same convention as cusparseLtSpMMAPruneCheck, spmma.hxx:88-94). */
 SPFY_API int spfy_prune24_check(int dtype, const void* in, size_t ld_in, size_t rows,
                                 size_t cols, int* d_invalid, spfy_stream_t stream);
+
+/* ------------------------------------------------------------------------
+ * 2:4 fine-tuning: the backward pass of a pruned layer and updates under a
+ * fixed mask.  No cusparseLt counterpart (a cusparseLt user keeps the dense
+ * pruned matrix and prunes and compresses its transpose again).
+ *
+ * spfy_transpose24 -- A: SM100-layout compressed operand of a rows x cols matrix
+ * whose columns are `taps` blocks of cols / taps.  Writes the SM100-layout
+ * compressed operand of A' [cols/taps] x [taps*rows]:
+ *     A'[ci][t'*rows + r] = A[r][(taps-1-t')*cols/taps + ci]
+ * taps = 1: A' = A^T (the data gradient of a Linear layer, dx = dy W, is spfy_spmma
+ * of A' with opB = T | SPFY_OUT_T).  taps = kh*kw with A's K in (kh, kw, c) order
+ * (spfy_permute_conv_weights): A' is the filter of the data-gradient convolution
+ * of a stride-1 layer (taps reversed = kernel flipped in both directions, channels
+ * in and out swapped), for spfy_spmma_conv* with pad' = kh - 1 - pad.
+ * rows % 8 == 0 and (cols / taps) % 8 == 0, so every 4x4 block of A maps whole onto
+ * a 4x4 block of A'.  The kept set comes from A's metadata, not from the values: an
+ * A' group keeps the entries A's metadata keeps in that column of the block, with
+ * A's stored bits (+-0 included).  When a group of A' does not get exactly two, the
+ * mask is not transposable: *d_invalid is set to 1 and the output is unspecified.
+ * d_invalid (optional, device int) is zeroed on the stream first; the call never
+ * syncs.  Padding rows / columns of A' hold +0 and the neutral nibble 0x4 (the
+ * output buffers need not be zeroed); A's padding is never read.  The output must
+ * not overlap the input.  Applying the call twice with the same taps gives back
+ * the original bytes.  Refusals: dtype not F16/BF16, rows / cols too large or
+ * rows % 8, (cols / taps) % 8 (SPFY_E_UNSUPPORTED); taps == 0, cols % taps,
+ * null or not 16-byte aligned buffers (SPFY_E_INVALID).
+ * ---------------------------------------------------------------------- */
+SPFY_API int spfy_transpose24(int dtype, const void* vals, const void* meta, size_t rows, size_t cols, size_t taps,
+                              void* vals_t, void* meta_t, int* d_invalid, spfy_stream_t stream);
+/* spfy_recompress24 -- new values under a fixed mask.
+ * in: dense rows x cols (F32, F16 or BF16, row-major, ld_in).  meta: SM100 metadata of
+ * a compressed operand of that shape (read only).  comp_vals (may be NULL): that
+ * operand's values, `dtype` (F16/BF16), rounded to nearest even from `in` at the kept
+ * positions (the bits themselves when in_dtype == dtype); padding +0.  out_masked (may
+ * be NULL, may alias in): `in` with every pruned position set to +0, in in's dtype,
+ * leading dimension ld_out.  One pass: it refreshes the forward operand from an fp32
+ * master after an optimizer step without moving the mask, projects a weight gradient
+ * onto the mask, or re-masks the master in place. */
+SPFY_API int spfy_recompress24(int in_dtype, const void* in, size_t ld_in, int dtype, size_t rows, size_t cols,
+                               const void* meta, void* comp_vals, void* out_masked, size_t ld_out, spfy_stream_t stream);
 
 /* ------------------------------------------------------------------------
  * A4  cusparseLtMatmul                           include/sparsify.me/spmma.hxx:106-114

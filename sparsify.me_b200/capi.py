@@ -15,7 +15,7 @@ LIB_PATH = os.environ.get("SPFY_LIB") or os.path.join(HERE, "lib", "libsparsifym
 
 # enums of include/spfy_b200.h
 F16, BF16, F32, F64 = 0, 1, 2, 3
-PRUNE_STRIP_MAG, PRUNE_TILE_MAG = 0, 1
+PRUNE_STRIP_MAG, PRUNE_TILE_MAG, PRUNE_TILE_TRANSPOSABLE = 0, 1, 2
 LAYOUT_CANONICAL, LAYOUT_SM100 = 0, 1
 OP_N, OP_T = 0, 1
 OUT_T = 0x10  # flag OR-ed into opB: D is written transposed, [n][m]
@@ -52,6 +52,8 @@ SIGNATURES = {
     "spfy_prune24": (c_int, [c_int, c_int, c_int, _P, _SZ, _P, _SZ, _P, _P, _P, _SZ, _SZ, _P]),
     "spfy_prune24_check": (c_int, [c_int, _P, _SZ, _SZ, _SZ, _P, _P]),
     "spfy_prune24_batched": (c_int, [c_int, c_int, c_int, _P, _SZ, _P]),
+    "spfy_transpose24": (c_int, [c_int, _P, _P, _SZ, _SZ, _SZ, _P, _P, _P, _P]),
+    "spfy_recompress24": (c_int, [c_int, _P, _SZ, c_int, _SZ, _SZ, _P, _P, _P, _SZ, _P]),
     "spfy_spmma_workspace_bytes": (c_int, [c_int, _SZ, _SZ, _SZ, POINTER(_SZ)]),
     "spfy_spmma": (c_int, [c_int, c_int, _SZ, _SZ, _SZ, c_float, _P, _P, _P, _SZ, c_float, _P, _SZ,
                            _P, _SZ, _P, _SZ, _P]),

@@ -93,6 +93,7 @@ int spfy_init(void) {
   int rc = device_info(&di);
   if (rc) return rc;
   spfy::warm_prune_kernels();
+  spfy::warm_transpose24_kernels();
   spfy::warm_spmma_kernels();
   spfy::warm_spmm_kernels();
   spfy::warm_gemm_kernels();

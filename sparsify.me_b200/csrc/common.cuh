@@ -132,6 +132,15 @@ template <> __device__ __forceinline__ float from_f32<float>(float v) { return v
 template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
 template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
+// SM100 compressed-operand layout (spfy_b200.h): byte offsets, within a value tile (16 KiB) and a metadata tile (2 KiB),
+// of the 16-byte value chunk and of the 16-bit metadata word of in-tile row r and 16-column unit q.  (prune.cu spells the
+// same sums out inline: in its kernels, folding them into these calls regroups 64-bit address arithmetic and changes
+// their SASS.)
+__host__ __device__ __forceinline__ uint32_t sm100_val_chunk(uint32_t r, uint32_t q) { return r * 128u + ((q ^ (r & 7u)) << 4); }
+__host__ __device__ __forceinline__ uint32_t sm100_meta_word(uint32_t r, uint32_t q) {
+  return (r >> 4) * 256u + (q & 1u) * 128u + (r & 7u) * 16u + (q >> 1) * 4u + ((r >> 3) & 1u) * 2u;
+}
+
 // CUDA loads device code lazily, kernel by kernel, at first use (tens of milliseconds for the big ones).
 // Each translation unit lists its kernels here so that spfy_init() can pay that once, outside anybody's timers.
 template <typename K>
@@ -140,6 +149,7 @@ inline void touch_kernel(K kernel) {
   (void)cudaFuncGetAttributes(&a, kernel);
 }
 void warm_prune_kernels();
+void warm_transpose24_kernels();
 void warm_spmma_kernels();
 void warm_spmm_kernels();
 void warm_gemm_kernels();

@@ -785,7 +785,9 @@ __device__ __forceinline__ void tile_fused_fetch(const Prune24Params& P, uint32_
                : make_uint2(0u, 0u);
 }
 
-template <bool BF16>
+// PATTERN (TILE_TRANSPOSABLE): the nibbles are the tile's pattern itself, so they stay two of four along columns even
+// where a kept value is +-0 (top2of4 on the pruned words may then name another zero); padding gets the neutral nibble.
+template <bool BF16, bool PATTERN>
 __device__ __forceinline__ void tile_fused_tiles(const Prune24Params& P, const TilePatterns& T, uint32_t tr, uint32_t tc,
                                                  bool active, uint32_t lane, const uint2 (&w)[4]) {
   {
@@ -797,7 +799,8 @@ __device__ __forceinline__ void tile_fused_tiles(const Prune24Params& P, const T
       tile_mag2<BF16>(w[i].x, mag[i * 4 + 0], mag[i * 4 + 1]);
       tile_mag2<BF16>(w[i].y, mag[i * 4 + 2], mag[i * 4 + 3]);
     }
-    const TileKeep keep(T.pat[tile_select(mag)]);
+    const uint32_t pat = T.pat[tile_select(mag)];
+    const TileKeep keep(pat);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const uint32_t row = r0 + i;
@@ -807,7 +810,14 @@ __device__ __forceinline__ void tile_fused_tiles(const Prune24Params& P, const T
         *reinterpret_cast<uint2*>(reinterpret_cast<char*>(P.out_dense + c0) + (uint64_t)row * ((uint32_t)P.ld_out * 2u)) =
             make_uint2(lo, hi);
       uint32_t i0, i1;
-      top2of4(lo, hi, i0, i1);
+      if (PATTERN) {
+        const uint32_t nib = (pat >> (4 * i)) & 0xfu;
+        const bool pad = !col_ok || row >= P.rows;
+        i0 = pad ? 0u : __ffs(nib) - 1u;
+        i1 = pad ? 1u : 31u - __clz(nib);
+      } else {
+        top2of4(lo, hi, i0, i1);
+      }
       const uint32_t cv = __byte_perm(lo, hi, (i0 + (i1 << 8)) * 0x22u + 0x1010u);
       // the unit's four nibbles meet in the lane of its first group
       uint32_t nibs = (i0 | i1 << 2) << (4u * (lane & 3u));
@@ -841,11 +851,11 @@ __device__ __forceinline__ void tile_fused_warp(const Prune24Params& P, const Ti
   const uint32_t tc = active ? (uint32_t)(t - (size_t)tr * tiles_c) : 0u;
   uint2 w[4];
   tile_fused_fetch(P, tr, tc, active, w);
-  tile_fused_tiles<BF16>(P, T, tr, tc, active, lane, w);
+  tile_fused_tiles<BF16, false>(P, T, tr, tc, active, lane, w);
 }
 
 // grid: x = 32-tile column chunks, y walks the tile rows with stride 8 * gridDim.y (no division, like prune24_tile_kernel)
-template <bool BF16>
+template <bool BF16, bool PATTERN>
 __global__ void __launch_bounds__(256, 3)
 prune24_tile_fused_kernel(const __grid_constant__ Prune24Params P) {
   __shared__ TilePatterns T;
@@ -865,7 +875,7 @@ prune24_tile_fused_kernel(const __grid_constant__ Prune24Params P) {
 #pragma unroll
     for (int i = 0; i < 4; ++i) w[i] = nw[i];
     tile_fused_fetch(P, tr + tr_step, tcc, col_in && tr + tr_step < tiles_r, nw);  // next tile in flight under this one
-    tile_fused_tiles<BF16>(P, T, tr, tcc, col_in, lane, w);
+    tile_fused_tiles<BF16, PATTERN>(P, T, tr, tcc, col_in, lane, w);
   }
 }
 
@@ -977,6 +987,29 @@ int fill_prune24(Prune24Params* out, int layout, const uint16_t* src, size_t ld_
   return SPFY_OK;
 }
 
+// the one-pass TILE prune + compress (see prune24_tile_fused_kernel)
+template <bool PATTERN>
+static int launch_tile_fused(int dtype, int layout, const uint16_t* src, size_t ld_in, void* out_dense, size_t ld_out,
+                             void* comp_vals, void* meta, size_t rows, size_t cols, cudaStream_t s) {
+  Prune24Params P;
+  int rc = fill_prune24(&P, layout, src, ld_in, out_dense, ld_out, comp_vals, meta, nullptr, rows, cols);
+  if (rc) return rc;
+  const size_t dom_cols = P.tile_order ? (size_t)P.k_tiles * 128 : cols;
+  int blocks = 1;
+  rc = capped_grid(ceil_div(ceil_div((size_t)P.dom_rows, 4) * (dom_cols / 4), 256), 16, &blocks);
+  if (rc) return rc;
+  const size_t fx = ceil_div(dom_cols / 4, 32), fy_all = ceil_div(ceil_div((size_t)P.dom_rows, 4), 8);
+  size_t fy = ceil_div((size_t)blocks, fx);
+  if (fy > fy_all) fy = fy_all;
+  if (fy > 65535) fy = 65535;
+  if (fy == 0) fy = 1;
+  const dim3 grid((unsigned)fx, (unsigned)fy);
+  if (dtype == SPFY_BF16) prune24_tile_fused_kernel<true, PATTERN><<<grid, 256, 0, s>>>(P);
+  else prune24_tile_fused_kernel<false, PATTERN><<<grid, 256, 0, s>>>(P);
+  SPFY_LAUNCH_OK("prune24_tile_fused_kernel");
+  return SPFY_OK;
+}
+
 }  // namespace
 }  // namespace spfy
 
@@ -993,8 +1026,10 @@ void spfy::warm_prune_kernels() {
   touch_kernel(prune24_tile_kernel<false, true>);
   touch_kernel(prune24_tile_kernel<true, false>);
   touch_kernel(prune24_tile_kernel<true, true>);
-  touch_kernel(prune24_tile_fused_kernel<false>);
-  touch_kernel(prune24_tile_fused_kernel<true>);
+  touch_kernel(prune24_tile_fused_kernel<false, false>);
+  touch_kernel(prune24_tile_fused_kernel<true, false>);
+  touch_kernel(prune24_tile_fused_kernel<false, true>);
+  touch_kernel(prune24_tile_fused_kernel<true, true>);
   touch_kernel(prune24_check_kernel);
 }
 
@@ -1066,11 +1101,16 @@ int spfy_compressed_bytes(int dtype, size_t rows, size_t cols, int layout, size_
   return SPFY_OK;
 }
 
+// can the one-pass prune + compress kernel take these buffers?
+static bool tile_fused_shape_ok(const void* in, size_t ld_in, const void* out_dense, size_t ld_out, const void* comp_vals,
+                                const void* meta, size_t cols) {
+  const bool vec = cols % 4 == 0 && ld_in % 4 == 0 && ld_out % 4 == 0 && (uintptr_t)in % 8 == 0 && (uintptr_t)out_dense % 8 == 0;
+  return vec && cols % 16 == 0 && (uintptr_t)meta % 2 == 0 && (uintptr_t)comp_vals % 4 == 0;
+}
 // can this TILE_MAG request go through the one-pass prune + compress kernel?
 static bool tile_fused_ok(const void* in, size_t ld_in, const void* out_dense, size_t ld_out, const void* comp_vals,
                           const void* meta, const uint64_t* mask, size_t cols) {
-  const bool vec = cols % 4 == 0 && ld_in % 4 == 0 && ld_out % 4 == 0 && (uintptr_t)in % 8 == 0 && (uintptr_t)out_dense % 8 == 0;
-  return (comp_vals || meta) && !mask && vec && cols % 16 == 0 && (uintptr_t)meta % 2 == 0 && (uintptr_t)comp_vals % 4 == 0;
+  return (comp_vals || meta) && !mask && tile_fused_shape_ok(in, ld_in, out_dense, ld_out, comp_vals, meta, cols);
 }
 
 int spfy_prune24(int dtype, int mode, int layout, const void* in, size_t ld_in, void* out_dense,
@@ -1101,26 +1141,8 @@ int spfy_prune24(int dtype, int mode, int layout, const void* in, size_t ld_in, 
       const char* e = dev_switch("SPFY_TILE_FUSED_MAX");
       return e ? (size_t)strtoull(e, nullptr, 10) : (size_t)8 << 20;
     }();
-    if (tile_fused_ok(src, ld_in, out_dense, ld_out, comp_vals, meta, mask, cols) && rows * cols <= fused_max) {
-      // one pass: prune + compress (see prune24_tile_fused_kernel)
-      Prune24Params P;
-      int rcf = fill_prune24(&P, layout, src, ld_in, out_dense, ld_out, comp_vals, meta, nullptr, rows, cols);
-      if (rcf) return rcf;
-      const size_t dom_cols = P.tile_order ? (size_t)P.k_tiles * 128 : cols;
-      int blocksf = 1;
-      rcf = capped_grid(ceil_div(ceil_div((size_t)P.dom_rows, 4) * (dom_cols / 4), 256), 16, &blocksf);
-      if (rcf) return rcf;
-      const size_t fx = ceil_div(dom_cols / 4, 32), fy_all = ceil_div(ceil_div((size_t)P.dom_rows, 4), 8);
-      size_t fy = ceil_div((size_t)blocksf, fx);
-      if (fy > fy_all) fy = fy_all;
-      if (fy > 65535) fy = 65535;
-      if (fy == 0) fy = 1;
-      const dim3 gridf((unsigned)fx, (unsigned)fy);
-      if (dtype == SPFY_BF16) prune24_tile_fused_kernel<true><<<gridf, 256, 0, s>>>(P);
-      else prune24_tile_fused_kernel<false><<<gridf, 256, 0, s>>>(P);
-      SPFY_LAUNCH_OK("prune24_tile_fused_kernel");
-      return SPFY_OK;
-    }
+    if (tile_fused_ok(src, ld_in, out_dense, ld_out, comp_vals, meta, mask, cols) && rows * cols <= fused_max)
+      return launch_tile_fused<false>(dtype, layout, src, ld_in, out_dense, ld_out, comp_vals, meta, rows, cols, s);
     int blocks = 1;
     int rc = capped_grid(ceil_div(ceil_div(rows, 4) * ceil_div(cols, 4), 256), 16, &blocks);  // cap: two waves of resident warps
     if (rc) return rc;
@@ -1147,6 +1169,13 @@ int spfy_prune24(int dtype, int mode, int layout, const void* in, size_t ld_in, 
     src = (const uint16_t*)out_dense;
     ld_src = ld_out;
     out_dense = nullptr;
+  } else if (mode == SPFY_PRUNE_TILE_TRANSPOSABLE) {
+    if (!out_dense)
+      return fail(SPFY_E_INVALID, "prune24: TILE_TRANSPOSABLE needs out_dense (it may alias the input)");
+    if (mask) return fail(SPFY_E_UNSUPPORTED, "prune24: TILE_TRANSPOSABLE writes no mask");
+    if (!tile_fused_shape_ok(src, ld_in, out_dense, ld_out, comp_vals, meta, cols))
+      return fail(SPFY_E_UNSUPPORTED, "prune24: TILE_TRANSPOSABLE needs cols %% 16 == 0 and 8-byte aligned rows");
+    return launch_tile_fused<true>(dtype, layout, src, ld_in, out_dense, ld_out, comp_vals, meta, rows, cols, s);
   } else if (mode != SPFY_PRUNE_STRIP_MAG) {
     return fail(SPFY_E_INVALID, "prune24: bad mode %d", mode);
   }

@@ -802,10 +802,12 @@ int make_tmap_im2col(CUtensorMap* map, int dtype, const void* x, const spfy_conv
   int lower[2] = {-(int)c.pad, -(int)c.pad};
   int upper[2] = {(int)c.pad - (int)(c.kw - 1), (int)c.pad - (int)(c.kh - 1)};
   cuuint32_t estr[4] = {1, (cuuint32_t)c.stride, (cuuint32_t)c.stride, 1};
-  CUresult r = enc(map, dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4,
-                   const_cast<void*>(x), dims, strides, lower, upper, /*channelsPerPixel*/ 64, /*pixelsPerColumn*/ BN, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = encode_with_context([&] {
+    return enc(map, dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4,
+               const_cast<void*>(x), dims, strides, lower, upper, /*channelsPerPixel*/ 64, /*pixelsPerColumn*/ BN, estr,
+               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  });
   if (r != CUDA_SUCCESS)
     return fail(SPFY_E_CUDA, "cuTensorMapEncodeIm2col failed (%d) for NHWC %zu x %zu x %zu x %zu, filter %zu x %zu stride %zu pad %zu",
                 (int)r, c.batch, c.h, c.w, c.c, c.kh, c.kw, c.stride, c.pad);

@@ -428,6 +428,16 @@ inline int get_encoder(EncodeTiledFn* out) {
   return SPFY_OK;
 }
 
+// The encoders need a current context.  A thread that has made no runtime call that needs one -- torch's autograd
+// backward threads, for one -- has none and gets CUDA_ERROR_INVALID_CONTEXT: bind the device's primary context (any
+// such runtime call does) and encode once more.
+template <typename Encode>
+inline CUresult encode_with_context(Encode&& encode) {
+  CUresult r = encode();
+  if (r == CUDA_ERROR_INVALID_CONTEXT && cudaFree(nullptr) == cudaSuccess) r = encode();
+  return r;
+}
+
 // A tiled tensor map of `rank` <= 3 dimensions, innermost first (`byte_strides` has rank - 1 entries): element strides 1,
 // no interleave, L2 promotion in 256-byte lines, out-of-bounds elements read as zero.
 inline int encode_tiled(CUtensorMap* map, int dtype, uint32_t rank, const void* base, const cuuint64_t* dims,
@@ -439,8 +449,10 @@ inline int encode_tiled(CUtensorMap* map, int dtype, uint32_t rank, const void* 
   const CUtensorMapDataType dt = dtype == SPFY_F32    ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
                                  : dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
                                                       : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  const CUresult r = enc(map, dt, rank, const_cast<void*>(base), dims, byte_strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  const CUresult r = encode_with_context([&] {
+    return enc(map, dt, rank, const_cast<void*>(base), dims, byte_strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
+               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  });
   if (r != CUDA_SUCCESS)
     return fail(SPFY_E_CUDA, "%s: cuTensorMapEncodeTiled failed (%d) for dims %llu x %llu x %llu, row pitch %llu bytes", who,
                 (int)r, (unsigned long long)dims[0], (unsigned long long)dims[1],

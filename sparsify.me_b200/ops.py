@@ -304,6 +304,137 @@ class SpmmaPlan:
             pass
 
 
+# --------------------------------------------------------------------- 2:4 fine-tuning
+def transpose24(comp, taps=1, out=None, invalid=None):
+    """spfy_transpose24: the compressed operand of A' [cols/taps, taps*rows] from the compressed A [rows, cols],
+        A'[ci][t'*rows + r] = A[r][(taps-1-t')*cols/taps + ci].
+    taps=1: A' = A^T, the operand of a Linear layer's data gradient, dx = dy W:
+        spmma_compressed(transpose24(comp), dy, op_b=OP_T, out_t=True)
+    taps=kh*kw (weights permuted with permute_conv_weights before pruning): A' is the flipped, channel-swapped filter
+    of a stride-1 convolution's data gradient, with dy and dx in NHWC:
+        spmma_conv_nhwc(transpose24(comp, taps=kh * kw), dy, kh, kw, stride=1, pad=kh - 1 - pad)
+    A's mask must keep two of four along columns too (PRUNE_TILE_TRANSPOSABLE, or TILE_MAG on weights without zeros).
+    `invalid`: optional int32 CUDA tensor, set to 0, or to 1 when the mask is not transposable (the result is then
+    unspecified).  Nothing here syncs.  Returns a Compressed24 (== out when given)."""
+    assert comp.layout == capi.LAYOUT_SM100
+    if comp.cols % taps:
+        raise capi.SpfyError(capi.E_INVALID, "transpose24", f"cols {comp.cols} is not a multiple of taps {taps}")
+    rows_t, cols_t = comp.cols // taps, taps * comp.rows
+    if out is None:
+        out = alloc_compressed(comp.dtype, rows_t, cols_t, comp.vals.device)
+    assert (out.rows, out.cols, out.dtype, out.layout) == (rows_t, cols_t, comp.dtype, capi.LAYOUT_SM100)
+    if invalid is not None:
+        assert invalid.dtype == torch.int32 and invalid.is_cuda
+    capi.spfy_transpose24(_DT[comp.dtype], _ptr(comp.vals), _ptr(comp.meta), comp.rows, comp.cols, taps,
+                          _ptr(out.vals), _ptr(out.meta), _ptr(invalid), _stream())
+    return out
+
+
+def recompress24(dense, comp, masked_out=None, values=True):
+    """spfy_recompress24: new values under comp's fixed mask.  `dense` [comp.rows, comp.cols] (fp32, fp16 or bf16,
+    row-major).  values=True: comp.vals <- dense at the positions comp.meta keeps, rounded to nearest even to comp.dtype
+    (the metadata is not touched).  masked_out (may be `dense`): dense with every pruned position set to +0.
+    The three jobs of a fine-tuning step: refresh the forward operand from an fp32 master, project a weight gradient
+    onto the mask, re-mask the master in place."""
+    assert comp.layout == capi.LAYOUT_SM100 and dense.dim() == 2 and dense.stride(1) == 1
+    assert tuple(dense.shape) == (comp.rows, comp.cols)
+    if masked_out is not None:
+        assert masked_out.dtype == dense.dtype and masked_out.shape == dense.shape and masked_out.stride(1) == 1
+    capi.spfy_recompress24(_dtype_code(dense), _ptr(dense), dense.stride(0), _DT[comp.dtype], comp.rows, comp.cols,
+                           _ptr(comp.meta), _ptr(comp.vals) if values else None, _ptr(masked_out),
+                           masked_out.stride(0) if masked_out is not None else 0, _stream())
+
+
+class _Linear24Fn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x2, weight, bias, layer):
+        del weight  # the forward operand is layer.comp; weight is an input so that its gradient reaches it
+        ctx.layer = layer
+        ctx.save_for_backward(x2)
+        ctx.has_bias = bias is not None
+        return spmma_compressed(layer.comp, x2, op_b=capi.OP_T, out_t=True,
+                                epilogue=Epilogue(bias=bias.detach()) if bias is not None else None)
+
+    @staticmethod
+    def backward(ctx, dy):
+        (x2,) = ctx.saved_tensors
+        layer = ctx.layer
+        dy = dy.to(layer.dtype).contiguous()
+        tokens, out_f = dy.shape
+        in_f = x2.shape[1]
+        dx = None
+        if ctx.needs_input_grad[0]:
+            dx = spmma_compressed(layer.comp_t, dy, op_b=capi.OP_T, out_t=True)  # dy W on sparse tensor cores
+        dw = None
+        if ctx.needs_input_grad[1]:
+            # dW [out, in] = dy^T x: column-major m = in, n = out, k = tokens on the dense tcgen05 GEMM, then masked
+            dt = _DT[layer.dtype]
+            dw = torch.empty(out_f, in_f, dtype=layer.dtype, device=dy.device)
+            wb = ctypes.c_size_t()
+            capi.spfy_gemm_workspace_bytes(dt, capi.OP_N, capi.OP_T, in_f, out_f, tokens, in_f, out_f, 1, ctypes.byref(wb))
+            ws = _workspace(wb.value, dy.device)
+            capi.spfy_gemm_strided_batched(dt, capi.GEMM_PRECISE, capi.OP_N, capi.OP_T, in_f, out_f, tokens, 1.0,
+                                           _ptr(x2), in_f, 0, _ptr(dy), out_f, 0, 0.0, _ptr(dw), in_f, 0, 1,
+                                           _ptr(ws), ws.numel(), _stream())
+            recompress24(dw, layer.comp, masked_out=dw, values=False)
+            dw = dw.float()
+        db = dy.float().sum(0) if ctx.has_bias and ctx.needs_input_grad[2] else None
+        return dx, dw, db, None
+
+
+class Linear24(torch.nn.Module):
+    """A 2:4 Linear layer for fine-tuning with a fixed mask, y = x W^T + b, on sparse tensor cores forward and backward.
+    State: `weight`, the fp32 master [out, in], kept masked; `bias` (fp32, optional); `comp` and `comp_t`, the 16-bit
+    compressed W and W^T.  The mask is chosen once, by PRUNE_TILE_TRANSPOSABLE, so that W^T is a 2:4 operand as well.
+      forward : spmma(comp, x) with the bias in the epilogue; x is [..., in] in `dtype`, and the flattened leading
+                dimensions must be a multiple of 8
+      backward: dx = dy W through comp_t (sparse tensor cores); dW = dy^T x on the dense tcgen05 GEMM, masked, fp32;
+                db = sum of dy
+    After optimizer.step(), call refresh(): it re-masks the master in place and rebuilds comp and comp_t from it (the
+    mask does not move).  forward refuses to run on a weight changed since the last refresh.  An NHWC 1x1 stride-1
+    convolution is this layer applied to the [..., channels] activation."""
+
+    def __init__(self, weight, bias, comp, comp_t, dtype):
+        super().__init__()
+        self.weight = torch.nn.Parameter(weight)
+        self.bias = torch.nn.Parameter(bias) if bias is not None else None
+        self.comp, self.comp_t, self.dtype = comp, comp_t, dtype
+        self._synced_version = self.weight._version
+
+    @classmethod
+    def from_dense(cls, w, b=None, dtype=torch.float16):
+        """Prune `w` [out, in] (out and in multiples of 8, in a multiple of 16) with PRUNE_TILE_TRANSPOSABLE in
+        `dtype`.  Raises ValueError if the mask is not transposable (one sync, here only)."""
+        with torch.no_grad():
+            w16 = w.detach().to(dtype).contiguous()
+            comp = prune24(w16, inplace=True, mode=capi.PRUNE_TILE_TRANSPOSABLE)
+            master = w.detach().float().contiguous().clone()
+            recompress24(master, comp, masked_out=master, values=False)
+            invalid = torch.empty(1, dtype=torch.int32, device=w.device)
+            comp_t = transpose24(comp, invalid=invalid)
+            if int(invalid.item()):
+                raise ValueError("Linear24: the pruned mask is not transposable")
+            bias = b.detach().float().contiguous().clone() if b is not None else None
+        return cls(master, bias, comp, comp_t, dtype)
+
+    @torch.no_grad()
+    def refresh(self):
+        """master -> comp.vals (mask fixed), master re-masked in place, comp -> comp_t.  No sync."""
+        recompress24(self.weight, self.comp, masked_out=self.weight)
+        transpose24(self.comp, out=self.comp_t)
+        self._synced_version = self.weight._version
+
+    def forward(self, x):
+        if self.weight._version != self._synced_version:
+            raise RuntimeError("Linear24: weight changed since the last refresh(); call refresh() after optimizer.step()")
+        in_f = self.comp.cols
+        x2 = x.reshape(-1, in_f).contiguous()
+        if x2.dtype != self.dtype:
+            raise TypeError(f"Linear24: input dtype {x2.dtype}, layer dtype {self.dtype}")
+        y = _Linear24Fn.apply(x2, self.weight, self.bias, self)
+        return y.view(*x.shape[:-1], self.comp.rows)
+
+
 # ----------------------------------------------------------------------------- A4
 def spmma_compressed(comp, b, c=None, out=None, alpha=1.0, beta=0.0, op_b=capi.OP_N, out_t=False, epilogue=None):
     """D = alpha * A(2:4) * op(B) + beta * C on tcgen05.mma.sp (cusparseLtMatmul, spmma.hxx:106-114).
