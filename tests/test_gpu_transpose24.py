@@ -51,7 +51,9 @@ def operand_from_mask(bits, keep):
     order = np.argsort(~kq, axis=-1, kind="stable")[..., :2]
     vals = np.take_along_axis(bits.reshape(rows, cols // 4, 4), order, -1).reshape(rows, -1)
     nib = (order[..., 0] | (order[..., 1] << 2)).astype(np.uint8)
-    return vals, (nib[:, 0::2] | (nib[:, 1::2] << 4)).astype(np.uint8)
+    meta = nib[:, 0::2].copy()  # an odd last group: low nibble only
+    meta[:, : nib.shape[1] // 2] |= nib[:, 1::2] << 4
+    return vals, meta
 
 
 # ------------------------------------------------------------------ transpose24

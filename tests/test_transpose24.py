@@ -58,6 +58,18 @@ def expected_sm100(orc, dtype, dense, taps):
     return orc.pack_sm100(ref["vals"], ref["meta"], *t.shape)
 
 
+def move_kept_pair(dense, bits, row, group):
+    """TILE-pruned zero-free `dense` with row `row` of group `group` keeping the other two of its four positions (their
+    values from `bits`, zero-free): the row stays 2:4, but two columns of that 4x4 block now keep three and two keep
+    one, so the mask is no longer transposable."""
+    out = dense.copy()
+    cs = slice(4 * group, 4 * group + 4)
+    kept = out[row, cs] != 0
+    assert kept.sum() == 2 and (bits[row, cs] != 0).all()
+    out[row, cs] = np.where(kept, 0, bits[row, cs])
+    return out
+
+
 def test_new_symbols_are_declared_exported_and_bound(spfy):
     from test_boundary import declared_symbols
     names = declared_symbols()
@@ -125,7 +137,8 @@ def test_refusals_need_no_device(spfy):
 
 
 @pytest.mark.parametrize("rows,cols,taps", [(8, 8, 1), (200, 72, 1), (64, 576, 1), (64, 576, 9), (136, 9 * 24, 9),
-                                            (256, 512, 4)])
+                                            (256, 512, 4), (8, 16, 1), (8, 16, 2), (128, 9 * 64, 9), (72, 9 * 64, 9),
+                                            (64, 9 * 128, 9), (64, 25 * 64, 25), (64, 49 * 64, 49)])
 @pytest.mark.parametrize("dtype", [0, 1])
 def test_transpose_rule_matches_the_oracle(orc, rows, cols, taps, dtype):
     dense = tile_pruned(orc, dtype, rows, cols, seed=rows * 31 + cols + taps)
@@ -145,3 +158,17 @@ def test_transpose_rule_flags_a_strip_mask(orc):
     bits = orc.from_f32(0, rng.uniform(0.25, 1.0, (64, 64)).astype(np.float32))
     a = orc.prune24_strip(0, bits, want_mask=False)
     assert transpose24_canonical(a["vals"], a["meta"], 64, 64, 1)[2] == 1
+
+
+@pytest.mark.parametrize("rows,cols,row,group", [(64, 64, 0, 0), (64, 64, 37, 9), (200, 136, 199, 33)])
+def test_transpose_rule_flags_one_moved_pair(orc, rows, cols, row, group):
+    """one row of one 4x4 block keeping the other two positions: still 2:4 along rows, flagged by the rule"""
+    rng = np.random.default_rng(rows + row)
+    bits = orc.from_f32(0, (rng.uniform(0.25, 1.0, (rows, cols)) * rng.choice([-1.0, 1.0], (rows, cols)))
+                        .astype(np.float32))
+    dense = orc.prune24_tile(0, bits)[0]
+    moved = move_kept_pair(dense, bits, row, group)
+    assert orc.prune24_check(0, moved) == 0
+    a = orc.prune24_strip(0, moved, want_mask=False)
+    assert np.array_equal(a["dense"], moved)
+    assert transpose24_canonical(a["vals"], a["meta"], rows, cols, 1)[2] == 1
