@@ -185,6 +185,34 @@ SPFY_API int spfy_prune24_check(int dtype, const void* in, size_t ld_in, size_t 
  * ---------------------------------------------------------------------- */
 SPFY_API int spfy_transpose24(int dtype, const void* vals, const void* meta, size_t rows, size_t cols, size_t taps,
                               void* vals_t, void* meta_t, int* d_invalid, spfy_stream_t stream);
+/* spfy_transpose24_conv -- the filter operands of a STRIDED convolution's data gradient.
+ * A: the forward filter, SM100-layout compressed m x (kh*kw*c) in (kh, kw, c) order
+ * (spfy_permute_conv_weights, then SPFY_PRUNE_TILE_TRANSPOSABLE).  The data gradient
+ * of a stride-s layer splits by output phase (a, b) = (ih mod s, iw mod s).  In one
+ * dimension phase a takes the taps T_a = {kh : (a + pad - kh) mod s == 0} in
+ * descending order, and
+ *     dx[s*i + a] = sum over kh in T_a of dy[i + (a + pad - kh)/s] * W[kh]
+ * (dy outside the image counts as 0): a stride-1 correlation of dy.  For each phase
+ * with taps in both dimensions, in (a, b) row-major order, the call writes the
+ * SM100-layout compressed c x (|T_a|*|T_b|*m) operand
+ *     A'_ab[ci][(th*|T_b| + tw)*m + r] = A[r][(kh(th)*kw + kw(tw))*c + ci]
+ * (th, tw: positions in T_a, T_b).  The operands lie back to back in vals_t / meta_t,
+ * each starting on a tile boundary: phase p at tile sum over earlier phases of
+ * ceil(c/128) * ceil(|T_a|*|T_b|*m/128) (16384 value and 2048 metadata bytes per
+ * tile); spfy_transpose24_conv_bytes gives the totals.  A phase with no taps gets no
+ * operand (1x1 stride 2: three of the four).  For s = 1 the output is byte for byte
+ * spfy_transpose24(taps = kh*kw).  With a TILE-transposable mask every tap's slice of
+ * the transposed filter is a valid 2:4 operand, so any subset of taps is too: nothing
+ * is pruned again.  Otherwise as spfy_transpose24: *d_invalid (optional) is zeroed and
+ * set to 1 for a mask that is not transposable, padding is +0 with nibble 0x4, the
+ * output buffers need not be zeroed, one launch, no sync.  Refusals: dtype not
+ * F16/BF16, m % 8, c % 8, kh or kw > 16, pad > 8, stride > 8 (SPFY_E_UNSUPPORTED);
+ * an empty dimension, null or not 16-byte aligned buffers (SPFY_E_INVALID). */
+SPFY_API int spfy_transpose24_conv_bytes(int dtype, size_t m, size_t c, size_t kh, size_t kw, size_t stride, size_t pad,
+                                         size_t* vals_bytes, size_t* meta_bytes);
+SPFY_API int spfy_transpose24_conv(int dtype, const void* vals, const void* meta, size_t m, size_t c, size_t kh,
+                                   size_t kw, size_t stride, size_t pad, void* vals_t, void* meta_t, int* d_invalid,
+                                   spfy_stream_t stream);
 /* spfy_recompress24 -- new values under a fixed mask.
  * in: dense rows x cols (F32, F16 or BF16, row-major, ld_in).  meta: SM100 metadata of
  * a compressed operand of that shape (read only).  comp_vals (may be NULL): that
@@ -270,6 +298,20 @@ SPFY_API int spfy_spmma_conv_ex(int dtype, const spfy_conv_desc* conv, size_t m,
                                 const void* comp_vals, const void* meta, const void* X, float beta,
                                 const void* C, size_t ldc, void* D, size_t ldd, int layout,
                                 const spfy_epilogue* epi, spfy_stream_t stream);
+/* spfy_spmma_conv_dgrad -- the data gradient of a convolution of any stride on sparse tensor cores:
+ *     dX = alpha * conv2d_input(W, dY) + beta * dX
+ * conv: the FORWARD layer (its h and w say which dX a floor-divided dY belongs to).  dY: NHWC [batch][ho][wo][m];
+ * dX: NHWC [batch][h][w][c], contiguous.  vals_t / meta_t: spfy_transpose24_conv of the layer's m x (kh*kw*c) filter.
+ * Each phase (a, b) with taps is one implicit GEMM, M = c, K = |T_a|*|T_b|*m, N = batch * H_a * W_b (H_a = ceil((h -
+ * a) / s)), whose im2col map walks dY with stride 1 from the phase's first offset, and whose NHWC output rows land on
+ * the pixels (s*i + a, s*j + b) of dX.  Every dX element is written: positions no tap reaches get beta * dX (+0 for beta
+ * = 0, nothing at all is written for beta = 1).  beta = 1 accumulates in place, e.g. where the shortcut's and the main
+ * branch's data gradients meet at a residual block's input.  A phase is one launch (the launches of one call may
+ * overlap: they write disjoint pixels); no device allocation, no sync.  Refusals: dtype not F16/BF16, m % 64, c % 8,
+ * kh or kw > 16, pad > 8, stride > 8, im2col corners of a phase outside [-128, 127] (SPFY_E_UNSUPPORTED); an empty
+ * dimension, a filter larger than the padded image, null or not 16-byte aligned buffers (SPFY_E_INVALID). */
+SPFY_API int spfy_spmma_conv_dgrad(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* vals_t,
+                                   const void* meta_t, const void* dY, float beta, void* dX, spfy_stream_t stream);
 /* weights [m][c * kh * kw] in (c, kh, kw) column order (what torch's unfold / a flattened conv weight uses)
  * -> [m][kh * kw * c] in (kh, kw, c) order; 16-bit elements */
 SPFY_API int spfy_permute_conv_weights(const void* in, void* out, size_t m, size_t c, size_t kh, size_t kw,

@@ -26,12 +26,13 @@ from .capi import (F16, BF16, F32, F64, PRUNE_STRIP_MAG, PRUNE_TILE_MAG, PRUNE_T
 from .ops import (sparsify, prune24, prune24_check, compressed_bytes, spmma_compressed, spmma,  # noqa: F401
                   threshold_to_coo, coo_to_csr, batched, Compressed24, SpmmaPlan, prune24_batched,
                   alloc_compressed, pack_compressed, unpack_compressed, spmma_conv, spmma_conv_nhwc, permute_conv_weights,
-                  Epilogue, fold_batchnorm, transpose24, recompress24, Linear24)
+                  Epilogue, fold_batchnorm, transpose24, recompress24, Linear24,
+                  Transpose24Conv, transpose24_conv, spmma_conv_dgrad_nhwc)
 from . import shapes  # noqa: F401
 from . import multigpu  # noqa: F401
 
 __all__ = [
     "capi", "sparsify", "prune24", "prune24_check", "compressed_bytes", "spmma_compressed", "spmma",
-    "threshold_to_coo", "coo_to_csr", "batched", "Compressed24", "SpmmaPlan", "prune24_batched", "alloc_compressed", "Epilogue", "fold_batchnorm", "transpose24", "recompress24", "Linear24", "pack_compressed", "unpack_compressed", "shapes", "multigpu", "SpfyError",
+    "threshold_to_coo", "coo_to_csr", "batched", "Compressed24", "SpmmaPlan", "prune24_batched", "alloc_compressed", "Epilogue", "fold_batchnorm", "transpose24", "recompress24", "Linear24", "Transpose24Conv", "transpose24_conv", "spmma_conv_dgrad_nhwc", "pack_compressed", "unpack_compressed", "shapes", "multigpu", "SpfyError",
     "launch_count", "last_error", "version",
 ]

@@ -54,6 +54,8 @@ SIGNATURES = {
     "spfy_prune24_batched": (c_int, [c_int, c_int, c_int, _P, _SZ, _P]),
     "spfy_transpose24": (c_int, [c_int, _P, _P, _SZ, _SZ, _SZ, _P, _P, _P, _P]),
     "spfy_recompress24": (c_int, [c_int, _P, _SZ, c_int, _SZ, _SZ, _P, _P, _P, _SZ, _P]),
+    "spfy_transpose24_conv_bytes": (c_int, [c_int, _SZ, _SZ, _SZ, _SZ, _SZ, _SZ, POINTER(_SZ), POINTER(_SZ)]),
+    "spfy_transpose24_conv": (c_int, [c_int, _P, _P, _SZ, _SZ, _SZ, _SZ, _SZ, _SZ, _P, _P, _P, _P]),
     "spfy_spmma_workspace_bytes": (c_int, [c_int, _SZ, _SZ, _SZ, POINTER(_SZ)]),
     "spfy_spmma": (c_int, [c_int, c_int, _SZ, _SZ, _SZ, c_float, _P, _P, _P, _SZ, c_float, _P, _SZ,
                            _P, _SZ, _P, _SZ, _P]),
@@ -62,6 +64,7 @@ SIGNATURES = {
     "spfy_spmma_ex": (c_int, [c_int, c_int, _SZ, _SZ, _SZ, c_float, _P, _P, _P, _SZ, c_float, _P, _SZ,
                               _P, _SZ, _P, _SZ, _P, _P]),
     "spfy_spmma_conv_ex": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _SZ, _P, _SZ, c_int, _P, _P]),
+    "spfy_spmma_conv_dgrad": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _P]),
     "spfy_permute_conv_weights": (c_int, [_P, _P, _SZ, _SZ, _SZ, _SZ, _P]),
     "spfy_spmma_plan_create": (c_int, [c_int, _P, _SZ, POINTER(c_void_p)]),
     "spfy_spmma_plan_create_replicated": (c_int, [c_int, _P, _SZ, _SZ, _P, POINTER(c_void_p)]),

@@ -141,6 +141,25 @@ __host__ __device__ __forceinline__ uint32_t sm100_meta_word(uint32_t r, uint32_
   return (r >> 4) * 256u + (q & 1u) * 128u + (r & 7u) * 16u + (q >> 1) * 4u + ((r >> 3) & 1u) * 2u;
 }
 
+// The data gradient of a stride-s convolution, split by output phase (spfy_transpose24_conv, spfy_spmma_conv_dgrad).  In
+// one spatial dimension of a k-tap filter with padding p, the dx rows ih = s*i + a (0 <= a < s) are
+//     dx[s*i + a] = sum over the taps kt = k0, k0 - s, ..., k0 - (taps-1)*s of dy[i + d0 + t] * W[kt],   t = 0, 1, ...
+// (dy outside [0, ho) counts as 0): a stride-1 correlation of dy with the phase's taps in descending order.  taps == 0:
+// no tap reaches the phase.
+struct DgradPhase {
+  uint32_t taps;  // taps of the phase
+  uint32_t k0;    // its largest filter index
+  int d0;         // offset into dy of its first tap (k0): (a + p - k0) / s, exact
+};
+inline DgradPhase dgrad_phase(size_t k, size_t s, size_t p, size_t a) {
+  const size_t r = (a + p) % s;  // the filter indices of phase a are r, r + s, ...
+  if (r >= k) return DgradPhase{0u, 0u, 0};
+  const size_t k0 = r + (k - 1 - r) / s * s;
+  return DgradPhase{(uint32_t)((k0 - r) / s + 1), (uint32_t)k0, ((int)a + (int)p - (int)k0) / (int)s};
+}
+// dx rows (or columns) of phase a: ceil((h - a) / s)
+inline size_t dgrad_phase_extent(size_t h, size_t s, size_t a) { return h > a ? (h - a + s - 1) / s : 0; }
+
 // CUDA loads device code lazily, kernel by kernel, at first use (tens of milliseconds for the big ones).
 // Each translation unit lists its kernels here so that spfy_init() can pay that once, outside anybody's timers.
 template <typename K>

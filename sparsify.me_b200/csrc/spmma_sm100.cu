@@ -103,7 +103,8 @@ struct alignas(64) ProblemDev {
   uint32_t conv;               // 0: B is a matrix
   uint32_t conv_c, conv_kw;    // channels (multiple of 64), filter width
   uint32_t conv_wo, conv_ho;   // output width / height
-  uint32_t conv_stride, conv_pad;
+  uint32_t conv_stride;
+  int32_t conv_off_h, conv_off_w;  // base pixel of output position (0, 0): -pad, or a data-gradient phase's dy offset
   // epilogue of the _ex entry points: v = (alpha * scale[row]) * acc + beta * C + bias[row], D = act(v).  epi != 0 selects
   // the epilogue code that applies it (also taken for beta != 0 with the transposed output, whose C is [n][m] like D);
   // epi == 0 runs the alpha / beta code of the plain entry points, unchanged.
@@ -111,6 +112,12 @@ struct alignas(64) ProblemDev {
   const float* bias;   // [m] or null
   uint32_t act;        // SPFY_ACT_*
   uint32_t epi;
+  // scattered NHWC output (spfy_spmma_conv_dgrad, kernels instantiated with SCATTER): position (image, i, j) of the
+  // [batch][conv_ho][conv_wo] grid is the row ((image * sc_h + sc_s * i + sc_a) * sc_w + sc_s * j + sc_b) of D [.][ldd],
+  // which is written with 16-byte stores instead of through tmap_d (and C, when beta != 0, read at the same row)
+  void* D;
+  uint64_t ldd;
+  uint32_t sc_h, sc_w, sc_s, sc_a, sc_b;
 };
 
 struct LaunchParams {
@@ -155,6 +162,12 @@ __device__ __forceinline__ float gelu_tanh(float x) {
   float t;
   asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.7978845608028654f * fmaf(0.044715f * x, x * x, x)));
   return 0.5f * x * (1.f + t);
+}
+
+// scattered output: the D (or C) row of position n of the problem's [batch][conv_ho][conv_wo] grid
+__device__ __forceinline__ size_t scatter_row(const ProblemDev* P, uint32_t n) {
+  const uint32_t t = n / P->conv_wo, j = n - t * P->conv_wo, img = t / P->conv_ho, i = t - img * P->conv_ho;
+  return ((size_t)img * P->sc_h + P->sc_s * i + P->sc_a) * P->sc_w + P->sc_s * j + P->sc_b;
 }
 
 // All three roles walk the same sequence of units: u = blockIdx.x, blockIdx.x + gridDim.x, ...
@@ -236,7 +249,8 @@ struct UnitWalker {
 // ------------------------------------------------------------------- kernel
 // EPI: some problem of the launch has an epilogue (ProblemDev::epi).  A launch without one compiles to the code the kernel
 // had before epilogues existed (152 registers instead of 168, measured 0.3-1 % faster on the ResNet-50 plans).
-template <bool BF16, bool OPB_T, bool EPI>
+// SCATTER: the transposed output goes to scattered rows (ProblemDev::D, spfy_spmma_conv_dgrad); only with OPB_T and EPI.
+template <bool BF16, bool OPB_T, bool EPI, bool SCATTER>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ LaunchParams L) {
   extern __shared__ uint8_t smem_raw[];
@@ -295,7 +309,8 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
       const CUtensorMap* tmap_b = nullptr;
       const uint8_t *a_vals = nullptr, *a_meta = nullptr;
       uint32_t pm = 0, k_tiles = 0, m_tiles = 0, G = 1, resident = 0, b3d = 0;
-      uint32_t conv = 0, conv_c = 64, conv_kw = 1, conv_wo = 1, conv_ho = 1, conv_stride = 1, conv_pad = 0, pk = 0;
+      uint32_t conv = 0, conv_c = 64, conv_kw = 1, conv_wo = 1, conv_ho = 1, conv_stride = 1, pk = 0;
+      int conv_off_h = 0, conv_off_w = 0;
       uint64_t hint_b = 0;
       const bool no_b = (L.dbg & 4u) != 0, no_a = (L.dbg & 16u) != 0;
       uint32_t tr_unit = 0;
@@ -313,7 +328,8 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
           conv = uni(P->conv); pk = uni(P->k);
           if (conv) {
             conv_c = uni(P->conv_c); conv_kw = uni(P->conv_kw); conv_wo = uni(P->conv_wo); conv_ho = uni(P->conv_ho);
-            conv_stride = uni(P->conv_stride); conv_pad = uni(P->conv_pad);
+            conv_stride = uni(P->conv_stride); conv_off_h = (int)uni((uint32_t)P->conv_off_h);
+            conv_off_w = (int)uni((uint32_t)P->conv_off_w);
           }
         }
         const uint32_t nt = W.nt, mt0 = W.mt0, g_count = W.g_count, mg = W.mg;
@@ -321,9 +337,9 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
         int cw = 0, ch = 0, cn = 0;
         if (conv) {
           const uint32_t p0 = nt * (uint32_t)BN, row = p0 / conv_wo;
-          cw = (int)((p0 - row * conv_wo) * conv_stride) - (int)conv_pad;
+          cw = (int)((p0 - row * conv_wo) * conv_stride) + conv_off_w;
           cn = (int)(row / conv_ho);
-          ch = (int)((row - (uint32_t)cn * conv_ho) * conv_stride) - (int)conv_pad;
+          ch = (int)((row - (uint32_t)cn * conv_ho) * conv_stride) + conv_off_h;
         }
         // the G tiles of a k-tile are adjacent in the operand, so one copy per array fetches a group's share of it
         const uint32_t rv0 = rows_valid_of(pm, mt0);
@@ -632,9 +648,16 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
                 const uint32_t r0 = lane >> 2, n_in = mc < pm ? pn - n0 : 0u;   // rows r0, r0 + 8, ... of the box
                 const uint16_t* src = Cptr + (size_t)(n0 + r0) * ldc + mc;
                 const uint32_t dst = sc + r0 * 64u + (lane & 3u) * 16u;
+                if (SCATTER) {
+                  for (uint32_t i = 0; i < 8; ++i) {
+                    const bool in = r0 + 8 * i < n_in;
+                    cp_async_16(dst + i * 512u, in ? Cptr + scatter_row(P, n0 + r0 + 8 * i) * ldc + mc : Cptr, in);
+                  }
+                } else {
 #pragma unroll
-                for (uint32_t i = 0; i < 8; ++i, src += 8 * ldc)
-                  cp_async_16(dst + i * 512u, r0 + 8 * i < n_in ? src : Cptr, r0 + 8 * i < n_in);
+                  for (uint32_t i = 0; i < 8; ++i, src += 8 * ldc)
+                    cp_async_16(dst + i * 512u, r0 + 8 * i < n_in ? src : Cptr, r0 + 8 * i < n_in);
+                }
                 cp_async_wait_all();
                 __syncwarp();
 #pragma unroll
@@ -719,7 +742,20 @@ spmma_kernel(const __grid_constant__ ProblemDev single, const __grid_constant__ 
             }
             fence_proxy_async_smem();
             __syncwarp();
-            if (lane == 0 && !no_store) {
+            if (SCATTER) {
+              // a staging row (64 bytes: 32 channels of one position) lands at the position's scattered row of D; lane l
+              // moves the 8 channels (l & 3) of rows l >> 2, + 8, ...  (m % 8 == 0: those 8 channels are all in or all out)
+              const uint32_t mc = m0 + quarter * 32 + (lane & 3u) * 8, r0 = lane >> 2;
+              uint16_t* D = reinterpret_cast<uint16_t*>(P->D);
+              const uint64_t ldd = P->ldd;
+              if (mc < pm && !no_store) {
+                for (uint32_t i = 0; i < 8; ++i) {
+                  const uint32_t r = r0 + 8 * i;
+                  if (n0 + r < pn)
+                    *reinterpret_cast<uint4*>(D + scatter_row(P, n0 + r) * ldd + mc) = ld_shared_v4(sc + r * 64u + (lane & 3u) * 16u);
+                }
+              }
+            } else if (lane == 0 && !no_store) {
               // (coordinates are (inner, outer): (n, m) for the row-major output, (m, n) for the transposed one)
               const int c0 = out_t ? (int)(m0 + quarter * 32) : (int)n0, c1 = out_t ? (int)n0 : (int)(m0 + quarter * 32);
               tma_store_2d(tmap_d, sc, c0, c1);
@@ -767,6 +803,21 @@ int make_tmap_grouped(CUtensorMap* map, int dtype, const void* base, uint64_t in
   return encode_tiled(map, dtype, 3, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, "spmma (grouped view)");
 }
 
+// the im2col view of an implicit GEMM's B: NHWC [batch][h][w][c], a kh x kw window whose base pixels run over
+// [lo, dim + up) per spatial dimension with `stride` -- the ho x wo output positions of every image
+struct Im2col {
+  size_t batch, h, w, c, kh, kw, stride;
+  int lo_h, lo_w, up_h, up_w;
+  size_t ho, wo;
+};
+
+// a forward convolution: the bounding box is [-pad, dim + pad - (filter - 1))
+Im2col im2col_of(const spfy_conv_desc& c) {
+  const int p = (int)c.pad;
+  return Im2col{c.batch, c.h, c.w, c.c, c.kh, c.kw, c.stride, -p, -p, p - (int)(c.kh - 1), p - (int)(c.kw - 1),
+                (c.h + 2 * c.pad - c.kh) / c.stride + 1, (c.w + 2 * c.pad - c.kw) / c.stride + 1};
+}
+
 struct HostProblem {
   int opB;
   size_t m, n, k;
@@ -774,10 +825,13 @@ struct HostProblem {
   void* D;
   size_t ldb, ldc, ldd;
   float alpha, beta;
-  const spfy_conv_desc* conv = nullptr;  // implicit GEMM: B is the NHWC activation tensor, never unfolded
+  bool conv = false;                     // implicit GEMM: B is the NHWC activation tensor, never unfolded (view `im`)
+  Im2col im{};
   bool out_t = false;                    // D is written transposed: [n][m] row-major, pitch ldd >= m (SPFY_OUT_T)
   spfy_epilogue epi{nullptr, nullptr, SPFY_ACT_NONE};
   bool ex = false;                       // called through an _ex entry: beta != 0 allowed with out_t (C is then [n][m])
+  bool scatter = false;                  // out_t rows scattered to the phase (sc_a, sc_b) of an sc_h x sc_w image
+  uint32_t sc_h = 0, sc_w = 0, sc_s = 1, sc_a = 0, sc_b = 0;
 };
 
 // the `opB` argument of the C ABI carries the output layout in bit 4 (SPFY_OUT_T)
@@ -791,16 +845,16 @@ int make_tmap_d(CUtensorMap* map, int dtype, const HostProblem& h, void* base) {
 }
 
 // NHWC activations {C, W, H, N} in im2col mode: one instruction gathers 128 consecutive output positions x 64 channels
-// of one filter tap.  The bounding box of base pixels is [-pad, dim + pad - (filter - 1)) per spatial dimension, walked
-// with the convolution stride -- exactly the output positions, row by row, image by image.
-int make_tmap_im2col(CUtensorMap* map, int dtype, const void* x, const spfy_conv_desc& c) {
+// of one filter tap.  The bounding box of base pixels (Im2col), walked with the convolution stride, holds exactly the
+// output positions, row by row, image by image.
+int make_tmap_im2col(CUtensorMap* map, int dtype, const void* x, const Im2col& c) {
   EncodeIm2colFn enc;
   int rc = get_im2col_encoder(&enc);
   if (rc) return rc;
   cuuint64_t dims[4] = {c.c, c.w, c.h, c.batch};
   cuuint64_t strides[3] = {c.c * 2, c.w * c.c * 2, c.h * c.w * c.c * 2};
-  int lower[2] = {-(int)c.pad, -(int)c.pad};
-  int upper[2] = {(int)c.pad - (int)(c.kw - 1), (int)c.pad - (int)(c.kh - 1)};
+  int lower[2] = {c.lo_w, c.lo_h};
+  int upper[2] = {c.up_w, c.up_h};
   cuuint32_t estr[4] = {1, (cuuint32_t)c.stride, (cuuint32_t)c.stride, 1};
   CUresult r = encode_with_context([&] {
     return enc(map, dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4,
@@ -809,8 +863,8 @@ int make_tmap_im2col(CUtensorMap* map, int dtype, const void* x, const spfy_conv
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   });
   if (r != CUDA_SUCCESS)
-    return fail(SPFY_E_CUDA, "cuTensorMapEncodeIm2col failed (%d) for NHWC %zu x %zu x %zu x %zu, filter %zu x %zu stride %zu pad %zu",
-                (int)r, c.batch, c.h, c.w, c.c, c.kh, c.kw, c.stride, c.pad);
+    return fail(SPFY_E_CUDA, "cuTensorMapEncodeIm2col failed (%d) for NHWC %zu x %zu x %zu x %zu, filter %zu x %zu stride %zu, "
+                "corners (%d, %d) / (%d, %d)", (int)r, c.batch, c.h, c.w, c.c, c.kh, c.kw, c.stride, c.lo_h, c.lo_w, c.up_h, c.up_w);
   return SPFY_OK;
 }
 
@@ -837,7 +891,9 @@ int validate(int dtype, const HostProblem& h, const char* who) {
   if ((!h.conv && h.ldb < b_inner) || h.ldd < (h.out_t ? h.m : h.n) || (h.beta != 0.f && h.ldc < (h.out_t ? h.m : h.n)))
     return fail(SPFY_E_INVALID, "%s: leading dimension too small", who);
   // TMA contract == the reference's own fp16 contract (spmma.hxx:45-49): multiples of 8
-  if ((!h.conv && h.ldb % 8) || h.ldd % 8 || (h.beta != 0.f && h.ldc % 8) || h.n % 8 || (h.opB == SPFY_OP_T && h.k % 8))
+  // (a scattered output is written position by position: n is free)
+  if ((!h.conv && h.ldb % 8) || h.ldd % 8 || (h.beta != 0.f && h.ldc % 8) || (!h.scatter && h.n % 8) ||
+      (h.opB == SPFY_OP_T && h.k % 8))
     return fail(SPFY_E_UNSUPPORTED,
                 "%s: n, ldb, ldc, ldd (and k for opB=T) must be multiples of 8 elements "
                 "(n=%zu k=%zu ldb=%zu ldc=%zu ldd=%zu)", who, h.n, h.k, h.ldb, h.ldc, h.ldd);
@@ -914,15 +970,16 @@ int fill_problem(ProblemDev* d, int dtype, const HostProblem& h, int cls) {
   const uint32_t box_outer = h.opB == SPFY_OP_N ? bk : 128u, box_groups = h.opB == SPFY_OP_N ? 2u : bk / 64u;
   if (h.conv) {
     d->b3d = 0;
-    rc = make_tmap_im2col(&d->tmap_b, dtype, h.B, *h.conv);
+    rc = make_tmap_im2col(&d->tmap_b, dtype, h.B, h.im);
     if (rc) return rc;
     d->conv = 1;
-    d->conv_c = (uint32_t)h.conv->c;
-    d->conv_kw = (uint32_t)h.conv->kw;
-    d->conv_wo = (uint32_t)((h.conv->w + 2 * h.conv->pad - h.conv->kw) / h.conv->stride + 1);
-    d->conv_ho = (uint32_t)((h.conv->h + 2 * h.conv->pad - h.conv->kh) / h.conv->stride + 1);
-    d->conv_stride = (uint32_t)h.conv->stride;
-    d->conv_pad = (uint32_t)h.conv->pad;
+    d->conv_c = (uint32_t)h.im.c;
+    d->conv_kw = (uint32_t)h.im.kw;
+    d->conv_wo = (uint32_t)h.im.wo;
+    d->conv_ho = (uint32_t)h.im.ho;
+    d->conv_stride = (uint32_t)h.im.stride;
+    d->conv_off_h = h.im.lo_h;
+    d->conv_off_w = h.im.lo_w;
   } else {
     if (d->b3d && make_tmap_grouped(&d->tmap_b, dtype, h.B, b_inner, b_outer, h.ldb, box_outer, box_groups) != SPFY_OK)
       d->b3d = 0;  // the driver refused the grouped view: fall back to 2-D boxes (64 inner elements each)
@@ -955,6 +1012,11 @@ int fill_problem(ProblemDev* d, int dtype, const HostProblem& h, int cls) {
   d->act = (uint32_t)h.epi.act;
   // an identity epilogue (no scale, no bias, no activation) runs the code of the plain entry points
   d->epi = h.epi.scale || h.epi.bias || h.epi.act != SPFY_ACT_NONE || (h.out_t && h.beta != 0.f);
+  if (h.scatter) {
+    d->D = h.D;
+    d->ldd = h.ldd;
+    d->sc_h = h.sc_h; d->sc_w = h.sc_w; d->sc_s = h.sc_s; d->sc_a = h.sc_a; d->sc_b = h.sc_b;
+  }
   // B is streamed once when one unit covers all of M; otherwise the other m-groups of the same
   // columns will want it from L2 shortly after
   d->hint_b = d->m_groups == 1 ? HINT_EVICT_FIRST : HINT_EVICT_NORMAL;
@@ -1023,10 +1085,10 @@ uint32_t make_idesc(int dtype, int opB) {
          ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 }
 
-template <bool BF16, bool OPB_T, bool EPI>
+template <bool BF16, bool OPB_T, bool EPI, bool SCATTER = false>
 int launch_t(const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid, cudaStream_t s,
              bool overlap_previous) {
-  int rc = allow_dynamic_smem<spmma_kernel<BF16, OPB_T, EPI>>(SMEM_LIMIT);
+  int rc = allow_dynamic_smem<spmma_kernel<BF16, OPB_T, EPI, SCATTER>>(SMEM_LIMIT);
   if (rc) return rc;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -1040,7 +1102,7 @@ int launch_t(const ProblemDev& single, const LaunchParams& L, uint32_t smem, int
   attr.val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = &attr;
   cfg.numAttrs = overlap_previous ? 1 : 0;
-  SPFY_CUDA_OK(cudaLaunchKernelEx(&cfg, spmma_kernel<BF16, OPB_T, EPI>, single, L));
+  SPFY_CUDA_OK(cudaLaunchKernelEx(&cfg, spmma_kernel<BF16, OPB_T, EPI, SCATTER>, single, L));
   SPFY_LAUNCH_OK("spmma_kernel");
   return SPFY_OK;
 }
@@ -1055,10 +1117,14 @@ int launch_e(int dtype, int opB, const ProblemDev& single, const LaunchParams& L
                           : launch_t<false, true, EPI>(single, L, smem, grid, s, overlap_previous);
 }
 
-// overlap_previous: the kernel launched just before on this stream is another launch of the same plan;
-// epi: some problem of the launch has an epilogue
+// overlap_previous: the kernel launched just before on this stream is another launch of the same plan (or another
+// phase of the same data gradient); epi: some problem of the launch has an epilogue; a single problem with a scattered
+// output (opB = T) takes the SCATTER kernels
 int launch(int dtype, int opB, bool epi, const ProblemDev& single, const LaunchParams& L, uint32_t smem, int grid,
            cudaStream_t s, bool overlap_previous = false) {
+  if (single.D)
+    return dtype == SPFY_BF16 ? launch_t<true, true, true, true>(single, L, smem, grid, s, overlap_previous)
+                              : launch_t<false, true, true, true>(single, L, smem, grid, s, overlap_previous);
   return epi ? launch_e<true>(dtype, opB, single, L, smem, grid, s, overlap_previous)
              : launch_e<false>(dtype, opB, single, L, smem, grid, s, overlap_previous);
 }
@@ -1118,7 +1184,8 @@ int conv_problem(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, c
   const size_t ho = (c.h + 2 * c.pad - c.kh) / c.stride + 1, wo = (c.w + 2 * c.pad - c.kw) / c.stride + 1;
   const size_t n = c.batch * ho * wo, k = c.kh * c.kw * c.c;
   HostProblem h{SPFY_OP_T, m, n, k, comp_vals, meta, X, C, D, /*ldb*/ k, ldc, ldd, alpha, beta};
-  h.conv = conv;
+  h.conv = true;
+  h.im = im2col_of(c);
   h.out_t = out_t;
   if (epi) h.epi = *epi;
   h.ex = ex;
@@ -1132,32 +1199,72 @@ uint32_t debug_mode() {
   return e ? (uint32_t)atoi(e) : 0u;
 }
 
+// one validated, non-empty problem in a launch of its own, built (tensor maps encoded) but not yet launched
+struct SingleLaunch {
+  ProblemDev d;
+  LaunchParams L;
+  uint32_t smem;
+  int grid;
+};
+int prepare_single(int dtype, const HostProblem& h, const DeviceInfo& di, SingleLaunch* out) {
+  const int cls = classify(h, false, di.sm_count);
+  ProblemDev& d = out->d;
+  int rc = fill_problem(&d, dtype, h, cls);
+  if (rc) return rc;
+  d.unit_begin = 0;
+  split_tail(&d, cls, di.sm_count);
+  LaunchParams& L = out->L;
+  memset(&L, 0, sizeof(L));
+  out->smem = 0;
+  geometry(cls, res_values_bytes(d), res_meta_bytes(d), &L, &out->smem);
+  L.table = nullptr;
+  L.num_problems = 1;
+  L.total_units = d.units;
+  L.idesc = make_idesc(dtype, h.opB);
+  L.dbg = debug_mode();
+  out->grid = (int)(d.units < (uint32_t)di.sm_count ? d.units : (uint32_t)di.sm_count);
+  return SPFY_OK;
+}
+
 // one validated problem (spfy_spmma*, spfy_spmma_conv*) in a launch of its own
 int run_single(int dtype, const HostProblem& h, cudaStream_t s) {
   if (h.m == 0 || h.n == 0) return SPFY_OK;
   DeviceInfo di;
   int rc = require_sm100(h.conv ? "spmma_conv" : "spmma", &di);
   if (rc) return rc;
-  const int cls = classify(h, false, di.sm_count);
-  ProblemDev d;
-  rc = fill_problem(&d, dtype, h, cls);
+  SingleLaunch sl;
+  rc = prepare_single(dtype, h, di, &sl);
   if (rc) return rc;
-  d.unit_begin = 0;
-  split_tail(&d, cls, di.sm_count);
-  LaunchParams L;
-  memset(&L, 0, sizeof(L));
-  uint32_t smem = 0;
-  geometry(cls, res_values_bytes(d), res_meta_bytes(d), &L, &smem);
-  L.table = nullptr;
-  L.num_problems = 1;
-  L.total_units = d.units;
-  L.idesc = make_idesc(dtype, h.opB);
-  L.dbg = debug_mode();
-  const int grid = (int)(d.units < (uint32_t)di.sm_count ? d.units : (uint32_t)di.sm_count);
 #ifdef SPFY_DEV_SWITCHES
-  if (const char* path = dev_switch("SPFY_SPMMA_TRACE")) return launch_traced(path, dtype, h.opB, d, L, smem, grid, s);
+  if (const char* path = dev_switch("SPFY_SPMMA_TRACE"))
+    return launch_traced(path, dtype, h.opB, sl.d, sl.L, sl.smem, sl.grid, s);
 #endif
-  return launch(dtype, h.opB, d.epi != 0, d, L, smem, grid, s);
+  return launch(dtype, h.opB, sl.d.epi != 0, sl.d, sl.L, sl.smem, sl.grid, s);
+}
+
+// the dX pixels of a strided data gradient that no filter tap reaches (bit a * s + b of `empty`: phase (a, b) has no
+// taps): +0 for beta == 0 (whatever dX held), else beta * dX.  16 bytes (8 channels) per thread and step.
+template <typename T>
+__global__ void __launch_bounds__(256)
+dgrad_fill_kernel(T* dx, size_t chunks, uint32_t c8, uint32_t h, uint32_t w, uint32_t s, uint64_t empty, float beta) {
+  for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < chunks; t += (size_t)gridDim.x * blockDim.x) {
+    const size_t px = t / c8;
+    const uint32_t x = (uint32_t)(px % w), y = (uint32_t)(px / w % h);
+    if (!(empty >> ((y % s) * s + x % s) & 1u)) continue;
+    uint4* p = reinterpret_cast<uint4*>(dx) + t;
+    if (beta == 0.f) {
+      *p = make_uint4(0u, 0u, 0u, 0u);
+    } else {
+      union {
+        uint4 v;
+        T e[8];
+      } u;
+      u.v = *p;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) u.e[i] = from_f32<T>(beta * to_f32(u.e[i]));
+      *p = u.v;
+    }
+  }
 }
 
 struct Plan {
@@ -1179,14 +1286,18 @@ struct Plan {
 }  // namespace spfy
 
 void spfy::warm_spmma_kernels() {
-  touch_kernel(spmma_kernel<false, false, false>);
-  touch_kernel(spmma_kernel<false, true, false>);
-  touch_kernel(spmma_kernel<true, false, false>);
-  touch_kernel(spmma_kernel<true, true, false>);
-  touch_kernel(spmma_kernel<false, false, true>);
-  touch_kernel(spmma_kernel<false, true, true>);
-  touch_kernel(spmma_kernel<true, false, true>);
-  touch_kernel(spmma_kernel<true, true, true>);
+  touch_kernel(spmma_kernel<false, false, false, false>);
+  touch_kernel(spmma_kernel<false, true, false, false>);
+  touch_kernel(spmma_kernel<true, false, false, false>);
+  touch_kernel(spmma_kernel<true, true, false, false>);
+  touch_kernel(spmma_kernel<false, false, true, false>);
+  touch_kernel(spmma_kernel<false, true, true, false>);
+  touch_kernel(spmma_kernel<true, false, true, false>);
+  touch_kernel(spmma_kernel<true, true, true, false>);
+  touch_kernel(spmma_kernel<false, true, true, true>);
+  touch_kernel(spmma_kernel<true, true, true, true>);
+  touch_kernel(dgrad_fill_kernel<__half>);
+  touch_kernel(dgrad_fill_kernel<__nv_bfloat16>);
   EncodeTiledFn enc;
   (void)get_encoder(&enc);
 }
@@ -1246,6 +1357,94 @@ int spfy_spmma_conv(int dtype, const spfy_conv_desc* conv, size_t m, float alpha
 int spfy_spmma_conv_nhwc(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,
                          const void* meta, const void* X, void* Y, size_t ldy, spfy_stream_t stream) {
   return spmma_conv_impl(dtype, conv, m, alpha, comp_vals, meta, X, 0.f, nullptr, 0, Y, ldy, true, nullptr, false, stream);
+}
+
+int spfy_spmma_conv_dgrad(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* vals_t,
+                          const void* meta_t, const void* dY, float beta, void* dX, spfy_stream_t stream) {
+  const char* who = "spmma_conv_dgrad";
+  if (dtype != SPFY_F16 && dtype != SPFY_BF16) return fail(SPFY_E_UNSUPPORTED, "%s: dtype %d (need F16/BF16)", who, dtype);
+  if (!conv) return fail(SPFY_E_INVALID, "%s: null descriptor", who);
+  const spfy_conv_desc& c = *conv;
+  if (!c.batch || !c.h || !c.w || !c.c || !c.kh || !c.kw || !c.stride || !m)
+    return fail(SPFY_E_INVALID, "%s: empty dimension", who);
+  if (m % 64)
+    return fail(SPFY_E_UNSUPPORTED, "%s: m (the channels of dY) must be a multiple of 64 (got %zu)", who, m);
+  if (c.c % 8) return fail(SPFY_E_UNSUPPORTED, "%s: c (the channels of dX) must be a multiple of 8 (got %zu)", who, c.c);
+  if (c.kh > 16 || c.kw > 16 || c.pad > 8 || c.stride > 8)
+    return fail(SPFY_E_UNSUPPORTED, "%s: filter / padding / stride outside what spfy_spmma_conv accepts", who);
+  if (c.h + 2 * c.pad < c.kh || c.w + 2 * c.pad < c.kw) return fail(SPFY_E_INVALID, "%s: filter larger than the padded image", who);
+  if (!vals_t || !meta_t || !dY || !dX) return fail(SPFY_E_INVALID, "%s: null operand", who);
+  if ((uintptr_t)vals_t % 16 || (uintptr_t)meta_t % 16 || (uintptr_t)dY % 16 || (uintptr_t)dX % 16)
+    return fail(SPFY_E_INVALID, "%s: operands must be 16-byte aligned", who);
+  const size_t s = c.stride, ho = (c.h + 2 * c.pad - c.kh) / s + 1, wo = (c.w + 2 * c.pad - c.kw) / s + 1;
+  // every phase, validated before any device work; the phase operands lie back to back in the order of
+  // spfy_transpose24_conv, whether or not the phase has dX pixels
+  HostProblem phases[64];
+  int count = 0;
+  uint64_t empty = 0;
+  size_t tiles = 0;
+  for (size_t a = 0; a < s; ++a)
+    for (size_t b = 0; b < s; ++b) {
+      const DgradPhase ph = dgrad_phase(c.kh, s, c.pad, a), pw = dgrad_phase(c.kw, s, c.pad, b);
+      const size_t ha = dgrad_phase_extent(c.h, s, a), wb = dgrad_phase_extent(c.w, s, b);
+      if (!ph.taps || !pw.taps) {
+        if (ha && wb) empty |= 1ull << (a * s + b);
+        continue;
+      }
+      const size_t k = (size_t)ph.taps * pw.taps * m;
+      const size_t first = tiles;
+      tiles += ceil_div(c.c, 128) * ceil_div(k, 128);
+      if (!ha || !wb) continue;
+      // a stride-1 correlation of dY: base pixels [d0, d0 + phase extent) per dimension
+      Im2col im{c.batch, ho, wo, m, ph.taps, pw.taps, 1, ph.d0, pw.d0, ph.d0 + (int)ha - (int)ho, pw.d0 + (int)wb - (int)wo,
+                ha, wb};
+      if (std::min({im.lo_h, im.lo_w, im.up_h, im.up_w}) < -128 || std::max({im.lo_h, im.lo_w, im.up_h, im.up_w}) > 127)
+        return fail(SPFY_E_UNSUPPORTED, "%s: phase (%zu, %zu) needs im2col corners outside [-128, 127]", who, a, b);
+      HostProblem h{SPFY_OP_T, c.c, c.batch * ha * wb, k, (const uint8_t*)vals_t + first * A_TILE_BYTES,
+                    (const uint8_t*)meta_t + first * E_TILE_BYTES, dY, dX, dX, /*ldb*/ k, c.c, c.c, alpha, beta};
+      h.conv = true;
+      h.im = im;
+      h.out_t = true;
+      h.ex = true;
+      h.scatter = true;
+      h.sc_h = (uint32_t)c.h; h.sc_w = (uint32_t)c.w; h.sc_s = (uint32_t)s; h.sc_a = (uint32_t)a; h.sc_b = (uint32_t)b;
+      int rc = validate(dtype, h, who);
+      if (rc) return rc;
+      phases[count++] = h;
+    }
+  // every phase built (tensor maps encoded) before any device work, so that a failure leaves dX untouched
+  DeviceInfo di;
+  int rc = require_sm100(who, &di);
+  if (rc) return rc;
+  std::vector<SingleLaunch> launches((size_t)count);
+  for (int i = 0; i < count; ++i) {
+    rc = prepare_single(dtype, phases[i], di, &launches[(size_t)i]);
+    if (rc) return rc;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (empty && beta != 1.f) {
+    const size_t chunks = c.batch * c.h * c.w * (c.c / 8);
+    int grid = 1;
+    rc = capped_grid(ceil_div(chunks, 256), 8, &grid);
+    if (rc) return rc;
+    if (dtype == SPFY_BF16)
+      dgrad_fill_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)dX, chunks, (uint32_t)(c.c / 8), (uint32_t)c.h,
+                                                             (uint32_t)c.w, (uint32_t)s, empty, beta);
+    else
+      dgrad_fill_kernel<__half><<<grid, 256, 0, st>>>((__half*)dX, chunks, (uint32_t)(c.c / 8), (uint32_t)c.h, (uint32_t)c.w,
+                                                      (uint32_t)s, empty, beta);
+    SPFY_LAUNCH_OK("dgrad_fill_kernel");
+  }
+  // The phases write disjoint pixels of dX, so each launch may start while the previous one still runs: a phase of a
+  // small layer (26-52 units at 14 x 14, b = 32) leaves most SMs to the next one.  SPFY_SPMMA_NO_OVERLAP (dev builds,
+  // read on every call) serialises them, for timing the two forms against each other.
+  const bool serial = dev_switch("SPFY_SPMMA_NO_OVERLAP") != nullptr;
+  for (int i = 0; i < count; ++i) {
+    const SingleLaunch& sl = launches[(size_t)i];
+    rc = launch(dtype, SPFY_OP_T, sl.d.epi != 0, sl.d, sl.L, sl.smem, sl.grid, st, i > 0 && !serial);
+    if (rc) return rc;
+  }
+  return SPFY_OK;
 }
 
 int spfy_spmma_conv_ex(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* comp_vals,

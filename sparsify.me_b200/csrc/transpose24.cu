@@ -2,6 +2,8 @@
 //
 //   spfy_transpose24  : SM100 compressed A -> SM100 compressed A' (A^T, or the flipped, channel-swapped filter of a
 //                       convolution's data gradient).  Valid when A's mask keeps two of four along columns too (TILE).
+//   spfy_transpose24_conv : the same for a strided convolution: one A' per output phase of its data gradient, each
+//                       built from the phase's subset of filter taps, all in one launch.
 //   spfy_recompress24 : new values under a fixed mask: dense (F32 / F16 / BF16) -> compressed values at the positions an
 //                       existing operand's metadata keeps, and / or the dense input with the pruned positions zeroed.
 //
@@ -19,6 +21,14 @@ namespace {
 // One CTA writes one 128 x 128 tile of A': warp w the 16-column unit w of every row, lane l the rows 4l .. 4l + 3.
 // Every lane of a warp reads the same A rows, 32 consecutive 4-column groups of them: 128 contiguous bytes of values.
 // ------------------------------------------------------------------------
+// PHASED (spfy_transpose24_conv): the output is several A', one per phase of a strided convolution's data gradient, back
+// to back in tile order.  Phase ph owns the tiles [tile_begin, next tile_begin) and its column tap t' = th * nb + tw
+// reads the source tap src0 - th * step_h - tw * step_w.  One phase with nb = 1, src0 = taps - 1 and step_h = 1 is the
+// plain transpose.
+constexpr int MAX_PHASES = 64;  // stride <= 8 in both dimensions
+struct Transpose24Phase {
+  uint32_t tile_begin, taps, nb, src0;
+};
 struct Transpose24Params {
   const uint8_t* vals;
   const uint8_t* meta;
@@ -27,17 +37,35 @@ struct Transpose24Params {
   uint32_t rows, C, taps;  // A: rows x (taps * C)
   uint32_t m_tiles;        // A: 128-row tiles
   uint32_t m_tiles_t;      // A': 128-row tiles (of C rows)
-  uint32_t tiles_t;        // A': tiles
+  uint32_t tiles_t;        // A': tiles (of all phases)
   int* invalid;
 };
+// the phase table, a kernel parameter of its own: the plain transpose passes a one-entry table it never reads, so its
+// launches do not carry the 1 KiB of a full one
+template <int N>
+struct Transpose24Phases {
+  uint32_t phases, step_h, step_w;
+  Transpose24Phase ph[N];
+};
 
+template <bool PHASED>
 __global__ void __launch_bounds__(256)
-transpose24_kernel(const __grid_constant__ Transpose24Params P) {
+transpose24_kernel(const __grid_constant__ Transpose24Params P,
+                   const __grid_constant__ Transpose24Phases<PHASED ? MAX_PHASES : 1> T) {
   const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
-  const uint32_t cols_t = P.taps * P.rows;
+  uint32_t cols_t = P.taps * P.rows;
   bool bad = false;
   for (uint32_t tile = blockIdx.x; tile < P.tiles_t; tile += gridDim.x) {
-    const uint32_t kt = tile / P.m_tiles_t, mt = tile - kt * P.m_tiles_t;  // storage order: k-tile major
+    uint32_t local = tile, nb = 1u, src0 = P.taps - 1u;
+    if (PHASED) {
+      uint32_t p = 0;
+      while (p + 1u < T.phases && tile >= T.ph[p + 1u].tile_begin) ++p;
+      local = tile - T.ph[p].tile_begin;
+      cols_t = T.ph[p].taps * P.rows;
+      nb = T.ph[p].nb;
+      src0 = T.ph[p].src0;
+    }
+    const uint32_t kt = local / P.m_tiles_t, mt = local - kt * P.m_tiles_t;  // storage order: k-tile major
     const uint32_t ci0 = mt * 128u + lane * 4u, j0 = kt * 128u + w * 16u;
     uint32_t ov[4][4];                  // [A' row j][group k]: the two kept values
     uint32_t on[4] = {0u, 0u, 0u, 0u};  // [A' row j]: the unit's four nibbles
@@ -53,7 +81,12 @@ transpose24_kernel(const __grid_constant__ Transpose24Params P) {
         continue;
       }
       const uint32_t tp = col / P.rows, r0 = col - tp * P.rows;
-      const uint32_t c = (P.taps - 1u - tp) * P.C + ci0;  // first column of the A block
+      uint32_t src = P.taps - 1u - tp;  // source tap of A' tap tp
+      if (PHASED) {
+        const uint32_t th = tp / nb;
+        src = src0 - th * T.step_h - (tp - th * nb) * T.step_w;
+      }
+      const uint32_t c = src * P.C + ci0;  // first column of the A block
       const uint32_t q = (c & 127u) >> 4, g = (c >> 2) & 3u;
       uint32_t v[4], n[4];
 #pragma unroll
@@ -198,11 +231,41 @@ void launch_recompress24(int dtype, int grid, const Recompress24Params& P, cudaS
 
 bool misaligned16(const void* p) { return (uintptr_t)p % 16 != 0; }
 
+// the phase table of spfy_transpose24_conv: every phase (a, b) with taps in both dimensions, in (a, b) row-major order;
+// `tiles` = the tiles of all of them
+int conv_phase_table(const char* who, size_t m, size_t c, size_t kh, size_t kw, size_t stride, size_t pad,
+                     Transpose24Phases<MAX_PHASES>* P, size_t* tiles) {
+  if (!m || !c || !kh || !kw || !stride) return fail(SPFY_E_INVALID, "%s: empty dimension", who);
+  if (m % 8 || c % 8) return fail(SPFY_E_UNSUPPORTED, "%s: m (%zu) and c (%zu) must be multiples of 8", who, m, c);
+  if (kh > 16 || kw > 16 || pad > 8 || stride > 8)
+    return fail(SPFY_E_UNSUPPORTED, "%s: filter / padding / stride outside what the convolutions accept", who);
+  if (m >= (1ull << 24) || c >= (1ull << 24)) return fail(SPFY_E_UNSUPPORTED, "%s: dimension too large", who);
+  P->phases = 0;
+  P->step_h = (uint32_t)(stride * kw);
+  P->step_w = (uint32_t)stride;
+  size_t t = 0;
+  for (size_t a = 0; a < stride; ++a)
+    for (size_t b = 0; b < stride; ++b) {
+      const DgradPhase ph = dgrad_phase(kh, stride, pad, a), pw = dgrad_phase(kw, stride, pad, b);
+      if (!ph.taps || !pw.taps) continue;
+      Transpose24Phase& q = P->ph[P->phases++];
+      q.tile_begin = (uint32_t)t;
+      q.taps = ph.taps * pw.taps;
+      q.nb = pw.taps;
+      q.src0 = ph.k0 * (uint32_t)kw + pw.k0;
+      t += ceil_div(c, 128) * ceil_div(q.taps * m, 128);
+    }
+  if (t >= (1ull << 22)) return fail(SPFY_E_UNSUPPORTED, "%s: more than 2^22 SM100 tiles", who);
+  *tiles = t;
+  return SPFY_OK;
+}
+
 }  // namespace
 }  // namespace spfy
 
 void spfy::warm_transpose24_kernels() {
-  touch_kernel(transpose24_kernel);
+  touch_kernel(transpose24_kernel<false>);
+  touch_kernel(transpose24_kernel<true>);
   touch_kernel(recompress24_kernel<SPFY_F32, SPFY_F16>);
   touch_kernel(recompress24_kernel<SPFY_F32, SPFY_BF16>);
   touch_kernel(recompress24_kernel<SPFY_F16, SPFY_F16>);
@@ -249,7 +312,53 @@ int spfy_transpose24(int dtype, const void* vals, const void* meta, size_t rows,
   int grid = 1;
   int rc = capped_grid(P.tiles_t, 8, &grid);
   if (rc) return rc;
-  transpose24_kernel<<<grid, 256, 0, s>>>(P);
+  transpose24_kernel<false><<<grid, 256, 0, s>>>(P, Transpose24Phases<1>{});
+  SPFY_LAUNCH_OK("transpose24_kernel");
+  return SPFY_OK;
+}
+
+int spfy_transpose24_conv_bytes(int dtype, size_t m, size_t c, size_t kh, size_t kw, size_t stride, size_t pad,
+                                size_t* vals_bytes, size_t* meta_bytes) {
+  if (dtype != SPFY_F16 && dtype != SPFY_BF16)
+    return fail(SPFY_E_UNSUPPORTED, "transpose24_conv_bytes: dtype %d (need F16/BF16)", dtype);
+  Transpose24Phases<MAX_PHASES> T;
+  size_t tiles = 0;
+  int rc = conv_phase_table("transpose24_conv_bytes", m, c, kh, kw, stride, pad, &T, &tiles);
+  if (rc) return rc;
+  if (vals_bytes) *vals_bytes = tiles * 16384;
+  if (meta_bytes) *meta_bytes = tiles * 2048;
+  return SPFY_OK;
+}
+
+int spfy_transpose24_conv(int dtype, const void* vals, const void* meta, size_t m, size_t c, size_t kh, size_t kw,
+                          size_t stride, size_t pad, void* vals_t, void* meta_t, int* d_invalid, spfy_stream_t stream) {
+  if (dtype != SPFY_F16 && dtype != SPFY_BF16)
+    return fail(SPFY_E_UNSUPPORTED, "transpose24_conv: dtype %d (need F16/BF16)", dtype);
+  Transpose24Phases<MAX_PHASES> T;
+  size_t tiles = 0;
+  int rc = conv_phase_table("transpose24_conv", m, c, kh, kw, stride, pad, &T, &tiles);
+  if (rc) return rc;
+  if (!vals || !meta || !vals_t || !meta_t) return fail(SPFY_E_INVALID, "transpose24_conv: null pointer");
+  if (misaligned16(vals) || misaligned16(meta) || misaligned16(vals_t) || misaligned16(meta_t))
+    return fail(SPFY_E_INVALID, "transpose24_conv: SM100 buffers must be 16-byte aligned");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (d_invalid) SPFY_CUDA_OK(cudaMemsetAsync(d_invalid, 0, sizeof(int), s));
+  Transpose24Params P;
+  P.vals = (const uint8_t*)vals;
+  P.meta = (const uint8_t*)meta;
+  P.vals_t = (uint8_t*)vals_t;
+  P.meta_t = (uint8_t*)meta_t;
+  P.rows = (uint32_t)m;
+  P.C = (uint32_t)c;
+  P.taps = (uint32_t)(kh * kw);
+  P.m_tiles = (uint32_t)ceil_div(m, 128);
+  P.m_tiles_t = (uint32_t)ceil_div(c, 128);
+  P.tiles_t = (uint32_t)tiles;
+  P.invalid = d_invalid;
+  int grid = 1;
+  rc = capped_grid(P.tiles_t, 8, &grid);
+  if (rc) return rc;
+  transpose24_kernel<true><<<grid, 256, 0, s>>>(P, T);
   SPFY_LAUNCH_OK("transpose24_kernel");
   return SPFY_OK;
 }

@@ -330,6 +330,95 @@ def transpose24(comp, taps=1, out=None, invalid=None):
     return out
 
 
+def _dgrad_phase(k, s, p, a):
+    """the taps of output phase a of a stride-s data gradient in one dimension (spfy_transpose24_conv):
+    (filter indices in descending order, dy offset of the first)"""
+    taps = [kt for kt in range(k - 1, -1, -1) if (a + p - kt) % s == 0]
+    return taps, ((a + p - taps[0]) // s if taps else 0)
+
+
+@dataclass
+class Transpose24Conv:
+    """The data-gradient filter operands of a stride-`stride` convolution (spfy_transpose24_conv): one SM100 operand per
+    output phase (a, b) with taps, back to back in `vals` / `meta`.  `phases`: [(a, b, taps_h, taps_w, Compressed24)],
+    the Compressed24 of each a view of c rows x len(taps_h)*len(taps_w)*m columns (taps in descending filter index)."""
+    vals: torch.Tensor
+    meta: torch.Tensor
+    m: int
+    c: int
+    kh: int
+    kw: int
+    stride: int
+    pad: int
+    dtype: torch.dtype
+    phases: list
+
+
+def transpose24_conv(comp, kh, kw, stride, pad, invalid=None):
+    """spfy_transpose24_conv: the operands of the data gradient of a stride-`stride`, pad-`pad` convolution whose filter
+    `comp` is m x kh*kw*c in (kh, kw, c) order (permute_conv_weights, then prune24 with PRUNE_TILE_TRANSPOSABLE).  Phase
+    (a, b) holds the dx pixels (s*i + a, s*j + b); its operand is the flipped, channel-swapped sub-filter of the taps
+    that reach them.  For stride 1 the one operand is transpose24(comp, taps=kh*kw), byte for byte.
+    `invalid`: optional int32 CUDA tensor, 0, or 1 when the mask is not transposable.  Nothing here syncs.
+    Use it with spmma_conv_dgrad_nhwc."""
+    assert comp.layout == capi.LAYOUT_SM100
+    if comp.cols % (kh * kw):
+        raise capi.SpfyError(capi.E_INVALID, "transpose24_conv", f"cols {comp.cols} is not a multiple of kh*kw {kh * kw}")
+    m, c = comp.rows, comp.cols // (kh * kw)
+    vb, mb = ctypes.c_size_t(), ctypes.c_size_t()
+    capi.spfy_transpose24_conv_bytes(_DT[comp.dtype], m, c, kh, kw, stride, pad, ctypes.byref(vb), ctypes.byref(mb))
+    dev = comp.vals.device
+    vals = torch.empty(vb.value, dtype=torch.uint8, device=dev)
+    meta = torch.empty(mb.value, dtype=torch.uint8, device=dev)
+    if invalid is not None:
+        assert invalid.dtype == torch.int32 and invalid.is_cuda
+    capi.spfy_transpose24_conv(_DT[comp.dtype], _ptr(comp.vals), _ptr(comp.meta), m, c, kh, kw, stride, pad,
+                               _ptr(vals), _ptr(meta), _ptr(invalid), _stream())
+    phases, tile = [], 0
+    for a in range(stride):
+        for b in range(stride):
+            th, tw = _dgrad_phase(kh, stride, pad, a)[0], _dgrad_phase(kw, stride, pad, b)[0]
+            if not th or not tw:
+                continue
+            cols = len(th) * len(tw) * m
+            tiles = -(-c // 128) * -(-cols // 128)
+            view = Compressed24(vals[tile * 16384:(tile + tiles) * 16384], meta[tile * 2048:(tile + tiles) * 2048], c, cols,
+                                comp.dtype, capi.LAYOUT_SM100)
+            phases.append((a, b, th, tw, view))
+            tile += tiles
+    return Transpose24Conv(vals, meta, m, c, kh, kw, stride, pad, comp.dtype, phases)
+
+
+def spmma_conv_dgrad_nhwc(op, dy, h, w, out=None, alpha=1.0, beta=0.0):
+    """spfy_spmma_conv_dgrad: dx = alpha * conv2d_input(W, dy) + beta * out for the forward layer of `op`
+    (transpose24_conv), any stride, on sparse tensor cores.  dy: NHWC [batch, ho, wo, m]; h, w: the forward input size
+    (a strided layer's ho, wo do not determine it).  Returns dx, NHWC [batch, h, w, c] (== out when given; beta != 0
+    needs out, and beta = 1 accumulates into it).  The backward data pass of a strided layer, dy and dx in NHWC:
+        w2 = permute_conv_weights(weight.view(m, -1), c, kh, kw)       # (kh, kw, c) order, before pruning
+        comp = prune24(w2, mode=PRUNE_TILE_TRANSPOSABLE)
+        op = transpose24_conv(comp, kh, kw, stride, pad)              # once per weight update
+        dx = spmma_conv_dgrad_nhwc(op, dy, h, w)
+    With beta=1 and out = the shortcut's dx, a residual downsample block's two data gradients meet in place.
+    The same call is a 2:4 transposed convolution (ConvTranspose2d with stride s, padding pad, output size h x w) of a
+    filter pruned in the forward orientation: x_up = spmma_conv_dgrad_nhwc(op, x, h, w)."""
+    assert dy.dim() == 4 and dy.is_contiguous() and dy.dtype == op.dtype
+    nb, ho, wo, m = dy.shape
+    s, p = op.stride, op.pad
+    if h + 2 * p < op.kh or w + 2 * p < op.kw or (ho, wo, m) != ((h + 2 * p - op.kh) // s + 1, (w + 2 * p - op.kw) // s + 1,
+                                                                  op.m):
+        raise capi.SpfyError(capi.E_INVALID, "spmma_conv_dgrad", f"dy {tuple(dy.shape)} does not match a {op.kh}x{op.kw} "
+                             f"stride {s} pad {p} layer with {op.m} outputs on {h}x{w} inputs")
+    if out is None:
+        if beta != 0.0:
+            raise capi.SpfyError(capi.E_INVALID, "spmma_conv_dgrad", "beta != 0 needs out")
+        out = torch.empty(nb, h, w, op.c, dtype=op.dtype, device=dy.device)
+    assert out.is_contiguous() and tuple(out.shape) == (nb, h, w, op.c) and out.dtype == op.dtype
+    desc = capi.ConvDesc(nb, h, w, op.c, op.kh, op.kw, s, p)
+    capi.spfy_spmma_conv_dgrad(_DT[op.dtype], ctypes.byref(desc), op.m, float(alpha), _ptr(op.vals), _ptr(op.meta),
+                               _ptr(dy), float(beta), _ptr(out), _stream())
+    return out
+
+
 def recompress24(dense, comp, masked_out=None, values=True):
     """spfy_recompress24: new values under comp's fixed mask.  `dense` [comp.rows, comp.cols] (fp32, fp16 or bf16,
     row-major).  values=True: comp.vals <- dense at the positions comp.meta keeps, rounded to nearest even to comp.dtype
