@@ -499,14 +499,14 @@ SPFY_API int spfy_spmm_bell_batched(int alg, int dtype, size_t rows, size_t cols
  * conventions: column-major, C_b[m x n, ldc] = alpha * op(A_b)[m x k] * op(B_b)[k x n]
  * + beta * C_b.  opX = N: the operand is stored as its op() shape; T: transposed.
  * dtype F16 / BF16: kind::f16, fp32 accumulation in TMEM.  dtype F32:
- *   SPFY_GEMM_PRECISE  3xTF32 -- each operand is split in shared memory into
- *                      hi (the 11 significant bits the tensor core reads) and lo = x - hi, and
- *                      hi*lo + lo*hi + hi*hi is accumulated in fp32: products exact to ~2^-21;
+ *   SPFY_GEMM_PRECISE  3xTF32 -- each operand is split into hi (the 11 significant bits
+ *                      the tensor core reads) and lo = x - hi, and hi*lo + lo*hi + hi*hi is
+ *                      accumulated in fp32: products exact to ~2^-19.  The long, streamed
+ *                      operand is split in registers into tensor memory (hi rounded to
+ *                      nearest); the other keeps its raw tile in shared memory as hi (the
+ *                      tensor core truncates it) with lo written behind it;
  *   SPFY_GEMM_FAST     one TF32 product.
- * SPFY_GEMM_CTA_PAIRS may be OR-ed into `precision`: 16-bit operands and SPFY_GEMM_FAST then run on CTA pairs
- * (tcgen05.mma.cta_group::2, M = 256: each CTA of a two-CTA cluster loads its own 128 rows of the long operand and
- * half of the other tile) when every problem has more than 128 rows of the long operand; same results.  Off by
- * default because it is slower on the ResNet shapes (profiles/r02_gemm_cta_pairs.txt).
+ * Any other `precision` is refused with SPFY_E_INVALID before any device work, for every dtype.
  * The operands are fetched by TMA, which needs 16-byte aligned bases and lda / ldb /
  * batch strides that are multiples of 16 bytes; an operand that misses this (ldb = k = 147
  * floats, the first conv layer of every ResNet) is first copied into the workspace with
@@ -517,7 +517,7 @@ SPFY_API int spfy_spmm_bell_batched(int alg, int dtype, size_t rows, size_t cols
  * of the operands whose lda / ldb need them; pass lda = 0 / ldb = 0 to size for a
  * misaligned base pointer as well).
  * ---------------------------------------------------------------------- */
-enum { SPFY_GEMM_PRECISE = 0, SPFY_GEMM_FAST = 1, SPFY_GEMM_CTA_PAIRS = 0x10 };
+enum { SPFY_GEMM_PRECISE = 0, SPFY_GEMM_FAST = 1 };
 SPFY_API int spfy_gemm_workspace_bytes(int dtype, int opA, int opB, size_t m, size_t n, size_t k,
                                        size_t lda, size_t ldb, size_t num_batches, size_t* bytes);
 SPFY_API int spfy_gemm_strided_batched(int dtype, int precision, int opA, int opB, size_t m, size_t n,

@@ -21,7 +21,6 @@ OP_N, OP_T = 0, 1
 OUT_T = 0x10  # flag OR-ed into opB: D is written transposed, [n][m]
 SPMM_ALG_DEFAULT, SPMM_ALG_CUDA_CORE, SPMM_ALG_TENSOR, SPMM_ALG_TENSOR_FAST = 0, 1, 2, 3
 GEMM_PRECISE, GEMM_FAST = 0, 1
-GEMM_CTA_PAIRS = 0x10  # flag, OR-ed into `precision`: the cta_group::2 kernel where it applies
 ACT_NONE, ACT_RELU, ACT_GELU_TANH = 0, 1, 2
 OK, E_INVALID, E_UNSUPPORTED, E_CUDA, E_WORKSPACE, E_NCCL = 0, -1, -2, -3, -4, -5
 

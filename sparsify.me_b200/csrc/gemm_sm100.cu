@@ -1,5 +1,5 @@
-// gemm_sm100.cu -- dense batched GEMM on tcgen05 (sm_100a): kind::f16 for fp16 / bf16 operands and
-// 3xTF32 (kind::tf32, split in shared memory) for fp32 operands at fp32-level accuracy.
+// gemm_sm100.cu -- dense batched GEMM on tcgen05 (sm_100a): kind::f16 for fp16 / bf16 operands, one kind::tf32
+// product for fp32 operands with SPFY_GEMM_FAST, and 3xTF32 at fp32-level accuracy for fp32 operands by default.
 //
 // Replaces the library contractions of the reference that are dense (or dense enough to be run densely):
 //     sparsifyme::batched::gemm          cublas{H,S}gemmBatched          include/sparsify.me/gemm.hxx:25-195
@@ -13,22 +13,23 @@
 // streamed dimension becomes Mu (128-row tiles = TMEM lanes) and the short one becomes Nu (one UMMA of up to 256
 // columns), e.g. a weight matrix with 64 rows costs N = 64 MMAs instead of a half-empty M = 128 tile.
 //
-// Persistent CTA of 320 threads, 1 CTA/SM, work unit = (problem, batch, m-tile, n-tile), n-tile fastest so that
-// CTAs running side by side share the streamed Au tile through L2:
+// Two kernels, both persistent with 1 CTA/SM and work unit = (problem, batch, m-group, n-tile), n-tile fastest so
+// that CTAs running side by side share the streamed Au tile through L2:
+//
+// tcgemm_kernel<KIND>: 16-bit operands, and fp32 operands with SPFY_GEMM_FAST.  192 threads:
 //   warp 0      producer : TMA tensor loads of the Au / Bu tiles of one 128-byte K slab per ring stage
-//   warp 1      MMA      : per stage 4 k-steps of 32 bytes; fp32 inputs issue three kind::tf32 MMAs per k-step
-//                          (hi*lo, lo*hi, hi*hi), 16-bit inputs one kind::f16 MMA
-//   warps 2-5   splitter : fp32 only: x -> hi = x rounded to TF32 (low 13 mantissa bits zero: the tensor core reads
-//                          it exactly), lo = x - hi (exact in fp32), hi over the raw tile and lo behind it;
-//                          the layout is irrelevant to an element-wise pass, so the swizzled tiles are
-//                          processed as flat bytes
-//   warps 6-9   epilogue : tcgen05.ld 32 columns at a time -> alpha / beta -> coalesced global stores
+//   warp 1      MMA      : per stage 4 k-steps of 32 bytes, one kind::f16 or kind::tf32 MMA each
+//   warps 2-5   epilogue : tcgen05.ld 16 columns at a time -> alpha / beta -> coalesced global stores
 // TMEM: two accumulator slots of 256 columns, so the epilogue of one unit overlaps the MMAs of the next.
 //
-// Accuracy of the fp32 path: hi carries 11 significant bits, |lo| <= 2^-11 |x| of which the tensor core reads the
-// leading 11 bits, and the lo*lo term (<= 2^-22) is dropped: every product is exact to ~2^-20 relative in the
-// worst case, accumulation is fp32.  The parity tests bound the result against an fp64 oracle by
-// 4e-6 * sum_k |a||b| (tests/test_gpu_tensor.py).
+// tcgemm_ts_kernel: fp32 operands with SPFY_GEMM_PRECISE (3xTF32, hi*lo + lo*hi + hi*hi).  480 threads; the streamed
+// Au tile is split in registers into hi and lo and stored to tensor memory, the MMAs read it from there, and the
+// small Bu tile keeps its raw bytes as hi with lo written behind it in shared memory (layout above the kernel).
+//
+// Accuracy of the 3xTF32 path: Au's hi is x rounded to TF32 (|lo| <= 2^-11 |x|), Bu's hi is x truncated to TF32 by
+// the tensor core (|lo| < 2^-10 |x|); the lo*lo term is dropped and each lo is read to TF32 precision, so every
+// product is exact to ~2^-19 relative in the worst case, accumulation is fp32.  The parity tests bound the result
+// against an fp64 oracle by 4e-6 * sum_k |a||b| (tests/test_gpu_tensor.py).
 #include "gemm_sm100.cuh"
 #include "tc_ptx.cuh"
 
@@ -44,8 +45,8 @@ constexpr int GM_BM = 128;        // rows of Au per tile (UMMA M)
 constexpr int GM_MAX_BN = 256;    // columns of one UMMA / TMEM slot
 constexpr int GM_ROW_BYTES = 128; // bytes of K per operand row and stage (one swizzle atom)
 constexpr int GM_A_BYTES = GM_BM * GM_ROW_BYTES;
-constexpr int GM_THREADS = 320;
-constexpr int GM_SPLIT_WARPS = 4, GM_EPI_WARPS = 4;
+constexpr int GM_THREADS = 192;  // producer, MMA and 4 epilogue warps
+constexpr int GM_EPI_WARPS = 4;
 constexpr int GM_ACC_SLOTS = 2;
 constexpr int GM_MAX_STAGES = 8;
 constexpr int GM_SMEM_LIMIT = 232448;
@@ -73,10 +74,11 @@ struct alignas(64) GemmProblemDev {
 struct GemmLaunch {
   const GemmProblemDev* table;  // null -> the single problem passed by value
   uint32_t num_problems, total_units;
-  uint32_t stages, stage_bytes, raw_bytes;  // stage = [Au raw 16 KiB][Bu raw bn_max*128] (+ the same again: lo parts)
+  uint32_t stages, stage_bytes, raw_bytes;  // stage = [Au 16 KiB][Bu bn_max*128]
+                                            // (3xTF32 kernel: Bu stage = [raw tile][lo tile], raw_bytes each)
   uint32_t bar_off;
-  uint32_t split;     // fp32: 3xTF32 (splitter warps run)
-  uint32_t write_hi;  // splitter also stores hi over the raw tile (independent of how the tensor core rounds)
+  uint32_t write_hi;  // 3xTF32 kernel (SPFY_GEMM_WRITE_HI, dev builds only): the Bu splitters also store hi = x rounded
+                      // to TF32 over the raw tile, instead of leaving the tensor core to truncate it
   uint32_t idesc;     // instruction descriptor without N and the major bits
   uint32_t kelems;    // elements of K per stage (32 fp32 / 64 half)
   const int* gate;    // optional device word: the launch does its work only if (*gate != 0) == gate_run_if
@@ -103,10 +105,6 @@ struct GemmWalker {
   __device__ __forceinline__ GemmWalker(const GemmProblemDev* s, const GemmLaunch& L)
       : single(s), table(L.table), num_problems(L.num_problems), total_units(L.total_units), u(blockIdx.x), p(0),
         stride(gridDim.x), p_begin(0), p_end(0) {}
-  // CTA pairs: both CTAs of a cluster walk the same units
-  __device__ __forceinline__ GemmWalker(const GemmProblemDev* s, const GemmLaunch& L, uint32_t first, uint32_t step)
-      : single(s), table(L.table), num_problems(L.num_problems), total_units(L.total_units), u(first), p(0), stride(step),
-        p_begin(0), p_end(0) {}
   __device__ __forceinline__ const GemmProblemDev* prob(uint32_t i) const { return table ? table + i : single; }
   __device__ __forceinline__ bool valid() const { return u < total_units; }
   __device__ __forceinline__ const GemmProblemDev* current() {
@@ -150,11 +148,7 @@ template <> struct OutT<KIND_BF16> { using type = __nv_bfloat16; };
 template <int KIND>
 __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base, uint32_t bar_acc_full, uint32_t bar_acc_empty,
                                               uint32_t slots, uint32_t slot_cols, uint32_t tile_cols, uint32_t warp,
-                                              uint32_t lane, uint32_t pair_rank = 0xffffffffu) {
-  // pair_rank != ~0: CTA pair (tcgemm2_kernel) -- a unit is two m-tiles, mine is number pair_rank, and the slot is handed
-  // back on the LEADER's barrier (the one thread that issues the MMAs for both CTAs waits there)
-  const bool pair = pair_rank != 0xffffffffu;
-  const uint32_t acc_empty_remote = pair ? mapa_shared(bar_acc_empty, 0) : 0u;
+                                              uint32_t lane) {
   using out_t = typename OutT<KIND>::type;
   const uint32_t quarter = warp & 3u;  // TMEM lanes [32*quarter, 32*quarter + 32)
   uint32_t job = 0;
@@ -173,13 +167,13 @@ __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base,
       alpha = P->alpha; beta = P->beta;
     }
     const uint32_t nt = W.nt, mg = W.md, b = W.bb;
-    const uint32_t g_count = pair ? 1u : min(g, m_tiles - mg * g);
+    const uint32_t g_count = min(g, m_tiles - mg * g);
     out_t* C = c_ptrs ? reinterpret_cast<out_t*>(c_ptrs[b]) : reinterpret_cast<out_t*>(Cbase) + (size_t)b * stride_c;
     const uint32_t slot = job % slots;
     mbar_wait(bar_acc_full + slot * 8, (job / slots) & 1u);
     tc_fence_after();
     for (uint32_t tile = 0; tile < g_count; ++tile) {
-    const uint32_t mt = pair ? mg * 2u + pair_rank : mg * g + tile;
+    const uint32_t mt = mg * g + tile;
     const uint32_t row = mt * GM_BM + quarter * 32u + lane;  // index along Mu
     const bool row_ok = row < mu;
     const bool warp_ok = mt * GM_BM + quarter * 32u < mu;
@@ -199,9 +193,7 @@ __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base,
         // accumulator fully read by this warp: hand the slot back to the MMA warp
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) {
-          if (pair) mbar_arrive_cluster(acc_empty_remote + slot * 8); else mbar_arrive(bar_acc_empty + slot * 8);
-        }
+        if (lane == 0) mbar_arrive(bar_acc_empty + slot * 8);
       }
       if (!row_ok || !ncols) continue;
       if (mu_contig) {
@@ -263,18 +255,16 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
   if (L.gate && (*L.gate != 0) != (L.gate_run_if != 0)) return;
 
   const uint32_t NS = L.stages;
-  const uint32_t bar_full = smem_base + L.bar_off;                   // [GM_MAX_STAGES] producer -> splitter / MMA
-  const uint32_t bar_conv = bar_full + GM_MAX_STAGES * 8;            // [GM_MAX_STAGES] splitter -> MMA
-  const uint32_t bar_empty = bar_conv + GM_MAX_STAGES * 8;           // [GM_MAX_STAGES] MMA -> producer
+  const uint32_t bar_full = smem_base + L.bar_off;                   // [GM_MAX_STAGES] producer -> MMA
+  const uint32_t bar_empty = bar_full + GM_MAX_STAGES * 8;           // [GM_MAX_STAGES] MMA -> producer
   const uint32_t bar_acc_full = bar_empty + GM_MAX_STAGES * 8;       // [GM_ACC_SLOTS]
   const uint32_t bar_acc_empty = bar_acc_full + GM_ACC_SLOTS * 8;    // [GM_ACC_SLOTS]
-  const uint32_t tmem_ptr_off = L.bar_off + (3 * GM_MAX_STAGES + 2 * GM_ACC_SLOTS) * 8;
+  const uint32_t tmem_ptr_off = L.bar_off + (2 * GM_MAX_STAGES + 2 * GM_ACC_SLOTS) * 8;
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem_gen + tmem_ptr_off);
 
   if (warp == 1 && lane == 0) {
     for (uint32_t s = 0; s < (uint32_t)GM_MAX_STAGES; ++s) {
       mbar_init(bar_full + s * 8, 1);
-      mbar_init(bar_conv + s * 8, GM_SPLIT_WARPS);
       mbar_init(bar_empty + s * 8, 1);
     }
     for (int a = 0; a < GM_ACC_SLOTS; ++a) {
@@ -348,9 +338,6 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
     const uint32_t kel = L.kelems;
     const uint32_t umma_k = kel / 4u;               // K elements per MMA (32 bytes)
     const uint32_t group_bytes = kel * GM_ROW_BYTES;
-    const uint32_t split = L.split;
-    const uint32_t wait_bar = split ? bar_conv : bar_full;
-    const uint32_t lo_off = L.raw_bytes >> 4;       // lo tiles sit raw_bytes behind the raw ones (16-byte units)
     // K-major: rows of 128 bytes, 8-row atoms 1024 bytes apart, a k-step advances 32 bytes inside the swizzled row.
     // MN-major: 128-byte groups of MN, 8 k-rows per 1024-byte atom (SBO), groups `group_bytes` apart (LBO); a k-step
     // is umma_k k-rows = umma_k * 128 bytes.
@@ -375,7 +362,7 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
       const uint32_t a_step = a_mn ? step_mn : 2u, b_step = b_mn ? step_mn : 2u;
       uint32_t k_left = pk;
       for (uint32_t kt = 0; kt < k_tiles; ++kt, k_left -= kel) {
-        mbar_wait(wait_bar + stage * 8, phase);
+        mbar_wait(bar_full + stage * 8, phase);
         tc_fence_after();
         const uint32_t sa = smem_base + stage * L.stage_bytes;
         const uint32_t a0 = (sa >> 4) & 0x3fffu, b0 = ((sa + GM_A_BYTES) >> 4) & 0x3fffu;
@@ -386,17 +373,8 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
             if (j < nk) {
               const uint64_t da = da_hi | (uint64_t)(a0 + a_step * j), db = db_hi | (uint64_t)(b0 + b_step * j);
               const uint32_t acc = (kt | j) ? 1u : 0u;
-              if (KIND == KIND_F32) {
-                if (split) {
-                  tc_mma_tf32(tmem_d, da, db + lo_off, idesc, acc);       // hi * lo
-                  tc_mma_tf32(tmem_d, da + lo_off, db, idesc, 1u);        // lo * hi
-                  tc_mma_tf32(tmem_d, da, db, idesc, 1u);                 // hi * hi
-                } else {
-                  tc_mma_tf32(tmem_d, da, db, idesc, acc);
-                }
-              } else {
-                tc_mma_f16(tmem_d, da, db, idesc, acc);
-              }
+              if (KIND == KIND_F32) tc_mma_tf32(tmem_d, da, db, idesc, acc);
+              else                  tc_mma_f16(tmem_d, da, db, idesc, acc);
             }
           }
           tc_commit(bar_empty + stage * 8);
@@ -405,41 +383,6 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
       }
       if (leader) tc_commit(bar_acc_full + slot * 8);
       ++job;
-    }
-  } else if (warp < 2 + GM_SPLIT_WARPS) {
-    // ===================== splitter (fp32 inputs only) =====================
-    if (L.split) {
-      const uint32_t t = threadIdx.x - 64u;
-      uint32_t stage = 0, phase = 0;
-      const GemmProblemDev* last = nullptr;
-      uint32_t k_tiles = 0, bn = 0;
-      const uint32_t raw = L.raw_bytes;
-      const bool write_hi = L.write_hi != 0;
-      for (; W.valid(); W.next()) {
-        const GemmProblemDev* P = W.current();
-        if (P != last) { last = P; k_tiles = P->k_tiles; bn = P->bn; }
-        const uint32_t used = (uint32_t)GM_A_BYTES + bn * (uint32_t)GM_ROW_BYTES;  // Au and Bu raw tiles are adjacent
-        for (uint32_t kt = 0; kt < k_tiles; ++kt) {
-          mbar_wait(bar_full + stage * 8, phase);
-          const uint32_t sa = smem_base + stage * L.stage_bytes;
-#pragma unroll 4
-          for (uint32_t off = t * 16u; off < used; off += GM_SPLIT_WARPS * 32u * 16u) {
-            const uint4 x = ld_shared_v4(sa + off);
-            // hi = x rounded to the nearest TF32 (half up in magnitude; a carry into the exponent is the right
-            // answer too), so |lo| <= 2^-11 |x| and x - hi is exact in fp32
-            const uint32_t h0 = (x.x + 0x1000u) & 0xffffe000u, h1 = (x.y + 0x1000u) & 0xffffe000u;
-            const uint32_t h2 = (x.z + 0x1000u) & 0xffffe000u, h3 = (x.w + 0x1000u) & 0xffffe000u;
-            const float l0 = __uint_as_float(x.x) - __uint_as_float(h0), l1 = __uint_as_float(x.y) - __uint_as_float(h1);
-            const float l2 = __uint_as_float(x.z) - __uint_as_float(h2), l3 = __uint_as_float(x.w) - __uint_as_float(h3);
-            st_shared_v4(sa + raw + off, __float_as_uint(l0), __float_as_uint(l1), __float_as_uint(l2), __float_as_uint(l3));
-            if (write_hi) st_shared_v4(sa + off, h0, h1, h2, h3);
-          }
-          fence_proxy_async_smem();  // generic-proxy writes -> visible to the tensor core's async-proxy reads
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar_conv + stage * 8);
-          if (++stage == NS) { stage = 0; phase ^= 1u; }
-        }
-      }
     }
   } else {
     gemm_epilogue<KIND>(W, tmem_base, bar_acc_full, bar_acc_empty, GM_ACC_SLOTS, GM_MAX_BN, GM_MAX_BN, warp, lane);
@@ -454,181 +397,9 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// CTA pairs (cta_group::2): the same GEMM on tiles of 256 rows of Au.
-//
-// The single-CTA kernel above is bound by the bytes that ENTER an SM, not by the tensor pipe: a 128 x 256 tile takes
-// (128 + 256) x 128 bytes of operands per K slab for 512 tensor cycles (96 B/clk, the L2 -> SM path gives ~25).  Two CTAs
-// of a cluster on the two SMs of a TPC run ONE tcgen05.mma of M = 256: each CTA loads its own 128 rows of Au and only
-// HALF of the Bu tile (the tensor cores read the other half from the peer's shared memory), so the weight tile enters
-// each SM half as often -- (128 + 128) x 128 bytes per slab and CTA -- and the ring is 6 deep instead of 4.
-//   both CTAs : producer warp (its Au tile + its half of Bu; the bytes are counted on the LEADER's `full` barrier),
-//               epilogue warps (own accumulator rows from own tensor memory; slot handed back on the leader's barrier)
-//   leader    : MMA warp: waits the leader's `full`, issues the MMAs for the pair, commits with a multicast arrive on
-//               the `empty` / `acc_full` barriers of both CTAs
-// Units: (problem, batch, pair of m-tiles, n-tile), n-tile fastest; both CTAs of a cluster walk the same sequence.
-// 16-bit operands and single-product TF32 only (no splitter warps).
-// ------------------------------------------------------------------------------------------------------------
-template <int KIND>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GM_THREADS, 1)
-tcgemm2_kernel(const __grid_constant__ GemmProblemDev single, const __grid_constant__ GemmLaunch L) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  // (no early return for a gated launch before the cluster barriers: both CTAs take the same branch)
-  const bool gated_off = L.gate && (*L.gate != 0) != (L.gate_run_if != 0);
-  if (gated_off) return;
-
-  const uint32_t NS = L.stages;
-  const uint32_t bar_full = smem_base + L.bar_off;                   // [GM_MAX_STAGES] used in the leader only
-  const uint32_t bar_empty = bar_full + GM_MAX_STAGES * 8;           // [GM_MAX_STAGES] per CTA (multicast commit)
-  const uint32_t bar_acc_full = bar_empty + GM_MAX_STAGES * 8;       // [GM_ACC_SLOTS]  per CTA (multicast commit)
-  const uint32_t bar_acc_empty = bar_acc_full + GM_ACC_SLOTS * 8;    // [GM_ACC_SLOTS]  used in the leader only
-  const uint32_t tmem_ptr_off = L.bar_off + (2 * GM_MAX_STAGES + 2 * GM_ACC_SLOTS) * 8;
-  volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem_gen + tmem_ptr_off);
-
-  if (warp == 1 && lane == 0) {
-    for (uint32_t s = 0; s < (uint32_t)GM_MAX_STAGES; ++s) {
-      mbar_init(bar_full + s * 8, 1);
-      mbar_init(bar_empty + s * 8, 1);
-    }
-    for (int a = 0; a < GM_ACC_SLOTS; ++a) {
-      mbar_init(bar_acc_full + a * 8, 1);
-      mbar_init(bar_acc_empty + a * 8, 2 * GM_EPI_WARPS);  // the epilogue warps of both CTAs
-    }
-    fence_barrier_init();
-  }
-  if (warp == 2) tmem_alloc_2cta(smem_base + tmem_ptr_off, 512);
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();  // the peer's barriers exist before anything of mine can arrive on them
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
-
-  GemmWalker W(&single, L, blockIdx.x >> 1, gridDim.x >> 1);
-
-  if (warp == 0) {
-    // ===================== producer (both CTAs) =====================
-    const bool leader = elect_one();
-    uint32_t stage = 0, phase = 0;
-    const GemmProblemDev* last = nullptr;
-    const CUtensorMap *tmap_a = nullptr, *tmap_b = nullptr;
-    uint32_t n_tiles = 1, m_pairs = 1, k_tiles = 0, bn = 0, a_mn = 0, b_mn = 0, a_bat = 0, b_bat = 0, unit_begin = 0;
-    const uint32_t kel = L.kelems;
-    const uint32_t gsz = kel;
-    const uint32_t group_bytes = kel * GM_ROW_BYTES;
-    const uint32_t full0 = mapa_shared(bar_full, 0);  // the leader's `full` barriers as seen from here
-    for (; W.valid(); W.next()) {
-      const GemmProblemDev* P = W.current();
-      if (P != last) {
-        last = P;
-        tmap_a = &P->tmap_a; tmap_b = &P->tmap_b;
-        if (leader) { prefetch_tmap(tmap_a); prefetch_tmap(tmap_b); }
-        n_tiles = uni(P->n_tiles); m_pairs = uni(P->m_groups); k_tiles = uni(P->k_tiles); bn = uni(P->bn);
-        a_mn = uni(P->a_mn); b_mn = uni(P->b_mn); a_bat = uni(P->a_batched); b_bat = uni(P->b_batched);
-        unit_begin = uni(P->unit_begin);
-      }
-      const uint32_t nt = W.nt, mp = W.md, b = W.bb;
-      const uint32_t mt = mp * 2u + rank;                 // my m-tile of the pair
-      const uint32_t half = bn >> 1, n0 = nt * bn + rank * half;  // my half of the Bu tile
-      const int ba = a_bat ? (int)b : 0, bb = b_bat ? (int)b : 0;
-      const uint32_t tx_pair = 2u * ((uint32_t)GM_A_BYTES + half * (uint32_t)GM_ROW_BYTES);
-      for (uint32_t kt = 0; kt < k_tiles; ++kt) {
-        mbar_wait(bar_empty + stage * 8, phase ^ 1u);
-        const uint32_t full = full0 + stage * 8;
-        const uint32_t sa = smem_base + stage * L.stage_bytes, sb = sa + GM_A_BYTES;
-        if (leader) {
-          if (rank == 0) mbar_expect_tx(bar_full + stage * 8, tx_pair);
-          if (!a_mn) {
-            tma_load_3d_2cta(sa, tmap_a, (int)(kt * kel), (int)(mt * GM_BM), ba, full, HINT_EVICT_NORMAL);
-          } else {
-            for (uint32_t g = 0; g * gsz < (uint32_t)GM_BM; ++g)
-              tma_load_3d_2cta(sa + g * group_bytes, tmap_a, (int)(mt * GM_BM + g * gsz), (int)(kt * kel), ba, full,
-                               HINT_EVICT_NORMAL);
-          }
-          if (!b_mn) {
-            tma_load_3d_2cta(sb, tmap_b, (int)(kt * kel), (int)n0, bb, full, HINT_EVICT_NORMAL);
-          } else {
-            for (uint32_t g = 0; g * gsz < half; ++g)
-              tma_load_3d_2cta(sb + g * group_bytes, tmap_b, (int)(n0 + g * gsz), (int)(kt * kel), bb, full,
-                               HINT_EVICT_NORMAL);
-          }
-        }
-        if (++stage == NS) { stage = 0; phase ^= 1u; }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer (leader CTA only) =====================
-    if (rank == 0) {
-      const bool leader = elect_one();
-      const uint32_t tmem_b = uni(tmem_base);
-      uint32_t stage = 0, phase = 0, job = 0;
-      const GemmProblemDev* last = nullptr;
-      uint32_t k_tiles = 0, pk = 0, bn = 0, a_mn = 0, b_mn = 0;
-      const uint32_t kel = L.kelems;
-      const uint32_t umma_k = kel / 4u;
-      const uint32_t group_bytes = kel * GM_ROW_BYTES;
-      const uint64_t desc_k = make_smem_desc(0, 16, 1024, LAYOUT_SW128);
-      const uint64_t desc_mn = KIND == KIND_F32 ? make_smem_desc(0, group_bytes, 512, LAYOUT_SW128_BASE32B)
-                                                : make_smem_desc(0, group_bytes, 1024, LAYOUT_SW128);
-      const uint32_t step_mn = (umma_k * GM_ROW_BYTES) >> 4;
-      for (; W.valid(); W.next()) {
-        const GemmProblemDev* P = W.current();
-        if (P != last) {
-          last = P;
-          k_tiles = uni(P->k_tiles); pk = uni(P->k); bn = uni(P->bn); a_mn = uni(P->a_mn); b_mn = uni(P->b_mn);
-        }
-        const uint32_t slot = job % GM_ACC_SLOTS, use = job / GM_ACC_SLOTS;
-        mbar_wait(bar_acc_empty + slot * 8, (use & 1u) ^ 1u);
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_b + slot * (uint32_t)GM_MAX_BN;
-        // M = 256 for the pair; N = the whole Bu tile (its halves sit in the two CTAs)
-        const uint32_t idesc = L.idesc | (a_mn << 15) | (b_mn << 16) | ((bn >> 3) << 17);
-        const uint64_t da_hi = a_mn ? desc_mn : desc_k, db_hi = b_mn ? desc_mn : desc_k;
-        const uint32_t a_step = a_mn ? step_mn : 2u, b_step = b_mn ? step_mn : 2u;
-        uint32_t k_left = pk;
-        for (uint32_t kt = 0; kt < k_tiles; ++kt, k_left -= kel) {
-          mbar_wait(bar_full + stage * 8, phase);
-          tc_fence_after();
-          const uint32_t sa = smem_base + stage * L.stage_bytes;
-          const uint32_t a0 = (sa >> 4) & 0x3fffu, b0 = ((sa + GM_A_BYTES) >> 4) & 0x3fffu;
-          const uint32_t nk = k_left >= kel ? 4u : (k_left + umma_k - 1u) / umma_k;
-          if (leader) {
-#pragma unroll
-            for (uint32_t j = 0; j < 4; ++j) {
-              if (j < nk) {
-                const uint64_t da = da_hi | (uint64_t)(a0 + a_step * j), db = db_hi | (uint64_t)(b0 + b_step * j);
-                const uint32_t acc = (kt | j) ? 1u : 0u;
-                if (KIND == KIND_F32) tc_mma_tf32_2cta(tmem_d, da, db, idesc, acc);
-                else                  tc_mma_f16_2cta(tmem_d, da, db, idesc, acc);
-              }
-            }
-            tc_commit_2cta(bar_empty + stage * 8, 3u);  // the stage is free in both CTAs
-          }
-          if (++stage == NS) { stage = 0; phase ^= 1u; }
-        }
-        if (leader) tc_commit_2cta(bar_acc_full + slot * 8, 3u);
-        ++job;
-      }
-    }
-  } else if (warp >= 2 + GM_SPLIT_WARPS) {
-    gemm_epilogue<KIND>(W, tmem_base, bar_acc_full, bar_acc_empty, GM_ACC_SLOTS, GM_MAX_BN, GM_MAX_BN, warp, lane, rank);
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();  // nobody retires (or frees tensor memory) while the peer may still arrive on its barriers
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_2cta(tmem_base, 512);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------------
 // fp32 operands at fp32-level accuracy (3xTF32) with the streamed operand in TENSOR MEMORY.
 //
-// Run from shared memory (the kernel above with `split`), 3xTF32 is bound by shared-memory bandwidth, not by the
+// With both operands split in shared memory, 3xTF32 is bound by shared-memory bandwidth, not by the
 // tensor pipe or HBM: per 32-wide K slab the (128 + N) x 128 bytes of operands are written by TMA, read and
 // written twice over by the splitter (hi, lo) and read three times by the MMAs -- 7 passes at 128 B/clk
 // (measured: 2000 cycles per slab at N = 64 against 720 for HBM).  Here the splitter warps take the raw Au tile
@@ -646,7 +417,7 @@ tcgemm2_kernel(const __grid_constant__ GemmProblemDev single, const __grid_const
 //                          handed back as soon as it has been read
 //   warps 11-14 Bu splitters: lo = x - trunc(x) behind the raw tile (the tensor core ignores the low 13 mantissa bits itself)
 //   warp 1      MMA      : per m-tile and k-step hi*lo, lo*hi, hi*hi; commits free the Bu stage and the TMEM operand slot
-//   warps 6-9   epilogue : as above, one accumulator per m-tile
+//   warps 6-9   epilogue : as in tcgemm_kernel, one accumulator per m-tile
 // TMEM (512 columns): accumulators [0, 256) = slots x 2 m-tiles x (64 or 128) columns -- two slots when every tile of the
 // launch has at most 64 columns, else one; Au operand ring [256, 512) = 2 slots x 2 m-tiles x (32 hi + 32 lo).
 // An MN-major Au tile is fetched unswizzled (a thread reads its row as 32 conflict-free 4-byte loads); an
@@ -659,8 +430,9 @@ constexpr int TS_T_SLOTS = 2;                       // TMEM operand slots (each 
 constexpr int TS_B_STAGES = 4;
 constexpr int TS_MAX_A_STAGES = 8;
 constexpr int TS_A_STAGE_BYTES = TS_G * GM_A_BYTES; // one K slab of the unit's m-tiles
-constexpr int TS_BSPLIT_WARPS = 4;
-constexpr int TS_THREADS = GM_THREADS + 32 + TS_BSPLIT_WARPS * 32;  // + warp 10 (Bu producer) + warps 11-14 (Bu splitters)
+constexpr int TS_ASPLIT_WARPS = 4;                  // warps 2-5
+constexpr int TS_BSPLIT_WARPS = 4;                  // warps 11-14
+constexpr int TS_THREADS = (2 + TS_ASPLIT_WARPS + GM_EPI_WARPS + 1 + TS_BSPLIT_WARPS) * 32;  // warps 0-14
 
 // (15 warps: a scheduler holds four of them, so a thread gets at most 16384 / 4 / 32 = 128 registers)
 __global__ void __launch_bounds__(TS_THREADS, 1)
@@ -686,11 +458,11 @@ tcgemm_ts_kernel(const __grid_constant__ GemmProblemDev single, const __grid_con
   if (warp == 1 && lane == 0) {
     for (uint32_t s = 0; s < (uint32_t)TS_MAX_A_STAGES; ++s) {
       mbar_init(bar_afull + s * 8, 1);
-      mbar_init(bar_aempty + s * 8, GM_SPLIT_WARPS);
+      mbar_init(bar_aempty + s * 8, TS_ASPLIT_WARPS);
     }
     for (uint32_t s = 0; s < (uint32_t)TS_B_STAGES; ++s) {
       mbar_init(bar_bfull + s * 8, 1);
-      mbar_init(bar_ready + s * 8, GM_SPLIT_WARPS + TS_BSPLIT_WARPS);
+      mbar_init(bar_ready + s * 8, TS_ASPLIT_WARPS + TS_BSPLIT_WARPS);
       mbar_init(bar_bfree + s * 8, 1);
     }
     for (uint32_t s = 0; s < (uint32_t)TS_T_SLOTS; ++s) mbar_init(bar_tfree + s * 8, 1);
@@ -840,7 +612,7 @@ tcgemm_ts_kernel(const __grid_constant__ GemmProblemDev single, const __grid_con
       if (leader) tc_commit(bar_acc_full + slot * 8);
       ++job;
     }
-  } else if (warp < 2 + GM_SPLIT_WARPS) {
+  } else if (warp < 2 + TS_ASPLIT_WARPS) {
     // ===================== Au splitters: thread = one row of a tile = one TMEM lane =====================
     const uint32_t row = (warp & 3u) * 32u + lane;  // the TMEM lane quarter a warp may touch is warp % 4
     uint32_t sa = 0, pha = 0, sb = 0, phb = 0, slab = 0;
@@ -1048,8 +820,7 @@ void blas_views(const TcGemmProblem& p, OperandView* va, OperandView* vb) {
   *vb = OperandView{p.B, p.n, p.k, p.ldb, p.strideB, p.opB != SPFY_OP_N};
 }
 
-// `pair`: CTA pairs split a Bu tile in halves, each a whole number of 16-column (or MN-group) units
-Orientation orient(int dtype, const TcGemmProblem& p, size_t max_bn, bool pair = false) {
+Orientation orient(int dtype, const TcGemmProblem& p, size_t max_bn) {
   OperandView va, vb;
   blas_views(p, &va, &vb);
   const size_t group = GM_ROW_BYTES / elem_bytes(dtype);
@@ -1058,7 +829,7 @@ Orientation orient(int dtype, const TcGemmProblem& p, size_t max_bn, bool pair =
   o[0].a = va; o[0].b = vb; o[0].mu = p.m; o[0].nu = p.n; o[0].mu_contig = true;
   o[1].a = vb; o[1].b = va; o[1].mu = p.n; o[1].nu = p.m; o[1].mu_contig = false;
   for (int i = 0; i < 2; ++i) {
-    split_nu(o[i].nu, (o[i].b.mn_major ? group : 16) * (pair ? 2 : 1), max_bn, &o[i].bn, &o[i].n_tiles);
+    split_nu(o[i].nu, o[i].b.mn_major ? group : 16, max_bn, &o[i].bn, &o[i].n_tiles);
     o[i].padded = round_up(o[i].mu, GM_BM) * (size_t)o[i].bn * o[i].n_tiles;
   }
   if (o[0].padded != o[1].padded) return o[0].padded < o[1].padded ? o[0] : o[1];
@@ -1114,10 +885,10 @@ void balance_tiles(const Orientation& o, size_t nb, size_t k_tiles, int sm_count
 
 // `launch_half_units`: units of the whole launch if every problem paired its m-tiles (the G = 2 rule looks at the launch,
 // not at one problem: a pointer-array batch is a table of one-batch problems)
-int fill_problem(GemmProblemDev* d, int dtype, const TcGemmProblem& p, bool ts, int sm_count, bool pair = false,
-                 bool alone = false, uint64_t launch_half_units = 0) {
+int fill_problem(GemmProblemDev* d, int dtype, const TcGemmProblem& p, bool ts, int sm_count, bool alone = false,
+                 uint64_t launch_half_units = 0) {
   memset(d, 0, sizeof(*d));
-  Orientation o = orient(dtype, p, ts ? TS_MAX_BN : GM_MAX_BN, pair);
+  Orientation o = orient(dtype, p, ts ? TS_MAX_BN : GM_MAX_BN);
   uint32_t g_balanced = 0;
   if (ts && alone && !dev_switch("SPFY_GEMM_NO_BALANCE"))
     balance_tiles(o, p.nb, ceil_div(p.k, GM_ROW_BYTES / elem_bytes(dtype)), sm_count,
@@ -1130,7 +901,7 @@ int fill_problem(GemmProblemDev* d, int dtype, const TcGemmProblem& p, bool ts, 
   const CUtensorMapSwizzle sw_b = f32 && o.b.mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B;
   int rc = make_operand_map(&d->tmap_a, dtype, o.a, p.nb, GM_BM, sw_a);
   if (rc) return rc;
-  rc = make_operand_map(&d->tmap_b, dtype, o.b, p.nb, pair ? o.bn / 2 : o.bn, sw_b);  // a CTA of a pair loads half a tile
+  rc = make_operand_map(&d->tmap_b, dtype, o.b, p.nb, o.bn, sw_b);
   if (rc) return rc;
   const size_t kel = GM_ROW_BYTES / elem_bytes(dtype);
   d->C = (uint8_t*)p.C;
@@ -1159,7 +930,6 @@ int fill_problem(GemmProblemDev* d, int dtype, const TcGemmProblem& p, bool ts, 
   if (ts && d->m_tiles >= 2 && 2 * half_units >= (uint64_t)sm_count && !dev_switch("SPFY_GEMM_G1"))
     d->g = TS_G;
   if (g_balanced) d->g = g_balanced;
-  if (pair) d->g = 2;  // a unit is a pair of m-tiles, one per CTA of the cluster
   d->m_groups = (uint32_t)ceil_div(d->m_tiles, d->g);
   const uint64_t units = (uint64_t)d->m_groups * d->n_tiles * d->nb;
   if (units >= (1ull << 31)) return fail(SPFY_E_UNSUPPORTED, "tc_gemm: too many tiles");
@@ -1173,15 +943,6 @@ int launch_kind(const GemmProblemDev& single, const GemmLaunch& L, uint32_t smem
   if (rc) return rc;
   tcgemm_kernel<KIND><<<grid, GM_THREADS, smem, s>>>(single, L);
   SPFY_LAUNCH_OK("tcgemm_kernel");
-  return SPFY_OK;
-}
-
-template <int KIND>
-int launch_pairs(const GemmProblemDev& single, const GemmLaunch& L, uint32_t smem, int grid, cudaStream_t s) {
-  int rc = allow_dynamic_smem<tcgemm2_kernel<KIND>>(GM_SMEM_LIMIT);
-  if (rc) return rc;
-  tcgemm2_kernel<KIND><<<grid, GM_THREADS, smem, s>>>(single, L);  // clusters of two (__cluster_dims__)
-  SPFY_LAUNCH_OK("tcgemm2_kernel");
   return SPFY_OK;
 }
 
@@ -1200,9 +961,6 @@ void warm_gemm_kernels() {
   touch_kernel(tcgemm_kernel<KIND_F16>);
   touch_kernel(tcgemm_kernel<KIND_BF16>);
   touch_kernel(tcgemm_kernel<KIND_F32>);
-  touch_kernel(tcgemm2_kernel<KIND_F16>);
-  touch_kernel(tcgemm2_kernel<KIND_BF16>);
-  touch_kernel(tcgemm2_kernel<KIND_F32>);
 }
 
 int tc_gemm_supported(int dtype, const TcGemmProblem& p, bool allow_repack) {
@@ -1269,6 +1027,8 @@ int repack_operand(int dtype, OperandView* v, size_t nb, uint8_t* ws, size_t ws_
 
 int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t count, void* ws, size_t ws_bytes,
                 cudaStream_t stream, const int* gate, int gate_run_if) {
+  if (precision != TC_GEMM_PRECISE && precision != TC_GEMM_FAST)
+    return fail(SPFY_E_INVALID, "tc_gemm: precision %d (need SPFY_GEMM_PRECISE or SPFY_GEMM_FAST)", precision);
   if (count == 0) return SPFY_OK;
   if (!problems) return fail(SPFY_E_INVALID, "tc_gemm: null problem list");
   DeviceInfo di;
@@ -1277,25 +1037,13 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
   std::vector<GemmProblemDev> table;
   table.reserve(count);
   uint32_t units = 0, bn_max = 16;
-  const bool want_pairs = (precision & TC_GEMM_CTA_PAIRS) != 0;
-  precision &= ~TC_GEMM_CTA_PAIRS;
-  const bool ts = dtype == SPFY_F32 && precision == TC_GEMM_PRECISE && !dev_switch("SPFY_GEMM_NO_TMEM_A");
+  const bool ts = dtype == SPFY_F32 && precision == TC_GEMM_PRECISE;
   // workspace: [device copy of the problem table (count > 1)][padded copies of operands TMA cannot address]
   uint8_t* ws8 = (uint8_t*)ws;
   const size_t ws_pad = ws8 ? (256 - (uintptr_t)ws8 % 256) % 256 : 0;
   if (ws8 && ws_bytes >= ws_pad) { ws8 += ws_pad; ws_bytes -= ws_pad; } else { ws8 = nullptr; ws_bytes = 0; }
   size_t ws_used = table_bytes(count);
   std::vector<Repacked> repacked;
-  // CTA pairs (tcgemm2_kernel) on request, when no operand needs splitting and every problem has at least two m-tiles.
-  // Not the default: measured on the ResNet shapes the pair kernel is 5-25 % SLOWER than the single-CTA one
-  // (profiles/r02_gemm_cta_pairs.txt) -- it halves the weight bytes entering each SM, but its loads run at 6.2 TB/s
-  // chip-wide against 11.2 TB/s (the L2 output limit) for single CTAs.
-  bool pair = want_pairs && !ts && !(dtype == SPFY_F32 && precision == TC_GEMM_PRECISE) && di.sm_count >= 2;
-  for (size_t i = 0; i < count && pair; ++i) {
-    if (check_problem(dtype, problems[i], true) != SPFY_OK || problems[i].m == 0 || problems[i].n == 0 || problems[i].nb == 0)
-      continue;
-    if (orient(dtype, problems[i], GM_MAX_BN, true).mu <= (size_t)GM_BM) pair = false;
-  }
   uint64_t launch_half_units = 0;
   for (size_t i = 0; i < count && ts; ++i) {
     if (check_problem(dtype, problems[i], true) != SPFY_OK || problems[i].m == 0 || problems[i].n == 0 || problems[i].nb == 0)
@@ -1319,7 +1067,7 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
       q.B = vb.base; q.ldb = vb.ld; q.strideB = vb.stride;
     }
     GemmProblemDev d;
-    rc = fill_problem(&d, dtype, q, ts, di.sm_count, pair, count == 1, launch_half_units);
+    rc = fill_problem(&d, dtype, q, ts, di.sm_count, count == 1, launch_half_units);
     if (rc) return rc;
     d.unit_begin = units;
     if ((uint64_t)units + d.units >= (1ull << 31)) return fail(SPFY_E_UNSUPPORTED, "tc_gemm: too many tiles");
@@ -1332,11 +1080,8 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
   GemmLaunch L;
   memset(&L, 0, sizeof(L));
   const bool f32 = dtype == SPFY_F32;
-  L.split = f32 && precision == TC_GEMM_PRECISE;
   // The tensor core ignores the low 13 mantissa bits of a TF32 operand (measured: tools/gpu_wh.sh, same error with and
   // without the store), so the 3xTF32 kernel leaves the raw Bu tile in place as "hi" and only writes lo = x - trunc(x).
-  // The shared-memory-only split of the kernel above keeps writing a rounded hi.
-  L.write_hi = ts ? 0 : 1;
   if (const char* e = dev_switch("SPFY_GEMM_WRITE_HI")) L.write_hi = (uint32_t)atoi(e);
   L.kelems = (uint32_t)(GM_ROW_BYTES / elem_bytes(dtype));
   L.gate = gate;
@@ -1362,8 +1107,7 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
     L.bar_off = L.b_off + L.stages * L.stage_bytes;
     smem = L.bar_off + GM_BAR_BYTES + 1024u;
   } else {
-    L.raw_bytes = (uint32_t)GM_A_BYTES + (pair ? bn_max / 2 : bn_max) * (uint32_t)GM_ROW_BYTES;
-    L.stage_bytes = L.raw_bytes * (L.split ? 2u : 1u);
+    L.stage_bytes = (uint32_t)GM_A_BYTES + bn_max * (uint32_t)GM_ROW_BYTES;
     uint32_t stages = (GM_SMEM_LIMIT - 1024u - GM_BAR_BYTES) / L.stage_bytes;
     if (stages > (uint32_t)GM_MAX_STAGES) stages = GM_MAX_STAGES;
     if (const char* e = dev_switch("SPFY_GEMM_STAGES")) {
@@ -1377,7 +1121,7 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
   }
   // instruction descriptor: D = F32; A / B format (F16 0, BF16 1, TF32 2); M = 128; N and majors per problem
   const uint32_t fmt = f32 ? 2u : (dtype == SPFY_BF16 ? 1u : 0u);
-  L.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)((pair ? 2 * GM_BM : GM_BM) >> 4) << 24);
+  L.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(GM_BM >> 4) << 24);
   L.num_problems = (uint32_t)table.size();
   L.total_units = units;
   L.table = nullptr;
@@ -1388,12 +1132,6 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
     // pageable source: the runtime stages the bytes before the call returns, so `table` may go out of scope
     SPFY_CUDA_OK(cudaMemcpyAsync(ws8, table.data(), need, cudaMemcpyHostToDevice, stream));
     L.table = reinterpret_cast<const GemmProblemDev*>(ws8);
-  }
-  if (pair) {
-    const int grid2 = 2 * (int)std::min<uint32_t>(units, (uint32_t)di.sm_count / 2);
-    if (f32) return launch_pairs<KIND_F32>(table[0], L, smem, grid2, stream);
-    if (dtype == SPFY_BF16) return launch_pairs<KIND_BF16>(table[0], L, smem, grid2, stream);
-    return launch_pairs<KIND_F16>(table[0], L, smem, grid2, stream);
   }
   const int grid = (int)std::min<uint32_t>(units, (uint32_t)di.sm_count);
   if (ts) return launch_ts(table[0], L, smem, grid, stream);

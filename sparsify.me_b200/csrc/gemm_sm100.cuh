@@ -23,7 +23,7 @@ struct TcGemmProblem {
   float alpha = 1.f, beta = 0.f;
 };
 
-enum { TC_GEMM_PRECISE = 0, TC_GEMM_FAST = 1, TC_GEMM_CTA_PAIRS = 0x10 /* flag: cta_group::2 kernel where it applies */ };  // fp32 inputs: 3xTF32 (fp32-level accuracy) / one TF32 product
+enum { TC_GEMM_PRECISE = 0, TC_GEMM_FAST = 1 };  // fp32 inputs: 3xTF32 (fp32-level accuracy) / one TF32 product
 
 // TMA contract for an operand: 16-byte aligned base, leading dimension and batch stride multiples of 16 bytes.
 // tc_gemm_run copies an operand that misses it into the workspace with padded rows first (one extra pass over that

@@ -319,74 +319,6 @@ __device__ __forceinline__ uint4 ld_shared_v4(uint32_t addr) {
   return v;
 }
 
-// ---- CTA pairs (cta_group::2): two CTAs of a cluster on the two SMs of a TPC run ONE MMA of M = 256.  Each CTA holds
-// its own 128 rows of A and HALF of the B tile; the leader (cluster rank 0) issues the MMAs for both, the accumulator
-// rows of a CTA land in its own tensor memory.
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n"
-               "barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// address of the same shared-memory location in the CTA of rank `rank` (shared::cluster window)
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA load into MY shared memory whose bytes are counted on an mbarrier of either CTA of the pair (`bar`: a
-// shared::cluster address, e.g. mapa_shared(bar, 0) for the leader's)
-__device__ __forceinline__ void tma_load_3d_2cta(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2,
-                                                 uint32_t bar, uint64_t hint) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-      " [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "l"(hint)
-      : "memory");
-}
-// executed by the same warp of BOTH CTAs of the pair
-__device__ __forceinline__ void tmem_alloc_2cta(uint32_t smem_dst, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(cols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2cta(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-// arrives on the mbarrier at this shared-memory offset in every CTA of `cta_mask` once the MMAs issued so far are done
-__device__ __forceinline__ void tc_commit_2cta(uint32_t bar, uint32_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"((uint16_t)cta_mask)
-               : "memory");
-}
-__device__ __forceinline__ void tc_mma_f16_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tc_mma_tf32_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                 uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
-      "}\n"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 }  // namespace ptx
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda)

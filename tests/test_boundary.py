@@ -50,6 +50,12 @@ def test_argument_errors_do_not_fall_back(spfy):
     assert e.value.code == capi.E_UNSUPPORTED
     with pytest.raises(spfy.SpfyError):
         capi.spfy_convert(capi.F64, capi.F16, ctypes.c_void_p(16), ctypes.c_void_p(16), 4, None)
+    for dt in (capi.F16, capi.BF16, capi.F32):
+        for prec in (0x10, 2):
+            with pytest.raises(spfy.SpfyError) as e:
+                capi.spfy_gemm_strided_batched(dt, prec, capi.OP_N, capi.OP_N, 8, 8, 8, 1.0, None, 8, 0, None, 8, 0, 0.0,
+                                               None, 8, 0, 1, None, 0, None)
+            assert e.value.code == capi.E_INVALID and "precision" in str(e.value)
 
 
 def test_host_tensors_are_rejected(spfy):

@@ -87,17 +87,34 @@ def test_gemm_half_matches_fp64(spfy, cuda, tdt, m, n, k, nb, ta, tb):
 @pytest.mark.parametrize("m,n,k,nb", [(200, 72, 104, 3), (520, 264, 1000, 2), (64, 392, 256, 2), (784, 256, 2304, 2),
                                       (1000, 520, 72, 1), (300, 16, 40, 2)])
 @pytest.mark.parametrize("ta,tb", [(0, 0), (1, 0), (0, 1), (1, 1)])
-def test_gemm_cta_pairs_give_the_same_results(spfy, cuda, tdt, m, n, k, nb, ta, tb):
-    """GEMM_CTA_PAIRS: tcgen05.mma.cta_group::2 (M = 256 across a two-CTA cluster, each CTA holding its own 128 rows of
-    the long operand and half of the other tile; odd tile counts, ragged edges, every major-ness) -- bitwise the
-    results of the single-CTA kernel (same products, same accumulation order), and within the fp64 bound"""
+def test_gemm_single_product_alpha_beta_matches_fp64(spfy, cuda, tdt, m, n, k, nb, ta, tb):
+    """the shared-memory kernel (fp16 / bf16, fp32 as one TF32 product) with alpha = 0.5, beta = 0.25: odd tile counts,
+    ragged edges, every major-ness, within the fp64 bound"""
     prec = spfy.GEMM_FAST if tdt == torch.float32 else spfy.GEMM_PRECISE
-    one, want, bound = gemm_case(spfy, cuda, tdt, m, n, k, nb, ta, tb, 0.5, 0.25, False, nb > 1, prec, True, seed=m + 7 * n + k)
-    two, _, _ = gemm_case(spfy, cuda, tdt, m, n, k, nb, ta, tb, 0.5, 0.25, False, nb > 1, prec | spfy.GEMM_CTA_PAIRS, True,
-                          seed=m + 7 * n + k)
-    assert np.array_equal(one, two)
+    got, want, bound = gemm_case(spfy, cuda, tdt, m, n, k, nb, ta, tb, 0.5, 0.25, False, nb > 1, prec, True, seed=m + 7 * n + k)
     tol = TF32_TOL if tdt == torch.float32 else 2.0 ** -7
-    assert np.all(np.abs(two - want) <= tol * bound + 1e-30)
+    assert np.all(np.abs(got - want) <= tol * bound + 1e-30)
+
+
+@pytest.mark.parametrize("tdt", [torch.float16, torch.bfloat16, torch.float32])
+@pytest.mark.parametrize("strided", [True, False])
+def test_gemm_refuses_unknown_precision(spfy, cuda, tdt, strided):
+    """precision is PRECISE or FAST for every dtype; anything else (0x10 once selected an opt-in kernel, 2 was read as
+    FAST for fp32 and ignored for 16-bit operands) is SPFY_E_INVALID with no launch and C untouched"""
+    m, n, k, nb = 200, 72, 104, 2
+    a = torch.rand(nb, k, m, device=cuda).to(tdt)
+    b = torch.rand(nb, n, k, device=cuda).to(tdt)
+    c = torch.rand(nb, n, m, device=cuda).to(tdt)
+    c0 = c.clone()
+    torch.cuda.synchronize()
+    for prec in (0x10, 2, spfy.GEMM_FAST | 0x10, -1):
+        before = spfy.launch_count()
+        with pytest.raises(spfy.SpfyError) as e:
+            spfy.batched.gemm(a, b, c, m, n, k, beta=0.5, precision=prec, strided=strided)
+        assert e.value.code == spfy.capi.E_INVALID and "precision" in str(e.value)
+        assert spfy.launch_count() == before
+    torch.cuda.synchronize()
+    assert torch.equal(c.view(torch.int8), c0.view(torch.int8))
 
 
 @pytest.mark.parametrize("strided", [True, False])

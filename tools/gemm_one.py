@@ -25,4 +25,4 @@ for _ in range(reps):
 e1.record()
 torch.cuda.synchronize()
 print(f"gemm {m}x{n}x{k} nb={nb}: {e0.elapsed_time(e1) / reps * 1e3:.1f} us "
-      f"(stages={os.environ.get('SPFY_GEMM_STAGES', '-')}, no_pairs={os.environ.get('SPFY_GEMM_NO_PAIRS', '-')})")
+      f"(stages={os.environ.get('SPFY_GEMM_STAGES', '-')})")

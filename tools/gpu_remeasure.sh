@@ -1,13 +1,8 @@
 #!/bin/bash
-# per-call (event pair per call) timings: dense GEMM beside cuBLAS with and without CTA pairs, COO SpMM table
+# per-call (event pair per call) timings: dense GEMM beside cuBLAS, COO SpMM table
 T=${1:-rm}; O=gpurun_out; mkdir -p $O
 export SPFY_LIB=$PWD/sparsify.me_b200/lib_dev/libsparsifyme_b200.so
-for sw in 1 0; do
-  if [ $sw = 1 ]; then export SPFY_GEMM_NO_PAIRS=1; else unset SPFY_GEMM_NO_PAIRS; fi
-  echo "== NO_PAIRS=$sw" >> $O/${T}_gemm.log
-  timeout 300 python tools/gemm_probe.py --time --dtype f16 >> $O/${T}_gemm.log 2>&1
-done
-unset SPFY_GEMM_NO_PAIRS
+timeout 300 python tools/gemm_probe.py --time --dtype f16 >> $O/${T}_gemm.log 2>&1
 timeout 300 python tools/gemm_probe.py --time --dtype f32 >> $O/${T}_gemm.log 2>&1
 cat $O/${T}_gemm.log
 unset SPFY_LIB
