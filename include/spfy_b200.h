@@ -312,6 +312,28 @@ SPFY_API int spfy_spmma_conv_ex(int dtype, const spfy_conv_desc* conv, size_t m,
  * dimension, a filter larger than the padded image, null or not 16-byte aligned buffers (SPFY_E_INVALID). */
 SPFY_API int spfy_spmma_conv_dgrad(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* vals_t,
                                    const void* meta_t, const void* dY, float beta, void* dX, spfy_stream_t stream);
+/* spfy_conv_wgrad24 -- the weight gradient of a 2:4 convolution, fp32, masked to the layer's pattern:
+ *     dW = alpha * mask(conv2d_weight(X, dY)) + beta * dW
+ * conv: the FORWARD layer.  X: NHWC [batch][h][w][c] (F16/BF16); dY: NHWC [batch][ho][wo][m], same dtype.  meta: SM100
+ * metadata of the layer's compressed m x (kh*kw*c) filter in (kh, kw, c) order (spfy_permute_conv_weights, then
+ * spfy_prune24).  dW: fp32 [m][kh*kw*c] row-major in (kh, kw, c) order -- the storage of a channels_last [m][c][kh][kw]
+ * weight.  Positions the metadata prunes are written +0 whatever alpha, beta and dW held; dW is not read when beta = 0.
+ * The contraction runs on tcgen05 (kind::f16, fp32 accumulators) with M = kh*kw*c, N = m and K = P = batch*ho*wo output
+ * positions, K split into S ranges of k_tiles stages of 64 positions; each split writes an fp32 partial to the
+ * workspace, and a second pass sums the partials in ascending split order, applies alpha, beta and the mask.  No atomics:
+ * the same inputs give the same bits.  S depends on the shape alone:
+ *     tiles   = ceil(kh*kw*c / 128) * ceil(m / 256),   stages = ceil(P / 64)
+ *     S0      = max(1, min(floor(148 / tiles), floor(stages / 8)))
+ *     k_tiles = ceil(stages / S0),   S = ceil(stages / k_tiles)
+ * (one wave of units on the 148 SMs of a B200, at least 8 stages a unit), and the workspace is S * m * kh*kw*c * 4 bytes;
+ * the query needs no device.  Two launches, no device allocation, no sync.  Refusals, before any launch: dtype not
+ * F16/BF16, c % 64, m % 8, kh or kw > 16, pad > 8, stride > 8 (SPFY_E_UNSUPPORTED); an empty dimension, a filter larger
+ * than the padded image, null or not 16-byte aligned buffers (SPFY_E_INVALID); a workspace smaller than the query
+ * (SPFY_E_WORKSPACE). */
+SPFY_API int spfy_conv_wgrad24_workspace_bytes(int dtype, const spfy_conv_desc* conv, size_t m, size_t* bytes);
+SPFY_API int spfy_conv_wgrad24(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* X,
+                               const void* dY, const void* meta, float beta, float* dW,
+                               void* workspace, size_t workspace_bytes, spfy_stream_t stream);
 /* weights [m][c * kh * kw] in (c, kh, kw) column order (what torch's unfold / a flattened conv weight uses)
  * -> [m][kh * kw * c] in (kh, kw, c) order; 16-bit elements */
 SPFY_API int spfy_permute_conv_weights(const void* in, void* out, size_t m, size_t c, size_t kh, size_t kw,

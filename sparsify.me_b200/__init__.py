@@ -27,12 +27,12 @@ from .ops import (sparsify, prune24, prune24_check, compressed_bytes, spmma_comp
                   threshold_to_coo, coo_to_csr, batched, Compressed24, SpmmaPlan, prune24_batched,
                   alloc_compressed, pack_compressed, unpack_compressed, spmma_conv, spmma_conv_nhwc, permute_conv_weights,
                   Epilogue, fold_batchnorm, transpose24, recompress24, Linear24,
-                  Transpose24Conv, transpose24_conv, spmma_conv_dgrad_nhwc)
+                  Transpose24Conv, transpose24_conv, spmma_conv_dgrad_nhwc, conv_wgrad24_nhwc, Conv2d24)
 from . import shapes  # noqa: F401
 from . import multigpu  # noqa: F401
 
 __all__ = [
     "capi", "sparsify", "prune24", "prune24_check", "compressed_bytes", "spmma_compressed", "spmma",
-    "threshold_to_coo", "coo_to_csr", "batched", "Compressed24", "SpmmaPlan", "prune24_batched", "alloc_compressed", "Epilogue", "fold_batchnorm", "transpose24", "recompress24", "Linear24", "Transpose24Conv", "transpose24_conv", "spmma_conv_dgrad_nhwc", "pack_compressed", "unpack_compressed", "shapes", "multigpu", "SpfyError",
+    "threshold_to_coo", "coo_to_csr", "batched", "Compressed24", "SpmmaPlan", "prune24_batched", "alloc_compressed", "Epilogue", "fold_batchnorm", "transpose24", "recompress24", "Linear24", "Transpose24Conv", "transpose24_conv", "spmma_conv_dgrad_nhwc", "conv_wgrad24_nhwc", "Conv2d24", "pack_compressed", "unpack_compressed", "shapes", "multigpu", "SpfyError",
     "launch_count", "last_error", "version",
 ]

@@ -64,6 +64,8 @@ SIGNATURES = {
                               _P, _SZ, _P, _SZ, _P, _P]),
     "spfy_spmma_conv_ex": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _SZ, _P, _SZ, c_int, _P, _P]),
     "spfy_spmma_conv_dgrad": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _P]),
+    "spfy_conv_wgrad24_workspace_bytes": (c_int, [c_int, _P, _SZ, POINTER(_SZ)]),
+    "spfy_conv_wgrad24": (c_int, [c_int, _P, _SZ, c_float, _P, _P, _P, c_float, _P, _P, _SZ, _P]),
     "spfy_permute_conv_weights": (c_int, [_P, _P, _SZ, _SZ, _SZ, _SZ, _P]),
     "spfy_spmma_plan_create": (c_int, [c_int, _P, _SZ, POINTER(c_void_p)]),
     "spfy_spmma_plan_create_replicated": (c_int, [c_int, _P, _SZ, _SZ, _P, POINTER(c_void_p)]),

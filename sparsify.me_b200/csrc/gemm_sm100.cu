@@ -5,7 +5,8 @@
 //     sparsifyme::batched::gemm          cublas{H,S}gemmBatched          include/sparsify.me/gemm.hxx:25-195
 //     sparsifyme::batched::strided_coo   cusparseSpMM COO_ALG4           include/sparsify.me/spmm.hxx:140-193
 //     sparsifyme::batched::spmm          cusparseSpMM blocked-ELL        include/sparsify.me/spmm.hxx:30-138
-// (the two SpMM entries scatter / expand their sparse operand into a dense one first, spmm.cu).
+// (the two SpMM entries scatter / expand their sparse operand into a dense one first, spmm.cu), and, as a mode of
+// tcgemm_kernel, the split-K weight gradient of a 2:4 convolution (spfy_conv_wgrad24, at the end of the file).
 //
 // The kernel works in "UMMA terms": D[Mu x Nu] = Au[Mu x K] * Bu[Nu x K]^T with fp32 accumulators in TMEM.  Each
 // operand may be K-major (K contiguous) or MN-major (its Mu / Nu dimension contiguous); the result is written
@@ -88,6 +89,12 @@ struct GemmLaunch {
   uint32_t a_stages;  // 3xTF32 kernel: depth of the Au ring (raw tiles only; the Bu ring has `stages` slots)
   uint32_t acc_slots, d_cols;  // 3xTF32 kernel: accumulator slots (2 x TS_G x 64 columns, or 1 x TS_G x 128)
   uint32_t b_off;     // ... and where the Bu ring starts
+  // weight-gradient mode of tcgemm_kernel (spfy_conv_wgrad24): the convolution behind the im2col map tmap_a
+  struct {
+    uint32_t c, kw, wo, ho, stride;
+    int off_h, off_w;    // base pixel of output position (0, 0): -pad
+    uint32_t dn, dh, dw; // one stage = 64 output positions = dn images + dh rows + dw columns
+  } wg;
 };
 
 // Units are numbered (batch, m-group, n-tile) with the n-tile fastest.  The walker keeps that position incrementally --
@@ -243,7 +250,63 @@ __device__ __forceinline__ void gemm_epilogue(GemmWalker& W, uint32_t tmem_base,
   }
 }
 
-template <int KIND>
+// Producer of tcgemm_kernel's weight-gradient mode (one problem; the unit's batch digit is its split of K)
+__device__ __forceinline__ void wgrad_producer(GemmWalker& W, const GemmLaunch& L, uint32_t smem_base, uint32_t bar_full,
+                                               uint32_t bar_empty) {
+  const uint32_t NS = L.stages;
+  const bool leader = elect_one();
+  uint32_t stage = 0, phase = 0;
+  const GemmProblemDev* P = W.current();  // (one problem)
+  if (leader) { prefetch_tmap(&P->tmap_a); prefetch_tmap(&P->tmap_b); }
+  const uint32_t mu = uni(P->mu), k_tiles = uni(P->k_tiles), bn = uni(P->bn);
+  const uint32_t cc = L.wg.c, kw = L.wg.kw, wo = L.wg.wo, ho = L.wg.ho, str = L.wg.stride;
+  const uint32_t dn = L.wg.dn, dh = L.wg.dh, dw = L.wg.dw;
+  const int off_h = L.wg.off_h, off_w = L.wg.off_w;
+  constexpr uint32_t GROUP_BYTES = 64u * GM_ROW_BYTES;  // one MN group: 64 k-rows (positions) x 64 elements
+  for (; W.valid(); W.next()) {
+    const uint32_t nt = W.nt, mt = W.md, s = W.bb;
+    // the tile's 64-row groups of Mu (mu is a multiple of 64): filter tap and channel offset of each (per unit, so
+    // the divisions stay out of the stage loop)
+    const uint32_t r0 = mt * (uint32_t)GM_BM, groups = min(2u, (mu - r0) / 64u);
+    const uint32_t tap0 = r0 / cc, c0 = r0 - tap0 * cc;
+    const uint32_t tap1 = c0 + 64u == cc ? tap0 + 1u : tap0, c1 = c0 + 64u == cc ? 0u : c0 + 64u;
+    const uint16_t th0 = (uint16_t)(tap0 / kw), tw0 = (uint16_t)(tap0 - th0 * kw);
+    const uint16_t th1 = (uint16_t)(tap1 / kw), tw1 = (uint16_t)(tap1 - th1 * kw);
+    // output position of the unit's first stage as (image, row, column), then stepped by 64 positions per stage
+    const uint32_t p0 = s * k_tiles * 64u, row = p0 / wo;
+    uint32_t w = p0 - row * wo, n = row / ho, h = row - n * ho;
+    const uint32_t tx = groups * GROUP_BYTES + bn * (uint32_t)GM_ROW_BYTES;
+    for (uint32_t kt = 0; kt < k_tiles; ++kt) {
+      mbar_wait(bar_empty + stage * 8, phase ^ 1u);
+      const uint32_t full = bar_full + stage * 8;
+      const uint32_t sa = smem_base + stage * L.stage_bytes, sb = sa + GM_A_BYTES;
+      if (leader) {
+        mbar_expect_tx(full, tx);
+        const int cw = (int)(w * str) + off_w, ch = (int)(h * str) + off_h;
+        tma_load_im2col_4d(sa, &P->tmap_a, (int)c0, cw, ch, (int)n, tw0, th0, full, HINT_EVICT_NORMAL);
+        if (groups > 1u)
+          tma_load_im2col_4d(sa + GROUP_BYTES, &P->tmap_a, (int)c1, cw, ch, (int)n, tw1, th1, full, HINT_EVICT_NORMAL);
+        for (uint32_t g = 0; g * 64u < bn; ++g)
+          tma_load_3d(sb + g * GROUP_BYTES, &P->tmap_b, (int)(nt * bn + g * 64u), (int)(p0 + kt * 64u), 0, full,
+                      HINT_EVICT_NORMAL);
+      }
+      w += dw;
+      if (w >= wo) { w -= wo; ++h; }
+      h += dh;
+      if (h >= ho) { h -= ho; ++n; }
+      n += dn;
+      if (++stage == NS) { stage = 0; phase ^= 1u; }
+    }
+  }
+}
+
+// WGRAD: the weight gradient of a convolution (spfy_conv_wgrad24), a mode that differs from the GEMM in the producer and
+// in what the epilogue writes.  Au = im2col(X) (Mu = kh*kw*c in (kh, kw, c) order, MN-major: each 64-row group of a
+// tile is one im2col load of 64 output positions x 64 channels at one filter tap), Bu = dY as {m, positions}
+// (MN-major), K = output positions.  The batch digit of a unit is its split s of K: k_tiles stages from position
+// s * k_tiles * 64 on (the last split runs past the end into zero fill), and the epilogue writes the fp32 partial tile to
+// slab s of the workspace (alpha 1, beta 0).  The MMA issuer is the GEMM's.
+template <int KIND, bool WGRAD = false>
 __global__ void __launch_bounds__(GM_THREADS, 1)
 tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_constant__ GemmLaunch L) {
   using out_t = typename OutT<KIND>::type;
@@ -282,50 +345,54 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
   GemmWalker W(&single, L);
 
   if (warp == 0) {
-    // ===================== producer =====================
-    const bool leader = elect_one();
-    uint32_t stage = 0, phase = 0;
-    const GemmProblemDev* last = nullptr;
-    const CUtensorMap *tmap_a = nullptr, *tmap_b = nullptr;
-    uint32_t m_tiles = 1, n_tiles = 1, k_tiles = 0, bn = 0, a_mn = 0, b_mn = 0, a_bat = 0, b_bat = 0, unit_begin = 0;
-    const uint32_t kel = L.kelems;                      // K elements per stage == k rows of an MN-major slab
-    const uint32_t gsz = kel;                           // MN elements per 128-byte group (32 fp32 / 64 half)
-    const uint32_t group_bytes = kel * GM_ROW_BYTES;    // one MN group: kel k-rows x 128 bytes
-    for (; W.valid(); W.next()) {
-      const GemmProblemDev* P = W.current();
-      if (P != last) {
-        last = P;
-        tmap_a = &P->tmap_a; tmap_b = &P->tmap_b;
-        if (leader) { prefetch_tmap(tmap_a); prefetch_tmap(tmap_b); }
-        m_tiles = uni(P->m_tiles); n_tiles = uni(P->n_tiles); k_tiles = uni(P->k_tiles); bn = uni(P->bn);
-        a_mn = uni(P->a_mn); b_mn = uni(P->b_mn); a_bat = uni(P->a_batched); b_bat = uni(P->b_batched);
-        unit_begin = uni(P->unit_begin);
-      }
-      const uint32_t nt = W.nt, mt = W.md, b = W.bb;  // (one m-tile per unit in this kernel: m-group = m-tile)
-      const int ba = a_bat ? (int)b : 0, bb = b_bat ? (int)b : 0;
-      const uint32_t tx = (uint32_t)GM_A_BYTES + bn * (uint32_t)GM_ROW_BYTES;
-      for (uint32_t kt = 0; kt < k_tiles; ++kt) {
-        mbar_wait(bar_empty + stage * 8, phase ^ 1u);
-        const uint32_t full = bar_full + stage * 8;
-        const uint32_t sa = smem_base + stage * L.stage_bytes, sb = sa + GM_A_BYTES;
-        if (leader) {
-          mbar_expect_tx(full, tx);
-          if (!a_mn) {
-            tma_load_3d(sa, tmap_a, (int)(kt * kel), (int)(mt * GM_BM), ba, full, HINT_EVICT_NORMAL);
-          } else {
-            for (uint32_t g = 0; g * gsz < (uint32_t)GM_BM; ++g)
-              tma_load_3d(sa + g * group_bytes, tmap_a, (int)(mt * GM_BM + g * gsz), (int)(kt * kel), ba, full,
-                          HINT_EVICT_NORMAL);
-          }
-          if (!b_mn) {
-            tma_load_3d(sb, tmap_b, (int)(kt * kel), (int)(nt * bn), bb, full, HINT_EVICT_NORMAL);
-          } else {
-            for (uint32_t g = 0; g * gsz < bn; ++g)
-              tma_load_3d(sb + g * group_bytes, tmap_b, (int)(nt * bn + g * gsz), (int)(kt * kel), bb, full,
-                          HINT_EVICT_NORMAL);
-          }
+    if constexpr (WGRAD) {
+      wgrad_producer(W, L, smem_base, bar_full, bar_empty);
+    } else {
+      // ===================== producer =====================
+      const bool leader = elect_one();
+      uint32_t stage = 0, phase = 0;
+      const GemmProblemDev* last = nullptr;
+      const CUtensorMap *tmap_a = nullptr, *tmap_b = nullptr;
+      uint32_t m_tiles = 1, n_tiles = 1, k_tiles = 0, bn = 0, a_mn = 0, b_mn = 0, a_bat = 0, b_bat = 0, unit_begin = 0;
+      const uint32_t kel = L.kelems;                      // K elements per stage == k rows of an MN-major slab
+      const uint32_t gsz = kel;                           // MN elements per 128-byte group (32 fp32 / 64 half)
+      const uint32_t group_bytes = kel * GM_ROW_BYTES;    // one MN group: kel k-rows x 128 bytes
+      for (; W.valid(); W.next()) {
+        const GemmProblemDev* P = W.current();
+        if (P != last) {
+          last = P;
+          tmap_a = &P->tmap_a; tmap_b = &P->tmap_b;
+          if (leader) { prefetch_tmap(tmap_a); prefetch_tmap(tmap_b); }
+          m_tiles = uni(P->m_tiles); n_tiles = uni(P->n_tiles); k_tiles = uni(P->k_tiles); bn = uni(P->bn);
+          a_mn = uni(P->a_mn); b_mn = uni(P->b_mn); a_bat = uni(P->a_batched); b_bat = uni(P->b_batched);
+          unit_begin = uni(P->unit_begin);
         }
-        if (++stage == NS) { stage = 0; phase ^= 1u; }
+        const uint32_t nt = W.nt, mt = W.md, b = W.bb;  // (one m-tile per unit in this kernel: m-group = m-tile)
+        const int ba = a_bat ? (int)b : 0, bb = b_bat ? (int)b : 0;
+        const uint32_t tx = (uint32_t)GM_A_BYTES + bn * (uint32_t)GM_ROW_BYTES;
+        for (uint32_t kt = 0; kt < k_tiles; ++kt) {
+          mbar_wait(bar_empty + stage * 8, phase ^ 1u);
+          const uint32_t full = bar_full + stage * 8;
+          const uint32_t sa = smem_base + stage * L.stage_bytes, sb = sa + GM_A_BYTES;
+          if (leader) {
+            mbar_expect_tx(full, tx);
+            if (!a_mn) {
+              tma_load_3d(sa, tmap_a, (int)(kt * kel), (int)(mt * GM_BM), ba, full, HINT_EVICT_NORMAL);
+            } else {
+              for (uint32_t g = 0; g * gsz < (uint32_t)GM_BM; ++g)
+                tma_load_3d(sa + g * group_bytes, tmap_a, (int)(mt * GM_BM + g * gsz), (int)(kt * kel), ba, full,
+                            HINT_EVICT_NORMAL);
+            }
+            if (!b_mn) {
+              tma_load_3d(sb, tmap_b, (int)(kt * kel), (int)(nt * bn), bb, full, HINT_EVICT_NORMAL);
+            } else {
+              for (uint32_t g = 0; g * gsz < bn; ++g)
+                tma_load_3d(sb + g * group_bytes, tmap_b, (int)(nt * bn + g * gsz), (int)(kt * kel), bb, full,
+                            HINT_EVICT_NORMAL);
+            }
+          }
+          if (++stage == NS) { stage = 0; phase ^= 1u; }
+        }
       }
     }
   } else if (warp == 1) {
@@ -385,7 +452,8 @@ tcgemm_kernel(const __grid_constant__ GemmProblemDev single, const __grid_consta
       ++job;
     }
   } else {
-    gemm_epilogue<KIND>(W, tmem_base, bar_acc_full, bar_acc_empty, GM_ACC_SLOTS, GM_MAX_BN, GM_MAX_BN, warp, lane);
+    gemm_epilogue<WGRAD ? KIND_F32 : KIND>(W, tmem_base, bar_acc_full, bar_acc_empty, GM_ACC_SLOTS, GM_MAX_BN, GM_MAX_BN, warp,
+                                           lane);
   }
 
   tc_fence_before();
@@ -753,6 +821,33 @@ repack_kernel(const T* __restrict__ src, size_t ld, size_t stride, T* __restrict
   }
 }
 
+// dW = alpha * (sum of the S slabs in ascending s) + beta * dW where the metadata keeps the element, +0 where it prunes it
+// (dW is not read when beta == 0).  One thread = one 2:4 group: 4 columns, one metadata nibble, one 16-byte store.
+__global__ void __launch_bounds__(256)
+wgrad24_reduce_kernel(const float4* __restrict__ part, uint32_t splits, size_t groups, uint32_t kq, const uint8_t* __restrict__ meta,
+                      uint32_t meta_m_tiles, float alpha, float beta, float4* dw) {
+  const size_t nthreads = (size_t)gridDim.x * blockDim.x;
+  for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < groups; t += nthreads) {
+    float4 v = part[t];
+    for (uint32_t s = 1; s < splits; ++s) {
+      const float4 p = part[(size_t)s * groups + t];
+      v.x += p.x; v.y += p.y; v.z += p.z; v.w += p.w;
+    }
+    const size_t r = t / kq;
+    const uint32_t row = (uint32_t)r, col = (uint32_t)(t - r * kq) * 4u;
+    const size_t st = (size_t)(col >> 7) * meta_m_tiles + (row >> 7);  // storage index of the metadata tile
+    const uint32_t word = *reinterpret_cast<const uint16_t*>(meta + st * 2048 + sm100_meta_word(row & 127u, (col & 127u) >> 4));
+    const uint32_t nib = word >> (4u * ((col >> 2) & 3u));
+    const uint32_t keep = (1u << (nib & 3u)) | (1u << ((nib >> 2) & 3u));
+    float4 o = make_float4(alpha * v.x, alpha * v.y, alpha * v.z, alpha * v.w);
+    if (beta != 0.f) {
+      const float4 d = dw[t];
+      o.x += beta * d.x; o.y += beta * d.y; o.z += beta * d.z; o.w += beta * d.w;
+    }
+    dw[t] = make_float4(keep & 1u ? o.x : 0.f, keep & 2u ? o.y : 0.f, keep & 4u ? o.z : 0.f, keep & 8u ? o.w : 0.f);
+  }
+}
+
 // ------------------------------------------------------------------------------------------ host side
 size_t elem_bytes(int dtype) { return dtype == SPFY_F32 ? 4 : 2; }
 
@@ -961,6 +1056,9 @@ void warm_gemm_kernels() {
   touch_kernel(tcgemm_kernel<KIND_F16>);
   touch_kernel(tcgemm_kernel<KIND_BF16>);
   touch_kernel(tcgemm_kernel<KIND_F32>);
+  touch_kernel(tcgemm_kernel<KIND_F16, true>);
+  touch_kernel(tcgemm_kernel<KIND_BF16, true>);
+  touch_kernel(wgrad24_reduce_kernel);
 }
 
 int tc_gemm_supported(int dtype, const TcGemmProblem& p, bool allow_repack) {
@@ -1140,6 +1238,140 @@ int tc_gemm_run(int dtype, int precision, const TcGemmProblem* problems, size_t 
   return launch_kind<KIND_F16>(table[0], L, smem, grid, stream);
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// Weight gradient of a 2:4 convolution (spfy_conv_wgrad24): tcgemm_kernel<KIND, true> writes S fp32 partial sums of
+// dW = dY^T im2col(X) to the workspace, one per split of the output positions, and wgrad24_reduce_kernel adds them up.
+// ------------------------------------------------------------------------------------------------------------
+namespace {
+
+// The split count targets one wave of units on the 148 SMs of a B200 with at least WG_MIN_STAGES stages (64 output
+// positions each) per unit.  It is a constant of the shape, not of the device, so that the workspace query needs no
+// device and a shape always sums in the same order.
+constexpr size_t WG_SMS = 148;
+constexpr size_t WG_MIN_STAGES = 8;
+
+struct WgradShape {
+  size_t ho, wo, positions, kk;  // kk = kh * kw * c
+  uint32_t m_tiles, n_tiles, bn, k_tiles, splits;  // m-tiles along kk, n-tiles along m, stages per split, S
+};
+
+int wgrad_shape(int dtype, const spfy_conv_desc* conv, size_t m, WgradShape* out) {
+  const char* who = "conv_wgrad24";
+  if (dtype != SPFY_F16 && dtype != SPFY_BF16) return fail(SPFY_E_UNSUPPORTED, "%s: dtype %d (need F16/BF16)", who, dtype);
+  if (!conv) return fail(SPFY_E_INVALID, "%s: null descriptor", who);
+  const spfy_conv_desc& c = *conv;
+  if (!c.batch || !c.h || !c.w || !c.c || !c.kh || !c.kw || !c.stride || !m)
+    return fail(SPFY_E_INVALID, "%s: empty dimension", who);
+  if (c.c % 64) return fail(SPFY_E_UNSUPPORTED, "%s: channels must be a multiple of 64 (got %zu)", who, c.c);
+  if (m % 8) return fail(SPFY_E_UNSUPPORTED, "%s: m (the channels of dY) must be a multiple of 8 (got %zu)", who, m);
+  if (c.kh > 16 || c.kw > 16 || c.pad > 8 || c.stride > 8)
+    return fail(SPFY_E_UNSUPPORTED, "%s: filter / padding / stride outside what the im2col tensor map encodes", who);
+  if (c.h + 2 * c.pad < c.kh || c.w + 2 * c.pad < c.kw) return fail(SPFY_E_INVALID, "%s: filter larger than the padded image", who);
+  WgradShape s;
+  s.ho = (c.h + 2 * c.pad - c.kh) / c.stride + 1;
+  s.wo = (c.w + 2 * c.pad - c.kw) / c.stride + 1;
+  s.positions = c.batch * s.ho * s.wo;
+  s.kk = c.kh * c.kw * c.c;
+  if (s.positions >= (1ull << 31) || m >= (1ull << 20) || c.c >= (1ull << 20) || c.batch * c.h * c.w >= (1ull << 31) ||
+      m * s.kk >= (1ull << 31))
+    return fail(SPFY_E_UNSUPPORTED, "%s: dimension too large", who);
+  split_nu(m, 64, GM_MAX_BN, &s.bn, &s.n_tiles);
+  s.m_tiles = (uint32_t)ceil_div(s.kk, GM_BM);
+  const size_t stages = ceil_div(s.positions, 64), tiles = (size_t)s.m_tiles * s.n_tiles;
+  const size_t s0 = std::max<size_t>(1, std::min(WG_SMS / tiles, stages / WG_MIN_STAGES));
+  s.k_tiles = (uint32_t)ceil_div(stages, s0);
+  s.splits = (uint32_t)ceil_div(stages, s.k_tiles);
+  *out = s;
+  return SPFY_OK;
+}
+
+size_t wgrad_workspace(const WgradShape& s, size_t m) { return (size_t)s.splits * m * s.kk * sizeof(float); }
+
+}  // namespace
+
+int conv_wgrad24_run(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* X, const void* dY,
+                     const void* meta, float beta, float* dW, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  const char* who = "conv_wgrad24";
+  WgradShape s;
+  int rc = wgrad_shape(dtype, conv, m, &s);
+  if (rc) return rc;
+  if (!X || !dY || !meta || !dW || !ws) return fail(SPFY_E_INVALID, "%s: null buffer", who);
+  if ((uintptr_t)X % 16 || (uintptr_t)dY % 16 || (uintptr_t)meta % 16 || (uintptr_t)dW % 16 || (uintptr_t)ws % 16)
+    return fail(SPFY_E_INVALID, "%s: buffers must be 16-byte aligned", who);
+  const size_t need = wgrad_workspace(s, m);
+  if (ws_bytes < need) return fail(SPFY_E_WORKSPACE, "%s: workspace %zu < %zu bytes", who, ws_bytes, need);
+  DeviceInfo di;
+  rc = require_sm100(who, &di);
+  if (rc) return rc;
+  const spfy_conv_desc& c = *conv;
+
+  GemmProblemDev d;
+  memset(&d, 0, sizeof(d));
+  rc = make_tmap_im2col(&d.tmap_a, dtype, X, im2col_of(c), 64);
+  if (rc) return rc;
+  rc = make_operand_map(&d.tmap_b, dtype, OperandView{dY, m, s.positions, m, 0, true}, 1, s.bn, CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc) return rc;
+  d.C = (uint8_t*)ws;
+  d.ldc = s.kk;
+  d.stride_c = m * s.kk;
+  d.mu = (uint32_t)s.kk;
+  d.nu = (uint32_t)m;
+  d.k = s.k_tiles * 64u;
+  d.nb = s.splits;
+  d.m_tiles = s.m_tiles;
+  d.n_tiles = s.n_tiles;
+  d.k_tiles = s.k_tiles;
+  d.g = 1;
+  d.m_groups = s.m_tiles;
+  d.bn = s.bn;
+  d.a_mn = d.b_mn = 1;
+  d.out_mu_contig = 1;
+  d.units = s.m_tiles * s.n_tiles * s.splits;
+  d.alpha = 1.f;
+
+  GemmLaunch L;
+  memset(&L, 0, sizeof(L));
+  L.kelems = 64;
+  L.stage_bytes = (uint32_t)GM_A_BYTES + s.bn * (uint32_t)GM_ROW_BYTES;
+  L.stages = std::min<uint32_t>((GM_SMEM_LIMIT - 1024u - GM_BAR_BYTES) / L.stage_bytes, GM_MAX_STAGES);
+  L.bar_off = L.stages * L.stage_bytes;
+  const uint32_t smem = L.bar_off + GM_BAR_BYTES + 1024u;
+  const uint32_t fmt = dtype == SPFY_BF16 ? 1u : 0u;
+  L.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(GM_BM >> 4) << 24);
+  L.num_problems = 1;
+  L.total_units = d.units;
+  L.wg.c = (uint32_t)c.c;
+  L.wg.kw = (uint32_t)c.kw;
+  L.wg.wo = (uint32_t)s.wo;
+  L.wg.ho = (uint32_t)s.ho;
+  L.wg.stride = (uint32_t)c.stride;
+  L.wg.off_h = L.wg.off_w = -(int)c.pad;
+  const size_t img = s.ho * s.wo;
+  L.wg.dn = (uint32_t)(64 / img);
+  L.wg.dh = (uint32_t)(64 % img / s.wo);
+  L.wg.dw = (uint32_t)(64 % img % s.wo);
+
+  const int grid = (int)std::min<uint32_t>(d.units, (uint32_t)di.sm_count);
+  const size_t groups = m * s.kk / 4;
+  int rgrid = 1;
+  rc = capped_grid(ceil_div(groups, 256), 8, &rgrid);
+  if (rc) return rc;
+  if (dtype == SPFY_BF16) {
+    rc = allow_dynamic_smem<tcgemm_kernel<KIND_BF16, true>>(GM_SMEM_LIMIT);
+    if (rc) return rc;
+    tcgemm_kernel<KIND_BF16, true><<<grid, GM_THREADS, smem, stream>>>(d, L);
+  } else {
+    rc = allow_dynamic_smem<tcgemm_kernel<KIND_F16, true>>(GM_SMEM_LIMIT);
+    if (rc) return rc;
+    tcgemm_kernel<KIND_F16, true><<<grid, GM_THREADS, smem, stream>>>(d, L);
+  }
+  SPFY_LAUNCH_OK("tcgemm_kernel (weight gradient)");
+  wgrad24_reduce_kernel<<<rgrid, 256, 0, stream>>>((const float4*)ws, s.splits, groups, (uint32_t)(s.kk / 4), (const uint8_t*)meta,
+                                                   (uint32_t)ceil_div(m, 128), alpha, beta, (float4*)dW);
+  SPFY_LAUNCH_OK("wgrad24_reduce_kernel");
+  return SPFY_OK;
+}
+
 }  // namespace spfy
 
 using namespace spfy;
@@ -1192,6 +1424,19 @@ int spfy_gemm_batched(int dtype, int precision, int opA, int opB, size_t m, size
   for (size_t b = 0; b < num_batches; ++b)
     ps[b] = make_problem(opA, opB, m, n, k, alpha, A_ptrs[b], lda, 0, B_ptrs[b], ldb, 0, beta, C_ptrs[b], ldc, 0, 1);
   return tc_gemm_run(dtype, precision, ps.data(), ps.size(), workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int spfy_conv_wgrad24_workspace_bytes(int dtype, const spfy_conv_desc* conv, size_t m, size_t* bytes) {
+  WgradShape s;
+  const int rc = wgrad_shape(dtype, conv, m, &s);
+  if (rc) return rc;
+  if (bytes) *bytes = wgrad_workspace(s, m);
+  return SPFY_OK;
+}
+
+int spfy_conv_wgrad24(int dtype, const spfy_conv_desc* conv, size_t m, float alpha, const void* X, const void* dY,
+                      const void* meta, float beta, float* dW, void* workspace, size_t workspace_bytes, spfy_stream_t stream) {
+  return conv_wgrad24_run(dtype, conv, m, alpha, X, dY, meta, beta, dW, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -392,4 +392,44 @@ inline int encode_tiled(CUtensorMap* map, int dtype, uint32_t rank, const void* 
   return SPFY_OK;
 }
 
+// the im2col view of an implicit GEMM's B: NHWC [batch][h][w][c], a kh x kw window whose base pixels run over
+// [lo, dim + up) per spatial dimension with `stride` -- the ho x wo output positions of every image
+struct Im2col {
+  size_t batch, h, w, c, kh, kw, stride;
+  int lo_h, lo_w, up_h, up_w;
+  size_t ho, wo;
+};
+
+// a forward convolution: the bounding box is [-pad, dim + pad - (filter - 1))
+inline Im2col im2col_of(const spfy_conv_desc& c) {
+  const int p = (int)c.pad;
+  return Im2col{c.batch, c.h, c.w, c.c, c.kh, c.kw, c.stride, -p, -p, p - (int)(c.kh - 1), p - (int)(c.kw - 1),
+                (c.h + 2 * c.pad - c.kh) / c.stride + 1, (c.w + 2 * c.pad - c.kw) / c.stride + 1};
+}
+
+// NHWC activations {C, W, H, N} in im2col mode: one instruction gathers `pixels` consecutive output positions x 64
+// channels of one filter tap (128 B swizzle: position j is the 128-byte row j of the box).  The bounding box of base
+// pixels (Im2col), walked with the convolution stride, holds exactly the output positions, row by row, image by image.
+// (spmma_sm100.cu: 128 positions, the columns of a B stage; gemm_sm100.cu's weight gradient: 64, the k-rows of a stage.)
+inline int make_tmap_im2col(CUtensorMap* map, int dtype, const void* x, const Im2col& c, uint32_t pixels) {
+  EncodeIm2colFn enc;
+  int rc = get_im2col_encoder(&enc);
+  if (rc) return rc;
+  cuuint64_t dims[4] = {c.c, c.w, c.h, c.batch};
+  cuuint64_t strides[3] = {c.c * 2, c.w * c.c * 2, c.h * c.w * c.c * 2};
+  int lower[2] = {c.lo_w, c.lo_h};
+  int upper[2] = {c.up_w, c.up_h};
+  cuuint32_t estr[4] = {1, (cuuint32_t)c.stride, (cuuint32_t)c.stride, 1};
+  CUresult r = encode_with_context([&] {
+    return enc(map, dtype == SPFY_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4,
+               const_cast<void*>(x), dims, strides, lower, upper, /*channelsPerPixel*/ 64, /*pixelsPerColumn*/ pixels, estr,
+               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  });
+  if (r != CUDA_SUCCESS)
+    return fail(SPFY_E_CUDA, "cuTensorMapEncodeIm2col failed (%d) for NHWC %zu x %zu x %zu x %zu, filter %zu x %zu stride %zu, "
+                "corners (%d, %d) / (%d, %d)", (int)r, c.batch, c.h, c.w, c.c, c.kh, c.kw, c.stride, c.lo_h, c.lo_w, c.up_h, c.up_w);
+  return SPFY_OK;
+}
+
 }  // namespace spfy

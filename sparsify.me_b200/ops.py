@@ -354,24 +354,29 @@ class Transpose24Conv:
     phases: list
 
 
-def transpose24_conv(comp, kh, kw, stride, pad, invalid=None):
+def transpose24_conv(comp, kh, kw, stride, pad, invalid=None, out=None):
     """spfy_transpose24_conv: the operands of the data gradient of a stride-`stride`, pad-`pad` convolution whose filter
     `comp` is m x kh*kw*c in (kh, kw, c) order (permute_conv_weights, then prune24 with PRUNE_TILE_TRANSPOSABLE).  Phase
     (a, b) holds the dx pixels (s*i + a, s*j + b); its operand is the flipped, channel-swapped sub-filter of the taps
     that reach them.  For stride 1 the one operand is transpose24(comp, taps=kh*kw), byte for byte.
-    `invalid`: optional int32 CUDA tensor, 0, or 1 when the mask is not transposable.  Nothing here syncs.
-    Use it with spmma_conv_dgrad_nhwc."""
+    `invalid`: optional int32 CUDA tensor, 0, or 1 when the mask is not transposable.  `out`: a Transpose24Conv of the
+    same layer to refill in place (returned).  Nothing here syncs.  Use it with spmma_conv_dgrad_nhwc."""
     assert comp.layout == capi.LAYOUT_SM100
     if comp.cols % (kh * kw):
         raise capi.SpfyError(capi.E_INVALID, "transpose24_conv", f"cols {comp.cols} is not a multiple of kh*kw {kh * kw}")
     m, c = comp.rows, comp.cols // (kh * kw)
+    if invalid is not None:
+        assert invalid.dtype == torch.int32 and invalid.is_cuda
+    if out is not None:
+        assert (out.m, out.c, out.kh, out.kw, out.stride, out.pad, out.dtype) == (m, c, kh, kw, stride, pad, comp.dtype)
+        capi.spfy_transpose24_conv(_DT[comp.dtype], _ptr(comp.vals), _ptr(comp.meta), m, c, kh, kw, stride, pad,
+                                   _ptr(out.vals), _ptr(out.meta), _ptr(invalid), _stream())
+        return out
     vb, mb = ctypes.c_size_t(), ctypes.c_size_t()
     capi.spfy_transpose24_conv_bytes(_DT[comp.dtype], m, c, kh, kw, stride, pad, ctypes.byref(vb), ctypes.byref(mb))
     dev = comp.vals.device
     vals = torch.empty(vb.value, dtype=torch.uint8, device=dev)
     meta = torch.empty(mb.value, dtype=torch.uint8, device=dev)
-    if invalid is not None:
-        assert invalid.dtype == torch.int32 and invalid.is_cuda
     capi.spfy_transpose24_conv(_DT[comp.dtype], _ptr(comp.vals), _ptr(comp.meta), m, c, kh, kw, stride, pad,
                                _ptr(vals), _ptr(meta), _ptr(invalid), _stream())
     phases, tile = [], 0
@@ -416,6 +421,40 @@ def spmma_conv_dgrad_nhwc(op, dy, h, w, out=None, alpha=1.0, beta=0.0):
     desc = capi.ConvDesc(nb, h, w, op.c, op.kh, op.kw, s, p)
     capi.spfy_spmma_conv_dgrad(_DT[op.dtype], ctypes.byref(desc), op.m, float(alpha), _ptr(op.vals), _ptr(op.meta),
                                _ptr(dy), float(beta), _ptr(out), _stream())
+    return out
+
+
+def conv_wgrad24_nhwc(comp, x, dy, kh, kw, stride=1, pad=0, out=None, alpha=1.0, beta=0.0):
+    """spfy_conv_wgrad24: dW = alpha * mask(conv2d_weight(x, dy)) + beta * out, fp32, for the forward layer whose filter
+    `comp` is m x kh*kw*c in (kh, kw, c) order; the mask is comp's, and every position it prunes is +0.  x: NHWC
+    [batch, h, w, c]; dy: NHWC [batch, ho, wo, m], both in comp.dtype.  Returns dW (== out when given), fp32 in
+    (kh, kw, c) order: a new [m, kh*kw*c] tensor, or `out`, which may be [m, kh*kw*c] row-major or a channels_last
+    [m, c, kh, kw] weight (the same storage).  beta != 0 needs out; beta = 1 accumulates into it."""
+    assert comp.layout == capi.LAYOUT_SM100
+    assert x.dim() == 4 and x.is_contiguous() and dy.dim() == 4 and dy.is_contiguous()
+    nb, h, w, c = x.shape
+    m, kk = comp.rows, kh * kw * c
+    if x.dtype != comp.dtype or dy.dtype != comp.dtype:
+        raise TypeError(f"conv_wgrad24_nhwc: x {x.dtype} and dy {dy.dtype} must be the layer dtype {comp.dtype}")
+    ho, wo = (h + 2 * pad - kh) // stride + 1, (w + 2 * pad - kw) // stride + 1
+    if comp.cols != kk or tuple(dy.shape) != (nb, ho, wo, m):
+        raise capi.SpfyError(capi.E_INVALID, "conv_wgrad24", f"x {tuple(x.shape)}, dy {tuple(dy.shape)} do not match a "
+                             f"{kh}x{kw} stride {stride} pad {pad} layer with filter {m} x {comp.cols}")
+    if out is None:
+        if beta != 0.0:
+            raise capi.SpfyError(capi.E_INVALID, "conv_wgrad24", "beta != 0 needs out")
+        out = torch.empty(m, kk, dtype=torch.float32, device=x.device)
+    dense = (out.is_contiguous() and tuple(out.shape) == (m, kk)) or (
+        tuple(out.shape) == (m, c, kh, kw) and out.is_contiguous(memory_format=torch.channels_last))
+    if out.dtype != torch.float32 or not dense:
+        raise ValueError(f"conv_wgrad24_nhwc: out must be fp32, [{m}, {kk}] contiguous or [{m}, {c}, {kh}, {kw}] "
+                         f"channels_last; got {out.dtype} {tuple(out.shape)} strides {out.stride()}")
+    desc = capi.ConvDesc(nb, h, w, c, kh, kw, stride, pad)
+    wb = ctypes.c_size_t()
+    capi.spfy_conv_wgrad24_workspace_bytes(_DT[comp.dtype], ctypes.byref(desc), m, ctypes.byref(wb))
+    ws = _workspace(wb.value, x.device)
+    capi.spfy_conv_wgrad24(_DT[comp.dtype], ctypes.byref(desc), m, float(alpha), _ptr(x), _ptr(dy), _ptr(comp.meta),
+                           float(beta), _ptr(out), _ptr(ws), ws.numel(), _stream())
     return out
 
 
@@ -522,6 +561,105 @@ class Linear24(torch.nn.Module):
             raise TypeError(f"Linear24: input dtype {x2.dtype}, layer dtype {self.dtype}")
         y = _Linear24Fn.apply(x2, self.weight, self.bias, self)
         return y.view(*x.shape[:-1], self.comp.rows)
+
+
+class _Conv2d24Fn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, bias, layer):
+        del weight  # the forward operand is layer.comp; weight is an input so that its gradient reaches it
+        ctx.layer = layer
+        ctx.save_for_backward(x)
+        ctx.has_bias = bias is not None
+        y = spmma_conv_nhwc(layer.comp, x.permute(0, 2, 3, 1), layer.kh, layer.kw, layer.stride, layer.padding,
+                            epilogue=Epilogue(bias=bias.detach()) if bias is not None else None)
+        return y.permute(0, 3, 1, 2)  # [N, M, Ho, Wo], channels_last
+
+    @staticmethod
+    def backward(ctx, dy):
+        (x,) = ctx.saved_tensors
+        layer = ctx.layer
+        xh = x.permute(0, 2, 3, 1)
+        dyh = dy.to(layer.dtype).permute(0, 2, 3, 1).contiguous()  # no copy when dy is channels_last in the layer dtype
+        dx = dw = db = None
+        if ctx.needs_input_grad[0]:
+            dx = spmma_conv_dgrad_nhwc(layer.op_t, dyh, x.shape[2], x.shape[3]).permute(0, 3, 1, 2)
+        if ctx.needs_input_grad[1]:
+            dw = conv_wgrad24_nhwc(layer.comp, xh, dyh, layer.kh, layer.kw, layer.stride, layer.padding,
+                                   out=torch.empty_like(layer.weight, memory_format=torch.channels_last))
+        if ctx.has_bias and ctx.needs_input_grad[2]:
+            db = dyh.float().sum((0, 1, 2))
+        return dx, dw, db, None
+
+
+class Conv2d24(torch.nn.Module):
+    """A 2:4 convolution for fine-tuning with a fixed mask, the convolutional twin of Linear24: forward and both
+    gradients on tcgen05, activations channels_last.  The filter is pruned in (kh, kw, c) order with
+    PRUNE_TILE_TRANSPOSABLE, so that the data gradient's flipped filter is a 2:4 operand as well.
+    State: `weight`, the fp32 master [m, c, kh, kw] in torch.channels_last, kept masked -- its storage is the (kh, kw, c)
+    order of the operand, so optimizers work on it unchanged and dW is written straight into a tensor of its layout;
+    `bias` (fp32, optional); `comp`, the 16-bit compressed filter; `op_t`, the data gradient's phase operands.
+      forward : spmma_conv_nhwc(comp, x) with the bias in the epilogue; x is [N, c, H, W] in `dtype` and channels_last
+                with N * Ho * Wo a multiple of 8, the result [N, m, Ho, Wo] channels_last
+      backward: dx = spmma_conv_dgrad_nhwc(op_t, dy) (any stride); dW = conv_wgrad24_nhwc, fp32, masked; db = sum of dy
+    After optimizer.step(), call refresh(): it re-masks the master in place and refills comp and op_t from it (the mask
+    does not move).  forward refuses to run on a weight changed since the last refresh."""
+
+    def __init__(self, weight, bias, comp, op_t, dtype, stride, padding):
+        super().__init__()
+        self.weight = torch.nn.Parameter(weight)
+        self.bias = torch.nn.Parameter(bias) if bias is not None else None
+        self.comp, self.op_t, self.dtype = comp, op_t, dtype
+        self.m, self.c, self.kh, self.kw = weight.shape
+        self.stride, self.padding = stride, padding
+        self._synced_version = self.weight._version
+
+    @classmethod
+    def from_dense(cls, weight, bias=None, stride=1, padding=0, dtype=torch.float16, groups=1, dilation=1):
+        """Prune `weight` [m, c, kh, kw] (c a multiple of 64, m a multiple of 64) in `dtype`.  Raises ValueError for
+        groups or dilation other than 1, for c or m off those multiples, and when the pruned mask is not transposable
+        (one sync, here only)."""
+        m, c, kh, kw = weight.shape
+        if groups != 1 or dilation != 1:
+            raise ValueError("Conv2d24: grouped and dilated convolutions are not supported")
+        if c % 64 or m % 64:
+            raise ValueError(f"Conv2d24: in and out channels must be multiples of 64 (got c = {c}, m = {m})")
+        with torch.no_grad():
+            master = weight.detach().float().contiguous(memory_format=torch.channels_last).clone(
+                memory_format=torch.channels_last)
+            w2 = master.permute(0, 2, 3, 1).reshape(m, kh * kw * c)  # a view: the (kh, kw, c) storage
+            w16 = w2.to(dtype).contiguous()
+            comp = prune24(w16, inplace=True, mode=capi.PRUNE_TILE_TRANSPOSABLE)
+            recompress24(w2, comp, masked_out=w2, values=False)
+            invalid = torch.empty(1, dtype=torch.int32, device=weight.device)
+            op_t = transpose24_conv(comp, kh, kw, stride, padding, invalid=invalid)
+            if int(invalid.item()):
+                raise ValueError("Conv2d24: the pruned mask is not transposable")
+            b = bias.detach().float().contiguous().clone() if bias is not None else None
+        return cls(master, b, comp, op_t, dtype, stride, padding)
+
+    def _w2d(self):
+        """the master as the [m, kh*kw*c] matrix of its storage"""
+        if not self.weight.is_contiguous(memory_format=torch.channels_last):
+            raise RuntimeError("Conv2d24: the weight is no longer channels_last")
+        return self.weight.permute(0, 2, 3, 1).reshape(self.m, -1)
+
+    @torch.no_grad()
+    def refresh(self):
+        """master -> comp.vals (mask fixed), master re-masked in place, comp -> op_t (in place).  No sync."""
+        w2 = self._w2d()
+        recompress24(w2, self.comp, masked_out=w2)
+        transpose24_conv(self.comp, self.kh, self.kw, self.stride, self.padding, out=self.op_t)
+        self._synced_version = self.weight._version
+
+    def forward(self, x):
+        if self.weight._version != self._synced_version:
+            raise RuntimeError("Conv2d24: weight changed since the last refresh(); call refresh() after optimizer.step()")
+        if x.dtype != self.dtype:
+            raise TypeError(f"Conv2d24: input dtype {x.dtype}, layer dtype {self.dtype}: convert with x.to({self.dtype})")
+        if x.dim() != 4 or not x.is_contiguous(memory_format=torch.channels_last):
+            raise ValueError("Conv2d24: the input must be a 4-D channels_last tensor: convert with "
+                             "x.contiguous(memory_format=torch.channels_last)")
+        return _Conv2d24Fn.apply(x, self.weight, self.bias, self)
 
 
 # ----------------------------------------------------------------------------- A4
