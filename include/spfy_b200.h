@@ -224,6 +224,76 @@ SPFY_API int spfy_transpose24_conv(int dtype, const void* vals, const void* meta
  * onto the mask, or re-masks the master in place. */
 SPFY_API int spfy_recompress24(int in_dtype, const void* in, size_t ld_in, int dtype, size_t rows, size_t cols,
                                const void* meta, void* comp_vals, void* out_masked, size_t ld_out, spfy_stream_t stream);
+/* spfy_optim24_step -- one optimizer step over a table of fp32 parameters, the
+ * refresh of the 2:4 layers' compressed operands included.
+ * algo SPFY_OPTIM_SGD follows torch's _multi_tensor_sgd, SPFY_OPTIM_ADAMW its
+ * _multi_tensor_adam with decoupled weight decay (AdamW), operation by operation
+ * in fp32; the hyperparameters of item i are groups[items[i].group].
+ *   SGD:   g += wd*p;  buf = *first ? g : buf*momentum + (1-dampening)*g;
+ *          g = nesterov ? g + momentum*buf : buf;  p -= lr*g
+ *          (momentum == 0: no buffer, g is used as is; first: an optional device
+ *          float, read and never written, so that a step skipped by found_inf
+ *          leaves the first step pending -- the caller clears it once a step
+ *          has been applied, e.g. by multiplying it by *found_inf)
+ *   AdamW: p *= 1 - lr*wd;  m = lerp(m, g, 1-beta1);  v = v*beta2 + (1-beta2)*g*g;
+ *          p -= lr/(1-beta1^t) * m / (sqrt(v)/sqrt(1-beta2^t) + eps)
+ *          with t = *step, the item's step count for this step (a device float,
+ *          already advanced; the call reads it and never writes it).
+ * grad_scale (optional, device float): every gradient is divided by it.
+ * found_inf (optional, device float): when *found_inf != 0 nothing is written
+ * anywhere (torch.amp.GradScaler's skipped step).  Both are read on the device, so
+ * a scaled step needs no host sync.
+ * Dense item (meta == NULL): rows * cols contiguous fp32 elements of param, grad
+ * and the state(s), updated elementwise (ld is not used).
+ * 2:4 item (meta != NULL): param is the fp32 master, rows x cols with leading
+ * dimension ld, grad and the states in the same layout; meta, vals: the SM100
+ * compressed operand of that shape (`dtype` F16/BF16).  At the positions meta
+ * keeps, param and state are updated; at the pruned positions +0 is written to
+ * param and state, whatever the gradient holds there (NaN and Inf included).
+ * vals receives the new master rounded to nearest even, byte for byte what
+ * spfy_recompress24(F32, param, ..., comp_vals = vals) would write.  vals_t
+ * (optional) receives byte for byte what spfy_transpose24_conv(vals, meta, rows,
+ * cols/(kh*kw), kh, kw, stride, pad) writes from the new vals: kh = kw = stride = 1,
+ * pad = 0 is spfy_transpose24(taps = 1), the W^T of a Linear layer.  meta and
+ * meta_t are only read and not written (the mask is fixed), nor are the padding
+ * bytes of vals and vals_t (they hold +0 since the operand was built).  Every
+ * element of param and state is read once and written once, every element of grad
+ * read once.  An item with rows * cols == 0 is skipped (its pointers may be NULL).
+ * One launch takes up to 192 items and 16 groups (fewer items when the strided
+ * convolutions among them bring more than 256 phases); larger tables take further
+ * launches, in table order.  The call makes no device allocation, no copy and no
+ * sync.
+ * Refusals, before any launch: bad algo, null tables, a null param or grad, a
+ * missing state (SGD with momentum: state1; AdamW: state1, state2 and step), fp32
+ * buffers not 4-byte (dense) or 16-byte (2:4) aligned, SM100 buffers not 16-byte
+ * aligned, ld < cols or ld % 4, a group out of range, negative lr or eps, nesterov
+ * without momentum or with dampening (SPFY_E_INVALID); a 16-bit dtype other than
+ * F16/BF16, rows or cols not multiples of 8, cols not kh*kw*c with c % 8 == 0, kh,
+ * kw > 16, pad > 8, stride > 8, items too large (SPFY_E_UNSUPPORTED). */
+enum { SPFY_OPTIM_SGD = 0, SPFY_OPTIM_ADAMW = 1 };
+typedef struct spfy_optim24_item {
+  float* param;
+  const float* grad;
+  float* state1;     /* SGD: momentum buffer (NULL when momentum == 0); AdamW: exp_avg */
+  float* state2;     /* AdamW: exp_avg_sq */
+  const float* step; /* AdamW: the step count of this step */
+  const float* first; /* SGD (optional, device): nonzero -> torch's first step, buf = g */
+  size_t rows, cols, ld;
+  size_t group;      /* index into groups */
+  int dtype;         /* 2:4 item: F16 / BF16 */
+  const void* meta;  /* NULL: dense item */
+  void* vals;
+  void* vals_t;      /* optional */
+  size_t kh, kw, stride, pad;  /* the convolution of vals_t */
+} spfy_optim24_item;
+typedef struct spfy_optim24_hparams {
+  double lr, momentum, dampening, weight_decay; /* SGD: lr, momentum, dampening, weight_decay */
+  double beta1, beta2, eps;                     /* AdamW: lr, betas, eps, weight_decay */
+  int nesterov;
+} spfy_optim24_hparams;
+SPFY_API int spfy_optim24_step(int algo, const spfy_optim24_item* items, size_t count,
+                               const spfy_optim24_hparams* groups, size_t n_groups, const float* grad_scale,
+                               const float* found_inf, spfy_stream_t stream);
 
 /* ------------------------------------------------------------------------
  * A4  cusparseLtMatmul                           include/sparsify.me/spmma.hxx:106-114

@@ -22,17 +22,18 @@ import os
 from . import capi  # noqa: F401  (fails loudly if the .so is missing)
 from .capi import (F16, BF16, F32, F64, PRUNE_STRIP_MAG, PRUNE_TILE_MAG, PRUNE_TILE_TRANSPOSABLE,  # noqa: F401
                    LAYOUT_CANONICAL, LAYOUT_SM100, OP_N, OP_T, OUT_T, SPMM_ALG_DEFAULT, SPMM_ALG_CUDA_CORE, SPMM_ALG_TENSOR,
-                   SPMM_ALG_TENSOR_FAST, ACT_NONE, ACT_RELU, ACT_GELU_TANH, GEMM_PRECISE, GEMM_FAST, SpfyError, launch_count, last_error, version)
+                   SPMM_ALG_TENSOR_FAST, ACT_NONE, ACT_RELU, ACT_GELU_TANH, GEMM_PRECISE, GEMM_FAST, OPTIM_SGD, OPTIM_ADAMW, SpfyError, launch_count, last_error, version)
 from .ops import (sparsify, prune24, prune24_check, compressed_bytes, spmma_compressed, spmma,  # noqa: F401
                   threshold_to_coo, coo_to_csr, batched, Compressed24, SpmmaPlan, prune24_batched,
                   alloc_compressed, pack_compressed, unpack_compressed, spmma_conv, spmma_conv_nhwc, permute_conv_weights,
                   Epilogue, fold_batchnorm, transpose24, recompress24, Linear24,
-                  Transpose24Conv, transpose24_conv, spmma_conv_dgrad_nhwc, conv_wgrad24_nhwc, Conv2d24)
+                  Transpose24Conv, transpose24_conv, spmma_conv_dgrad_nhwc, conv_wgrad24_nhwc, Conv2d24,
+                  SGD24, AdamW24)
 from . import shapes  # noqa: F401
 from . import multigpu  # noqa: F401
 
 __all__ = [
     "capi", "sparsify", "prune24", "prune24_check", "compressed_bytes", "spmma_compressed", "spmma",
-    "threshold_to_coo", "coo_to_csr", "batched", "Compressed24", "SpmmaPlan", "prune24_batched", "alloc_compressed", "Epilogue", "fold_batchnorm", "transpose24", "recompress24", "Linear24", "Transpose24Conv", "transpose24_conv", "spmma_conv_dgrad_nhwc", "conv_wgrad24_nhwc", "Conv2d24", "pack_compressed", "unpack_compressed", "shapes", "multigpu", "SpfyError",
+    "threshold_to_coo", "coo_to_csr", "batched", "Compressed24", "SpmmaPlan", "prune24_batched", "alloc_compressed", "Epilogue", "fold_batchnorm", "transpose24", "recompress24", "Linear24", "Transpose24Conv", "transpose24_conv", "spmma_conv_dgrad_nhwc", "conv_wgrad24_nhwc", "Conv2d24", "SGD24", "AdamW24", "pack_compressed", "unpack_compressed", "shapes", "multigpu", "SpfyError",
     "launch_count", "last_error", "version",
 ]

@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libsparsifyme_b200.so")
-SOURCES = ["api.cu", "prune.cu", "transpose24.cu", "spmma_sm100.cu", "gemm_sm100.cu", "spmm.cu", "multigpu.cu"]
+SOURCES = ["api.cu", "prune.cu", "transpose24.cu", "spmma_sm100.cu", "gemm_sm100.cu", "spmm.cu", "multigpu.cu", "optim24.cu"]
 NVCC_FLAGS = [
     "-std=c++17", "-O3", "-lineinfo",
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -22,6 +22,7 @@ OUT_T = 0x10  # flag OR-ed into opB: D is written transposed, [n][m]
 SPMM_ALG_DEFAULT, SPMM_ALG_CUDA_CORE, SPMM_ALG_TENSOR, SPMM_ALG_TENSOR_FAST = 0, 1, 2, 3
 GEMM_PRECISE, GEMM_FAST = 0, 1
 ACT_NONE, ACT_RELU, ACT_GELU_TANH = 0, 1, 2
+OPTIM_SGD, OPTIM_ADAMW = 0, 1
 OK, E_INVALID, E_UNSUPPORTED, E_CUDA, E_WORKSPACE, E_NCCL = 0, -1, -2, -3, -4, -5
 
 
@@ -53,6 +54,7 @@ SIGNATURES = {
     "spfy_prune24_batched": (c_int, [c_int, c_int, c_int, _P, _SZ, _P]),
     "spfy_transpose24": (c_int, [c_int, _P, _P, _SZ, _SZ, _SZ, _P, _P, _P, _P]),
     "spfy_recompress24": (c_int, [c_int, _P, _SZ, c_int, _SZ, _SZ, _P, _P, _P, _SZ, _P]),
+    "spfy_optim24_step": (c_int, [c_int, _P, _SZ, _P, _SZ, _P, _P, _P]),
     "spfy_transpose24_conv_bytes": (c_int, [c_int, _SZ, _SZ, _SZ, _SZ, _SZ, _SZ, POINTER(_SZ), POINTER(_SZ)]),
     "spfy_transpose24_conv": (c_int, [c_int, _P, _P, _SZ, _SZ, _SZ, _SZ, _SZ, _SZ, _P, _P, _P, _P]),
     "spfy_spmma_workspace_bytes": (c_int, [c_int, _SZ, _SZ, _SZ, POINTER(_SZ)]),
@@ -136,6 +138,21 @@ class Prune24Item(ctypes.Structure):
     """struct spfy_prune24_item"""
     _fields_ = [("in_", c_void_p), ("ld_in", c_size_t), ("out_dense", c_void_p), ("ld_out", c_size_t),
                 ("comp_vals", c_void_p), ("meta", c_void_p), ("rows", c_size_t), ("cols", c_size_t)]
+
+
+class Optim24Item(ctypes.Structure):
+    """struct spfy_optim24_item"""
+    _fields_ = [("param", c_void_p), ("grad", c_void_p), ("state1", c_void_p), ("state2", c_void_p), ("step", c_void_p),
+                ("first", c_void_p), ("rows", c_size_t), ("cols", c_size_t), ("ld", c_size_t), ("group", c_size_t),
+                ("dtype", c_int), ("meta", c_void_p), ("vals", c_void_p), ("vals_t", c_void_p), ("kh", c_size_t),
+                ("kw", c_size_t), ("stride", c_size_t), ("pad", c_size_t)]
+
+
+class Optim24Hparams(ctypes.Structure):
+    """struct spfy_optim24_hparams"""
+    _fields_ = [("lr", ctypes.c_double), ("momentum", ctypes.c_double), ("dampening", ctypes.c_double),
+                ("weight_decay", ctypes.c_double), ("beta1", ctypes.c_double), ("beta2", ctypes.c_double),
+                ("eps", ctypes.c_double), ("nesterov", c_int)]
 
 
 def last_error():

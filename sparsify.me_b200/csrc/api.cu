@@ -97,6 +97,7 @@ int spfy_init(void) {
   spfy::warm_spmma_kernels();
   spfy::warm_spmm_kernels();
   spfy::warm_gemm_kernels();
+  spfy::warm_optim24_kernels();
   touch_kernel(convert_kernel<float, __half>);
   touch_kernel(convert_kernel<float, __nv_bfloat16>);
   touch_kernel(convert_kernel<__half, float>);

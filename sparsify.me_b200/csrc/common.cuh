@@ -172,6 +172,7 @@ void warm_transpose24_kernels();
 void warm_spmma_kernels();
 void warm_spmm_kernels();
 void warm_gemm_kernels();
+void warm_optim24_kernels();
 
 inline size_t dtype_bytes(int dtype) {
   switch (dtype) {

@@ -10,6 +10,7 @@ current stream.  Nothing here computes on the host.
 """
 import ctypes
 import sys
+import weakref
 from dataclasses import dataclass
 
 import torch
@@ -473,6 +474,10 @@ def recompress24(dense, comp, masked_out=None, values=True):
                            masked_out.stride(0) if masked_out is not None else 0, _stream())
 
 
+# the Linear24 / Conv2d24 that owns a weight Parameter, by id(weight): how SGD24 / AdamW24 find a 2:4 layer's operands
+_LAYERS24 = weakref.WeakValueDictionary()
+
+
 class _Linear24Fn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x2, weight, bias, layer):
@@ -528,6 +533,7 @@ class Linear24(torch.nn.Module):
         self.bias = torch.nn.Parameter(bias) if bias is not None else None
         self.comp, self.comp_t, self.dtype = comp, comp_t, dtype
         self._synced_version = self.weight._version
+        _LAYERS24[id(self.weight)] = self
 
     @classmethod
     def from_dense(cls, w, b=None, dtype=torch.float16):
@@ -612,6 +618,7 @@ class Conv2d24(torch.nn.Module):
         self.m, self.c, self.kh, self.kw = weight.shape
         self.stride, self.padding = stride, padding
         self._synced_version = self.weight._version
+        _LAYERS24[id(self.weight)] = self
 
     @classmethod
     def from_dense(cls, weight, bias=None, stride=1, padding=0, dtype=torch.float16, groups=1, dilation=1):
@@ -660,6 +667,253 @@ class Conv2d24(torch.nn.Module):
             raise ValueError("Conv2d24: the input must be a 4-D channels_last tensor: convert with "
                              "x.contiguous(memory_format=torch.channels_last)")
         return _Conv2d24Fn.apply(x, self.weight, self.bias, self)
+
+
+def _non_overlapping_dense(t):
+    expected = 1
+    for size, stride in sorted(zip(t.shape, t.stride()), key=lambda e: e[1]):
+        if size != 1:
+            if stride != expected:
+                return False
+            expected *= size
+    return True
+
+
+def _layer24_of(p):
+    layer = _LAYERS24.get(id(p))
+    return layer if layer is not None and layer.weight is p else None
+
+
+class _Optim24(torch.optim.Optimizer):
+    """spfy_optim24_step behind torch.optim.Optimizer: one step() updates every parameter that has a gradient in one
+    library launch (up to 192 parameters and 16 parameter groups per launch; more take further launches).  The weight of a Linear24 / Conv2d24 is a 2:4 item: updated at
+    the kept positions, re-masked, and the layer's compressed operands refilled in the same pass, so no refresh() is
+    needed.  Every other parameter must be a non-overlapping, dense fp32 tensor; it is updated elementwise.  State
+    tensors carry torch's names and the parameter's layout, so state_dict() moves to and from the torch optimizer.
+    GradScaler: grad_scale and found_inf are read on the device (no sync); a step with found_inf != 0 writes nothing."""
+    _ALGO = None
+    _step_supports_amp_scaling = True
+
+    def __init__(self, params, defaults):
+        for k in ("amsgrad", "maximize", "foreach", "fused", "differentiable"):
+            if defaults.get(k):
+                raise ValueError(f"{type(self).__name__}: {k}=True is not supported")
+        super().__init__(params, defaults)
+
+    def add_param_group(self, param_group):
+        super().add_param_group(param_group)
+        group = self.param_groups[-1]
+        try:
+            self._check_group(group)
+            device = None
+            for g in self.param_groups:
+                for p in g["params"]:
+                    if p.dtype != torch.float32:
+                        raise TypeError(f"{type(self).__name__}: parameters must be fp32, got {p.dtype}")
+                    if not _non_overlapping_dense(p):
+                        raise ValueError(f"{type(self).__name__}: a parameter of strides {p.stride()} is not dense")
+                    if device is not None and p.device != device:
+                        raise ValueError(f"{type(self).__name__}: parameters on {device} and {p.device}")
+                    device = p.device
+        except (TypeError, ValueError):
+            self.param_groups.pop()
+            raise
+
+    def _check_group(self, group):
+        if group["lr"] < 0.0:
+            raise ValueError(f"Invalid learning rate: {group['lr']}")
+        for k in ("amsgrad", "maximize", "foreach", "fused", "differentiable"):
+            if group.get(k):
+                raise ValueError(f"{type(self).__name__}: {k}=True is not supported")
+
+    def _table(self):
+        """The item table of the parameters with a gradient: (ctypes items, ctypes hparams, params, layers, keep-alive
+        tensors, AdamW step counts, SGD first-step flags as (param, flag)).  Creates missing state; needs no device."""
+        items, params, layers, keep, steps, firsts = [], [], [], [], [], []
+        hps = (capi.Optim24Hparams * len(self.param_groups))()
+        for gi, group in enumerate(self.param_groups):
+            self._hparams(group, hps[gi])
+            for p in group["params"]:
+                g = p.grad
+                if g is None:
+                    continue
+                if g.is_sparse:
+                    raise TypeError(f"{type(self).__name__} does not support sparse gradients")
+                if g.stride() != p.stride():
+                    g = torch.empty_like(p).copy_(g)  # the kernel reads the gradient in the parameter's layout
+                    keep.append(g)
+                state = self.state[p]
+                it = capi.Optim24Item(param=p.data_ptr(), grad=g.data_ptr(), rows=1, cols=p.numel(), ld=p.numel(),
+                                      group=gi)
+                for k, s in self._states(p, state, it, firsts):
+                    if s.stride() != p.stride() or s.device != p.device:
+                        s = state[k] = torch.empty_like(p).copy_(s)
+                    setattr(it, "state1" if k in ("momentum_buffer", "exp_avg") else "state2", s.data_ptr())
+                if "step" in state:
+                    st = state["step"]
+                    if st.device != p.device or st.dtype != torch.float32:
+                        st = state["step"] = st.to(device=p.device, dtype=torch.float32)
+                    it.step = st.data_ptr()
+                    steps.append(st)
+                layer = _layer24_of(p)
+                if layer is not None:
+                    self._item24(layer, it)
+                    layers.append(layer)
+                items.append(it)
+                params.append(p)
+        return (capi.Optim24Item * len(items))(*items), hps, params, layers, keep, steps, firsts
+
+    @staticmethod
+    def _item24(layer, it):
+        comp = layer.comp
+        op_t = layer.op_t if isinstance(layer, Conv2d24) else layer.comp_t
+        if any(t.device != layer.weight.device for t in (comp.vals, comp.meta, op_t.vals)):
+            raise ValueError(f"{type(layer).__name__}: the compressed operands are not on the weight's device")
+        it.rows, it.cols, it.dtype = comp.rows, comp.cols, _DT[layer.dtype]
+        it.meta, it.vals = comp.meta.data_ptr(), comp.vals.data_ptr()
+        if isinstance(layer, Conv2d24):
+            it.ld = layer._w2d().stride(0)
+            it.vals_t = layer.op_t.vals.data_ptr()
+            it.kh, it.kw, it.stride, it.pad = layer.kh, layer.kw, layer.stride, layer.padding
+        else:
+            w = layer.weight
+            if tuple(w.shape) != (comp.rows, comp.cols) or w.stride(1) != 1:
+                raise ValueError("Linear24: the weight is no longer a row-major [out, in] matrix")
+            it.ld = w.stride(0)
+            it.vals_t = layer.comp_t.vals.data_ptr()
+            it.kh = it.kw = it.stride = 1
+
+    @torch.no_grad()
+    def step(self, closure=None):
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        for group in self.param_groups:  # the table holds raw addresses: refuse host memory before anything changes
+            for p in group["params"]:
+                if p.grad is not None and not p.is_cuda:
+                    raise capi.SpfyError(capi.E_INVALID, type(self).__name__, f"a parameter on {p.device}: "
+                                         "sparsify.me_b200 has no host path")
+        items, hps, params, layers, keep, steps, firsts = self._table()
+        if not params:
+            return loss
+        grad_scale = getattr(self, "grad_scale", None)
+        found_inf = getattr(self, "found_inf", None)
+        if grad_scale is not None:
+            grad_scale = grad_scale.to(device=params[0].device, dtype=torch.float32)
+            keep.append(grad_scale)
+        if found_inf is not None:
+            found_inf = found_inf.to(device=params[0].device, dtype=torch.float32)
+            keep.append(found_inf)
+        inc = 1.0 if found_inf is None else 1.0 - found_inf.reshape(())
+        if steps:  # AdamW: the count advances by 1 - found_inf, on the stream, before the kernel reads it
+            torch._foreach_add_(steps, inc)
+        try:
+            capi.spfy_optim24_step(self._ALGO, items, len(items), hps, len(hps), _ptr(grad_scale), _ptr(found_inf),
+                                   _stream())
+        except capi.SpfyError:
+            if steps:  # refused before any launch: the state is as it was
+                torch._foreach_sub_(steps, inc)
+            raise
+        if firsts:  # SGD: a first step is done once it was applied; a skipped one (found_inf != 0) stays pending
+            if found_inf is None:
+                for p, _ in firsts:
+                    del self._first[p]
+            else:
+                torch._foreach_mul_([f for _, f in firsts], found_inf.reshape(()))
+        torch.autograd.graph.increment_version(params)
+        for layer in layers:
+            layer._synced_version = layer.weight._version  # its operands were refilled by the same launch
+        return loss
+
+
+class SGD24(_Optim24):
+    """torch.optim.SGD for models with Linear24 / Conv2d24 layers: the update of torch's _multi_tensor_sgd in fp32,
+    the 2:4 layers refreshed by the same launch.  maximize, foreach, fused and differentiable are not supported.
+        opt = SGD24(model.parameters(), lr=0.1, momentum=0.9)
+        loss.backward(); opt.step()          # no refresh()"""
+    _ALGO = capi.OPTIM_SGD
+
+    def __init__(self, params, lr=1e-3, momentum=0.0, dampening=0.0, weight_decay=0.0, nesterov=False, *,
+                 maximize=False, foreach=None, differentiable=False, fused=None):
+        if lr < 0.0:
+            raise ValueError(f"Invalid learning rate: {lr}")
+        if momentum < 0.0:
+            raise ValueError(f"Invalid momentum value: {momentum}")
+        if weight_decay < 0.0:
+            raise ValueError(f"Invalid weight_decay value: {weight_decay}")
+        if nesterov and (momentum <= 0 or dampening != 0):
+            raise ValueError("Nesterov momentum requires a momentum and zero dampening")
+        # param -> device float, 1 while torch's first step (buf = grad) is still to be applied to the parameter
+        self._first = {}
+        super().__init__(params, dict(lr=lr, momentum=momentum, dampening=dampening, weight_decay=weight_decay,
+                                      nesterov=nesterov, maximize=maximize, foreach=foreach,
+                                      differentiable=differentiable, fused=fused))
+
+    def _check_group(self, group):
+        super()._check_group(group)
+        if group["nesterov"] and (group["momentum"] <= 0 or group["dampening"] != 0):
+            raise ValueError("Nesterov momentum requires a momentum and zero dampening")
+
+    @staticmethod
+    def _hparams(group, h):
+        h.lr, h.momentum, h.dampening = group["lr"], group["momentum"], group["dampening"]
+        h.weight_decay, h.nesterov = group["weight_decay"], int(bool(group["nesterov"]))
+
+    def load_state_dict(self, state_dict):
+        super().load_state_dict(state_dict)
+        self._first.clear()  # a loaded momentum buffer has seen its first step
+
+    def _states(self, p, state, it, firsts):
+        if self.param_groups[it.group]["momentum"] == 0:
+            return []
+        if state.get("momentum_buffer") is None:
+            state["momentum_buffer"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+            self._first[p] = torch.ones((), dtype=torch.float32, device=p.device)
+        flag = self._first.get(p)
+        if flag is not None:
+            it.first = flag.data_ptr()
+            firsts.append((p, flag))
+        return [("momentum_buffer", state["momentum_buffer"])]
+
+
+class AdamW24(_Optim24):
+    """torch.optim.AdamW for models with Linear24 / Conv2d24 layers: the update of torch's _multi_tensor_adam with
+    decoupled weight decay in fp32, the 2:4 layers refreshed by the same launch.  The bias corrections come from the
+    `step` state, a device float, so a step needs no host value.  amsgrad, maximize, foreach, fused and differentiable
+    are not supported."""
+    _ALGO = capi.OPTIM_ADAMW
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, amsgrad=False, *,
+                 maximize=False, foreach=None, capturable=False, differentiable=False, fused=None):
+        if lr < 0.0:
+            raise ValueError(f"Invalid learning rate: {lr}")
+        if eps < 0.0:
+            raise ValueError(f"Invalid epsilon value: {eps}")
+        if not 0.0 <= betas[0] < 1.0 or not 0.0 <= betas[1] < 1.0:
+            raise ValueError(f"Invalid beta parameters: {betas}")
+        if weight_decay < 0.0:
+            raise ValueError(f"Invalid weight_decay value: {weight_decay}")
+        super().__init__(params, dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, amsgrad=amsgrad,
+                                      maximize=maximize, foreach=foreach, capturable=capturable,
+                                      differentiable=differentiable, fused=fused, decoupled_weight_decay=True))
+
+    def _check_group(self, group):
+        super()._check_group(group)
+        if group["eps"] < 0.0:
+            raise ValueError(f"Invalid epsilon value: {group['eps']}")
+
+    @staticmethod
+    def _hparams(group, h):
+        h.lr, h.weight_decay, h.eps = group["lr"], group["weight_decay"], group["eps"]
+        h.beta1, h.beta2 = group["betas"]
+
+    def _states(self, p, state, it, firsts):
+        if "step" not in state:
+            state["step"] = torch.zeros((), dtype=torch.float32, device=p.device)
+            state["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+            state["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+        return [("exp_avg", state["exp_avg"]), ("exp_avg_sq", state["exp_avg_sq"])]
 
 
 # ----------------------------------------------------------------------------- A4
