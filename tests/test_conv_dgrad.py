@@ -145,9 +145,13 @@ def test_refusals_need_no_device(spfy):
 
 
 # (kh = kw, stride, pad): s in {1, 2, 3}, k in {1, 2, 3, 5, 7}; first dy offsets negative (pad < k - 1), zero and positive
-# (1x1 with pad 1: phase 1 reads dy one position ahead)
+# (1x1 with pad 1: phase 1 reads dy one position ahead).  Then each dimension of the geometries of
+# test_gpu_conv24_geometry.py: pad >= filter, stride > filter (phases without taps), 1 x k filters' 1-tap dimension with
+# pad 3, and the contract's maxima (16 taps with pad 8 at stride 1 and 8, 11 taps at stride 4)
 PHASE_CASES = [(3, 1, 1), (5, 1, 0), (1, 2, 0), (1, 2, 1), (2, 2, 0), (3, 2, 1), (3, 2, 0), (5, 2, 2), (7, 2, 3),
-               (1, 3, 1), (2, 3, 2), (3, 3, 1), (5, 3, 0), (7, 3, 3), (3, 3, 4)]
+               (1, 3, 1), (2, 3, 2), (3, 3, 1), (5, 3, 0), (7, 3, 3), (3, 3, 4),
+               (1, 1, 1), (3, 1, 3), (1, 2, 3), (3, 3, 2), (5, 3, 2), (1, 4, 0), (3, 4, 1), (2, 5, 0), (11, 4, 2),
+               (16, 1, 8), (16, 8, 8)]
 
 
 @pytest.mark.parametrize("k,s,p", PHASE_CASES)

@@ -21,13 +21,14 @@ TDT = {0: torch.float16, 1: torch.bfloat16}
 
 
 def pruned_filter(spfy, orc, cuda, m, c, k, dt, seed):
-    """a TILE-transposable pruned m x (k*k*c) filter in (kh, kw, c) order: (comp, dense bits, fp64 NCHW weight).  The
-    values are zero-free, so TILE_MAG keeps what PRUNE_TILE_TRANSPOSABLE keeps; it stands in where that mode's one-pass
-    kernel refuses the width (k*k*c % 16, e.g. c = 72)."""
-    wt = to_dev(zero_free(orc, dt, (m, c * k * k), seed=seed), dt, cuda)
-    mode = spfy.PRUNE_TILE_TRANSPOSABLE if (c * k * k) % 16 == 0 else spfy.PRUNE_TILE_MAG
-    comp, dense = prune_dev(spfy, bits_of(spfy.permute_conv_weights(wt, c, k, k)), dt, cuda, mode)
-    return comp, bits_of(dense), dense.double().view(m, k, k, c).permute(0, 3, 1, 2)
+    """a TILE-transposable pruned m x (kh*kw*c) filter in (kh, kw, c) order, k = kh = kw or k = (kh, kw): (comp, dense
+    bits, fp64 NCHW weight).  The values are zero-free, so TILE_MAG keeps what PRUNE_TILE_TRANSPOSABLE keeps; it stands in
+    where that mode's one-pass kernel refuses the width (kh*kw*c % 16, e.g. c = 72)."""
+    kh, kw = k if isinstance(k, tuple) else (k, k)
+    wt = to_dev(zero_free(orc, dt, (m, c * kh * kw), seed=seed), dt, cuda)
+    mode = spfy.PRUNE_TILE_TRANSPOSABLE if (c * kh * kw) % 16 == 0 else spfy.PRUNE_TILE_MAG
+    comp, dense = prune_dev(spfy, bits_of(spfy.permute_conv_weights(wt, c, kh, kw)), dt, cuda, mode)
+    return comp, bits_of(dense), dense.double().view(m, kh, kw, c).permute(0, 3, 1, 2)
 
 
 def rand_nhwc(shape, dt, cuda, seed):
