@@ -520,6 +520,29 @@ SPFY_API int spfy_coo_to_csr(const int32_t* row_idx, size_t nnz, size_t rows,
  *   TENSOR      : the tensor-core route or SPFY_E_UNSUPPORTED / SPFY_E_WORKSPACE.
  *   TENSOR_FAST : same with ONE TF32 product per fp32 multiply (10-bit mantissas; the accuracy
  *                 class of cuBLAS's TF32 mode).  16-bit operands: identical to TENSOR.
+ * Special values (fp32).  Finite values and their products are handled as by spfy_gemm_* (below)
+ * on the tensor-core routes and in IEEE fp32 on the CUDA-core kernels.  Inf and NaN in B follow
+ * one of two semantics, by kernel:
+ *   stored entries : only the stored entries of A are multiplied (cuSPARSE's semantics), so a
+ *                    non-finite B[kk][j] reaches only the rows of C_b that store an entry in
+ *                    column kk; IEEE classes (Inf * 0 = NaN for a stored zero).  The per-non-zero
+ *                    CUDA-core kernels: CUDA_CORE below 35 % non-zeros and DEFAULT below its
+ *                    tensor threshold (CSR, COO), and the blocked-ELL CUDA-core kernel (padding
+ *                    ids < 0 store nothing; a stored block multiplies all of its values).
+ *   dense image    : A is multiplied as a dense matrix whose structural zeros are real zeros,
+ *                    and 0 * Inf = NaN, so a non-finite B[kk][j] makes all of column j of C_b
+ *                    non-finite (NaN in the rows that do not store column kk).  Every
+ *                    tensor-core route (TENSOR, TENSOR_FAST, DEFAULT from 2 % non-zeros for CSR /
+ *                    COO -- 20 % when B needs the padded copy, ldb = k = 147 --, DEFAULT for
+ *                    blocked-ELL) and the CUDA-core dense walk (CUDA_CORE from 35 %).
+ *                    Blocked-ELL exceptions: a batch chunk in which some block-row repeats an
+ *                    id, and DEFAULT without a tensor route (e.g. a workspace sized for
+ *                    CUDA_CORE), run on the blocked-ELL CUDA-core kernel: stored entries, IEEE.
+ * So DEFAULT switches between the two with the density of A.  Classes of the non-finite outputs:
+ * IEEE on the CUDA-core kernels; NaN on TENSOR (and DEFAULT on the tensor route), as PRECISE;
+ * on TENSOR_FAST those of SPFY_GEMM_FAST, except that the image of a CSR / COO A is built by fp32
+ * additions of the stored values, so a NaN in A stays NaN.  beta = 0: C is written, never read
+ * (a NaN in C does not survive), on every route.
  * ---------------------------------------------------------------------- */
 enum {
   SPFY_SPMM_ALG_DEFAULT = 0,
@@ -598,6 +621,26 @@ SPFY_API int spfy_spmm_bell_batched(int alg, int dtype, size_t rows, size_t cols
  *                      nearest); the other keeps its raw tile in shared memory as hi (the
  *                      tensor core truncates it) with lo written behind it;
  *   SPFY_GEMM_FAST     one TF32 product.
+ * Special values.  beta = 0: C is written, never read (a NaN in C does not survive).  Finite
+ * operands whose products and sums stay inside the fp32 range give finite results, except that
+ * PRECISE: the streamed operand's hi is rounded to nearest, the other's truncated.  A finite
+ * value of the streamed operand with |x| >= 0x7f7ff000 (3.4020e38, the top 2^-11 of the fp32
+ * range) rounds to hi = ±Inf, lo = ∓Inf: every output it reaches (its whole row or column of
+ * C) is NaN.  In the other operand such values give finite, accurate results.  The streamed
+ * operand is op(A) when the kernel maps m onto its 128-row tiles, op(B) when it maps n there
+ * (orient() in gemm_sm100.cu: the mapping that issues fewer padded MACs, ties to the larger of
+ * m and n); the SpMM tensor routes call it with op(A) = the dense image of A, row-major, and
+ * for CSR / COO with n = n * num_batches (the batches of B side by side).
+ * Non-finite operands, per mode:
+ *   F16 / BF16         IEEE: Inf * finite nonzero = ±Inf, Inf * 0 = NaN, Inf - Inf = NaN, NaN
+ *                      stays NaN.
+ *   SPFY_GEMM_FAST     IEEE on the operands as the tensor core reads them, truncated to TF32: a
+ *                      NaN whose payload lies only in the low 13 mantissa bits reads as ±Inf.
+ *   SPFY_GEMM_PRECISE  an Inf or NaN operand splits into hi = ±Inf / NaN and lo = NaN, so every
+ *                      output it reaches (row i of C for A[i][kk], column j for B[kk][j]) is
+ *                      NaN, also where IEEE gives ±Inf.  Other outputs are unaffected.
+ * With non-finite operands (and finite ones below 0x7f7ff000), in every mode an output is
+ * non-finite exactly where the IEEE result is.
  * Any other `precision` is refused with SPFY_E_INVALID before any device work, for every dtype.
  * The operands are fetched by TMA, which needs 16-byte aligned bases and lda / ldb /
  * batch strides that are multiples of 16 bytes; an operand that misses this (ldb = k = 147

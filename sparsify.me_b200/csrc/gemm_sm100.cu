@@ -31,6 +31,16 @@
 // the tensor core (|lo| < 2^-10 |x|); the lo*lo term is dropped and each lo is read to TF32 precision, so every
 // product is exact to ~2^-19 relative in the worst case, accumulation is fp32.  The parity tests bound the result
 // against an fp64 oracle by 4e-6 * sum_k |a||b| (tests/test_gpu_tensor.py).
+// Special values: rounding Au's hi carries into the Inf exponent for a finite |x| >= 0x7f7ff000 (the top 2^-11 of the
+// fp32 range), so hi = ±Inf, lo = ∓Inf and every output such a value reaches is NaN; Bu's truncated hi stays finite.
+// A guard that truncates there instead costs the Au splitters, which bound this kernel, extra instructions per value.
+// Measured on a B200 (1000 W limit), old and new builds alternating, three runs each (spread <= 0.011 ms), bench.py
+// --workload coo, 14.14 ms per step without a guard:
+//   |x| < EDGE ? 0x1000 : 0 added to x (FSETP on |x| + a predicated move, 2 per value)   14.79 ms  (+4.6 %)
+//   compare on x << 1 and select (3 per value)                                           15.13 ms  (+7 %)
+//   max of |x| over the 16 values of a piece, guarded path only when it reaches EDGE      15.70 ms  (+11 %)
+// and the fp32 GEMM sweep of profiling/gemm_timing 4-8 % slower.  So no guard is taken: spfy_b200.h states the range.
+// An Inf or NaN operand has lo = NaN on either side: every output it reaches is NaN (tests/test_gpu_fp32_edges.py).
 #include "gemm_sm100.cuh"
 #include "tc_ptx.cuh"
 
